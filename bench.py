@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- VQ lookup throughput on B200 (BASELINE.json metric: "VQ lookup vectors/sec at K=512, D=256").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): N = 8 x 64 x 64 latent vectors, D = 256, K = 512 codebook, fp32, per GPU.
 One "step" = one eval-mode lookup of the whole batch: nearest-code assignment (tcgen05 filter + exact
@@ -14,8 +14,12 @@ everything VectorQuantizer.forward returns (vq_img.py:228-244).  Inputs are synt
   roofline : the dominant kernel (assign_tc_kernel): 2*N*K*D flops / its CUDA-event duration vs the
           measured dense bf16/fp16 tensor peak of MEASURED_PEAKS.json.
   cpu_baseline : the oracle port of the reference's CPU path on the box's host cores (rank 0, N=1).
-With --impl reference the reference's CPU path itself is timed (oracle port; /root/reference is
-absent on the GPU box) on the same workload.
+With --impl reference the reference's CPU path itself is timed (oracle port, or the original module when
+VQSEG_REF points to a checkout of it) on the same workload.
+--dump-outputs DIR writes what the last timed step returned (quantize, embed_index, loss, code_usage; rank 0's
+with several GPUs) as DIR/<name>.npy, floats as float32 and integers as float64.  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.  The GPU arm's last step reads ring slot
+(steps - 1) % ring; slot 0 is the seed-0 batch and codebook, which tests/golden pins as case "c2_randn".
 """
 import argparse
 import json
@@ -77,8 +81,19 @@ def cpu_reference_step(model, x):
         return model(x)
 
 
+def dump_outputs(out_dir, outputs):
+    """(quantize, embed_index, loss, code_usage) of one forward -> out_dir/<name>.npy: floating outputs as float32,
+    integer ones as float64 (exact for any index).  The C2 batch comes to 32 MiB of quantize + 256 KiB of indices."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in zip(("quantize", "embed_index", "loss", "code_usage"), outputs):
+        t = t.detach().cpu()
+        t = t.to(torch.float32 if t.is_floating_point() else torch.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+
+
 def build_cpu_model(e):
-    """The reference's CPU path: the live module if /root/reference exists, else the oracle port."""
+    """The reference's CPU path: the original module if VQSEG_REF points to a checkout of it, else the oracle port."""
     from oracle.ref_loader import load_reference_vq_img
     ref = load_reference_vq_img()
     if ref is not None:
@@ -102,8 +117,10 @@ def run_reference(args, rank, world):
         cpu_reference_step(model, x)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_reference_step(model, x)
+        out = cpu_reference_step(model, x)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     val = N_VEC * args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": "vectors/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3,
@@ -299,7 +316,7 @@ def extras_c5(dev, rank, world, n=4 << 20, d=256, k=65536):
 
 
 def extras_cpu_port(budget_s=25.0):
-    """The reference's CPU path (oracle port, or the live module when /root/reference exists) beside the extras, at the
+    """The reference's CPU path (oracle port, or the original module when VQSEG_REF is set) beside the extras, at the
     largest sizes that finish in seconds: it cannot hold configs 4 and 5 at full size (BASELINE.md 2)."""
     from oracle import vq_oracle as O
     torch.set_num_threads(os.cpu_count())
@@ -349,13 +366,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch eagerly instead of replaying CUDA graphs")
     ap.add_argument("--no-extras", action="store_true", help="skip the extras (configs 1, 4, 5, multi-GPU parity)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
-        if args.steps > 50:
-            args.steps = 50                       # bounded: ~0.1 s per step on host cores
         run_reference(args, rank, world)
         return
 
@@ -416,10 +434,12 @@ def main():
     barrier()
     ev0.record()
     for i in range(args.steps):
-        step(i)
+        out = step(i)
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)    # before any further call overwrites the captured graph's outputs
     # ---- dominant kernel duration: CUDA events recorded by the C ABI on the launching stream around the filter
     # (which=0) and rescoring (which=1) kernels.  Captured into a second set of graphs so the kernels are timed
     # under the same launch conditions as the timed region (graph replay, ring of cold inputs).

@@ -1,21 +1,20 @@
 """Loads the LIVE reference hot path (vector_quantizer/vq_img.py) by file path -- TEST INFRASTRUCTURE.
 
-Only usable where /root/reference exists (the authoring container).  It is used to pin the
-restated oracle (tests/test_oracle.py) and to generate tests/golden/*.pt
-(tests/golden/make_golden.py).  Nothing that runs on the GPU box may depend on it.
-`import vector_quantizer` (the package) fails here because easydict is not installed, but
-vq_img.py itself needs only torch + einops (SURVEY.md §8c).
+Only usable where the environment variable VQSEG_REF names a checkout of the original chaeyeongyun/VQ_SEG
+repository; without one, reference_root() is None and the tests that need the live reference skip.  It is used to
+pin the restated oracle (tests/test_oracle.py) and to generate tests/golden/*.pt (tests/golden/make_golden.py): the
+stored goldens are the pin everywhere else, and nothing on the product path may depend on this module.
+`import vector_quantizer` (the package) needs easydict, but vq_img.py itself needs only torch + einops
+(SURVEY.md §8c).
 """
 import importlib.util
 import os
 
-_CANDIDATES = [os.environ.get("VQSEG_REF", ""), "/root/reference"]
-
 
 def reference_root():
-    for root in _CANDIDATES:
-        if root and os.path.isfile(os.path.join(root, "vector_quantizer", "vq_img.py")):
-            return root
+    root = os.environ.get("VQSEG_REF", "")
+    if root and os.path.isfile(os.path.join(root, "vector_quantizer", "vq_img.py")):
+        return root
     return None
 
 

@@ -27,6 +27,6 @@ def golden_seghead():
 
 @pytest.fixture(scope="session")
 def ref_vq():
-    """The live reference vq_img module, or None when /root/reference is absent (GPU box)."""
+    """The live reference vq_img module, or None without a reference checkout (VQSEG_REF, oracle/ref_loader.py)."""
     from oracle.ref_loader import load_reference_vq_img
     return load_reference_vq_img()

@@ -21,7 +21,7 @@ import cases  # noqa: E402
 
 def main():
     R = load_reference_vq_img()
-    assert R is not None, "reference not found (needs /root/reference)"
+    assert R is not None, "reference not found: set VQSEG_REF to a checkout of the original repository"
     torch.set_num_threads(os.cpu_count())
     out = {"meta": {"torch": torch.__version__, "threads": torch.get_num_threads(),
                     "cpu_capability": torch.backends.cpu.get_cpu_capability()}}

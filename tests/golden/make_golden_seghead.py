@@ -46,7 +46,7 @@ def run_case(cls, build, distance):
 
 def main():
     R = load_reference_seghead()
-    assert R is not None, "reference not found (needs /root/reference)"
+    assert R is not None, "reference not found: set VQSEG_REF to a checkout of the original repository"
     torch.set_num_threads(os.cpu_count())
     out = {"meta": {"torch": torch.__version__, "threads": torch.get_num_threads()}, "seghead": {}}
     for name, (build, distance) in cases.SEGHEAD_CASES.items():

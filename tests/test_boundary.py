@@ -8,9 +8,10 @@ import pytest
 import torch
 
 import vq_seg_b200 as V
+from oracle.ref_loader import reference_root
 from oracle.vq_oracle import OracleVectorQuantizer
 
-REF_CFG = "/root/reference/config"
+REF_CFG = os.path.join(reference_root() or "", "config")
 
 
 def test_constructor_signature_matches_reference(ref_vq):
@@ -73,7 +74,7 @@ def test_make_vq_module():
         V.make_vq_module({"num_embeddings": [0, 512]}, chans, 5)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="reference configs only exist in the authoring container")
+@pytest.mark.skipif(reference_root() is None, reason="needs a reference checkout (VQSEG_REF) for its config/*.json")
 def test_every_reference_vq_cfg_constructs():
     n = 0
     for dirpath, _, files in os.walk(REF_CFG):

@@ -1,4 +1,4 @@
-"""Drop-in evidence against the UNMODIFIED reference models (authoring container only: needs /root/reference).
+"""Drop-in evidence against the UNMODIFIED reference models (needs a checkout of the original repository: VQSEG_REF).
 `vq_seg_b200.install()` swaps the class into the reference's modules; `make_model` of the reference then builds
 the north-star network (VQRePTUnet1x1v2, config/vqreptunet1x1v2.json) with B200 codebooks, and its state_dict
 keys are the reference's.  Construction only: the forward needs a GPU (covered by test_gpu_parity.py)."""
@@ -10,10 +10,12 @@ import types
 
 import pytest
 
-REF = "/root/reference"
+from oracle.ref_loader import reference_root
+
+REF = reference_root()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the authoring container")
+@pytest.mark.skipif(REF is None, reason="needs a reference checkout (VQSEG_REF)")
 def test_reference_model_builds_with_b200_codebooks():
     # packages the reference imports that are not installed here (SURVEY 8b): easydict, pretrainedmodels
     class EasyDict(dict):

@@ -1,5 +1,5 @@
 """Pins the restated CPU oracle: (1) against the committed golden vectors produced by the live
-reference, (2) against the live reference itself when /root/reference is present."""
+reference, (2) against the live reference itself when VQSEG_REF names a checkout of it."""
 import pytest
 import torch
 
@@ -7,8 +7,20 @@ import cases
 from oracle import vq_oracle as O
 
 
+@pytest.fixture
+def golden_threads(golden, golden_seghead):
+    """ATen splits a float reduction (the mse loss, softmax's sum, ...) over its intra-op threads, so the last bits of
+    a CPU result depend on the thread count: the oracle runs with the count the goldens were recorded with."""
+    threads = {golden["meta"]["threads"], golden_seghead["meta"]["threads"]}
+    assert len(threads) == 1
+    n = torch.get_num_threads()
+    torch.set_num_threads(threads.pop())
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.mark.parametrize("name", list(cases.FORWARD_CASES))
-def test_oracle_matches_golden_forward(golden, name):
+def test_oracle_matches_golden_forward(golden, golden_threads, name):
     rec = golden["forward"][name]
     x, e = cases.FORWARD_CASES[name]()
     assert cases.sha(x) == rec["x_sha"] and cases.sha(e) == rec["e_sha"], "seeded inputs drifted"
@@ -28,7 +40,7 @@ def test_oracle_matches_golden_forward(golden, name):
 
 
 @pytest.mark.parametrize("name", cases.KMEANS_CASES)
-def test_oracle_matches_golden_kmeans(golden, name):
+def test_oracle_matches_golden_kmeans(golden, golden_threads, name):
     rec = golden["kmeans"][name]
     x, k, iters, init_idx, use_cos = cases.kmeans_case(name)
     assert cases.sha(x) == rec["x_sha"]
@@ -51,7 +63,7 @@ def test_euclidean_dist_restatement_is_cdist():
 
 def test_live_reference_forward_backward(ref_vq):
     if ref_vq is None:
-        pytest.skip("/root/reference not present (GPU box): golden vectors are the pin there")
+        pytest.skip("no reference checkout (VQSEG_REF): golden vectors are the pin")
     torch.manual_seed(5)
     for (b, c, h, w, k, wgt) in [(2, 64, 16, 16, 128, 1), (1, 256, 8, 8, 512, 0.25), (2, 512, 12, 12, 64, 0)]:
         ref = ref_vq.VectorQuantizer(dim=c, num_embeddings=k, commitment_weight=wgt)
@@ -80,7 +92,7 @@ def test_live_reference_forward_backward(ref_vq):
 
 def test_live_reference_kmeans_same_rng(ref_vq):
     if ref_vq is None:
-        pytest.skip("/root/reference not present")
+        pytest.skip("no reference checkout (VQSEG_REF)")
     x = torch.relu(torch.randn(2, 200, 32))
     torch.manual_seed(11); m1, b1 = ref_vq.kmeans(x, 16, 5)
     torch.manual_seed(11); m2, b2 = O.kmeans(x, 16, 5)
@@ -89,7 +101,7 @@ def test_live_reference_kmeans_same_rng(ref_vq):
 
 def test_live_reference_kmeans_init_module(ref_vq):
     if ref_vq is None:
-        pytest.skip("/root/reference not present")
+        pytest.skip("no reference checkout (VQSEG_REF)")
     ref = ref_vq.VectorQuantizer(dim=32, num_embeddings=20, kmeans_init=True)
     port = O.OracleVectorQuantizer(dim=32, num_embeddings=20, kmeans_init=True)
     x = torch.relu(torch.randn(2, 32, 12, 12))
@@ -102,9 +114,7 @@ def test_live_reference_kmeans_init_module(ref_vq):
     assert ref.codebook.initted and port.codebook.initted
 
 
-def test_live_reference_cosine(ref_vq, golden):
-    if ref_vq is None:
-        pytest.skip("/root/reference not present")
+def test_live_reference_cosine(golden, golden_threads):
     for name, build in cases.COSINE_CASES.items():
         x, e = build()
         port = O.OracleVectorQuantizer(dim=x.shape[1], num_embeddings=e.shape[0], distance="cosine")
@@ -130,7 +140,7 @@ def test_make_vq_module_port():
 
 
 @pytest.mark.parametrize("name", list(cases.SEGHEAD_CASES))
-def test_seghead_oracle_matches_golden(golden_seghead, name):
+def test_seghead_oracle_matches_golden(golden_seghead, golden_threads, name):
     """The restated segmentation head (oracle/seghead_oracle.py) against the live reference's outputs and
     gradients: same torch build -> bit-equal."""
     from oracle.seghead_oracle import OracleVQSegmentationHead
@@ -165,7 +175,7 @@ def test_live_reference_seghead_kmeans_init():
     from oracle.seghead_oracle import OracleVQSegmentationHead
     R = load_reference_seghead()
     if R is None:
-        pytest.skip("/root/reference not present (GPU box): golden vectors are the pin there")
+        pytest.skip("no reference checkout (VQSEG_REF): golden vectors are the pin")
     x, _ = cases.SEGHEAD_CASES["sh_c3_d32"][0]()
     for distance in ("euclidean", "cosine"):
         torch.manual_seed(5)
