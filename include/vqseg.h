@@ -217,7 +217,8 @@ int    vqseg_ema_update_f32(const int64_t* counts, const float* sums, float* clu
  *   cosine != 0: einsum('n d, e d -> n e') over rows the caller has already l2-normalised
  *                (CosinesimSegHead.forward :104); idx = first argmax (:107).
  * counts_out (nullable) = bincount(idx, K) (:174), zeroed by the call.  K <= 32, D <= 382, K*D small enough for
- * shared memory (VQSEG_EUNSUPPORTED otherwise: a segmentation head has K = classes, D = last decoder width).
+ * shared memory (VQSEG_EUNSUPPORTED otherwise: a segmentation head has K = classes, D = last decoder width;
+ * vqseg_seghead_map_f32 below takes any K and D).
  * score_out (nullable, Euclidean only, same strides): the wrapper's class scores softmax_k(1 - d_k / sum_j d_j)
  * (VQSegmentationHead.forward :243-247 with the default nn.Softmax2d activation), written by the same kernel.  */
 int    vqseg_dist_map_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
@@ -242,6 +243,34 @@ int    vqseg_sim_map_bwd_f32(const float* g, int64_t oB, int64_t oP, int64_t oK,
                              int64_t sB, int64_t sP, int64_t sD,
                              const float* E, int64_t K,
                              float* gx_out, int64_t gxB, int64_t gxP, int64_t gxD, float* gE_out, void* stream);
+
+/* ---- segmentation head for any class count and feature width ------------------------------------------------
+ * Same outputs and arithmetic as vqseg_dist_map_f32 (Euclidean map bit-equal to ATen's CPU cdist, including MKL's
+ * K-blocked chains for D + 2 > 384; cosine: the plain D-term chain over caller-normalised rows) for any K >= 1 and
+ * D >= 1.  `algo` picks the kernel:
+ *   VQSEG_SEGHEAD_AUTO  : the per-pixel kernels of vqseg_dist_map_f32 where their limits hold (K <= 32, D <= 382:
+ *                         the reference's 3-class heads), the tiled kernels otherwise;
+ *   VQSEG_SEGHEAD_PIXEL : the per-pixel kernels only (VQSEG_EUNSUPPORTED beyond their limits);
+ *   VQSEG_SEGHEAD_TILED : the register-tiled kernels (a block owns 128 pixels x 64 classes per step).
+ * No workspace; counts_out (nullable) is zeroed by the call.                                                      */
+#define VQSEG_SEGHEAD_AUTO   0
+#define VQSEG_SEGHEAD_PIXEL  1
+#define VQSEG_SEGHEAD_TILED  2
+int    vqseg_seghead_map_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
+                             const float* E, int64_t K, int cosine,
+                             float* dist_out, int64_t oB, int64_t oP, int64_t oK,
+                             int64_t* idx_out, int64_t* counts_out, float* score_out, int algo, void* stream);
+/* backward of vqseg_seghead_map_f32.  cosine == 0: as vqseg_dist_map_bwd_f32 (`map` = the distance map, `score`
+ * nullable); cosine != 0: as vqseg_sim_map_bwd_f32 with `map` = the similarity map (the tiled kernels take
+ * <xn, gxn> = sum_k g_k sim_k from it), score must be null.  g and map share strides; gE_out is zeroed by the call
+ * and accumulated with fp32 atomics.  ws must hold vqseg_seghead_map_bwd_workspace_bytes (16 bytes per pixel for
+ * the tiled kernels, 0 for the per-pixel ones).                                                                   */
+size_t vqseg_seghead_map_bwd_workspace_bytes(int64_t n_rows, int64_t D, int64_t K, int algo);
+int    vqseg_seghead_map_bwd_f32(const float* g, const float* map, int64_t oB, int64_t oP, int64_t oK,
+                                 const float* x, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
+                                 const float* E, int64_t K, int cosine, const float* score,
+                                 float* gx_out, int64_t gxB, int64_t gxP, int64_t gxD, float* gE_out,
+                                 int algo, void* ws, size_t ws_bytes, void* stream);
 
 
 #ifdef __cplusplus

@@ -45,6 +45,10 @@ SIGNATURES = {
     "vqseg_dist_map_bwd_f32": (ci, [vp, vp, i64, i64, i64, vp, i64, i64, i64, i64, i64, i64, vp, i64,
                                     vp, i64, i64, i64, vp, vp, vp]),
     "vqseg_sim_map_bwd_f32": (ci, [vp, i64, i64, i64, vp, i64, i64, i64, i64, i64, i64, vp, i64, vp, i64, i64, i64, vp, vp]),
+    "vqseg_seghead_map_f32": (ci, [vp, i64, i64, i64, i64, i64, i64, vp, i64, ci, vp, i64, i64, i64, vp, vp, vp, ci, vp]),
+    "vqseg_seghead_map_bwd_workspace_bytes": (sz, [i64, i64, i64, ci]),
+    "vqseg_seghead_map_bwd_f32": (ci, [vp, vp, i64, i64, i64, vp, i64, i64, i64, i64, i64, i64, vp, i64, ci, vp,
+                                       vp, i64, i64, i64, vp, ci, vp, sz, vp]),
 }
 
 

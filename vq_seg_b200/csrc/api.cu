@@ -75,14 +75,6 @@ __global__ void __launch_bounds__(256) assign_prologue_kernel(unsigned long long
   if (threadIdx.x == 0) { hdr->ticket = 0u; hdr->stale = 0u; if (stale) hdr->rebuilds += 1u; }
 }
 
-// MKL's sgemm K-blocking as probed on the reference CPU path (DESIGN.md §parity): one chain up to
-// 384 terms, two halves up to 768, 384-blocks beyond.
-static int auto_kblock(long long L) {
-  if (L <= 384) return 0;
-  if (L <= 768) return (int)((L + 1) / 2);
-  return 384;
-}
-
 #ifdef VQSEG_DEV
 long long* g_dev_trace = nullptr;            // developer build only (libvqseg_dev.so): clock stamps of the pipeline roles
 #endif

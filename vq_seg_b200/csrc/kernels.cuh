@@ -116,4 +116,24 @@ int tc4_layout(const Rows& x, long long K_pad, int n_dc);   // 0: unsupported, 1
 int launch_assign_tc4(const Rows& x, const Tc4Args& a, int layout, cudaStream_t st);    // layout 3: prepared samples
 int launch_samples_prepare(const Rows& x, long long rows_padded, int D_pad, unsigned char* img, float2* norms, cudaStream_t st);
 
+// MKL's sgemm K-blocking as probed on the reference CPU path (DESIGN.md §parity): one chain up to
+// 384 terms, two halves up to 768, 384-blocks beyond.  0: one chain.
+inline int auto_kblock(long long L) {
+  if (L <= 384) return 0;
+  if (L <= 768) return (int)((L + 1) / 2);
+  return 384;
+}
+
+// ---- seghead_tiled.cu: register-tiled map and backward of the segmentation head (any K, any D)
+// kb: the chain's K-block, normalised (0 < kb <= D + 2, or <= D for cosine).  Outputs as in vqseg_seghead_map_f32;
+// counts must be zeroed by the caller.
+int launch_seghead_map_tiled(const Rows& x, const float* E, int K, bool cosine, int kb, float* dist, long long oB,
+                             long long oP, long long oK, long long* idx, unsigned long long* counts, float* score,
+                             cudaStream_t st);
+size_t seghead_bwd_tiled_workspace_bytes(long long n_rows);
+// gE must be zeroed by the caller; cosine: dist is the similarity map
+int launch_seghead_map_bwd_tiled(const Rows& x, const float* E, int K, bool cosine, const float* g, const float* dist,
+                                 long long oB, long long oP, long long oK, const float* score, const RowsOut& gx,
+                                 float* gE, void* ws, cudaStream_t st);
+
 }  // namespace vqseg

@@ -14,6 +14,7 @@
 // form of ATen's _euclidean_dist, |.|^2 in ATen's CPU summation order -- bit-equal to the CPU reference.
 // Limits (loud errors beyond): K <= 32, D + 2 <= 384 (single-chain regime of the CPU GEMM), K*D*4 <= 96 KiB.
 #include "common.cuh"
+#include "kernels.cuh"
 
 namespace vqseg {
 
@@ -442,6 +443,71 @@ int vqseg_sim_map_bwd_f32(const float* g, int64_t oB, int64_t oP, int64_t oK,
   if (K <= 8) return launch_dm_bwd<8>(xr, E, (int)K, g, g, oB, oP, oK, gx, gE_out, nullptr, st, 1);
   if (K <= 16) return launch_dm_bwd<16>(xr, E, (int)K, g, g, oB, oP, oK, gx, gE_out, nullptr, st, 1);
   return launch_dm_bwd<32>(xr, E, (int)K, g, g, oB, oP, oK, gx, gE_out, nullptr, st, 1);
+}
+
+// -1: bad algo, 0: per-pixel kernels, 1: tiled kernels, VQSEG_EUNSUPPORTED: per-pixel forced beyond its limits
+static int seghead_kernel(int64_t K, int64_t D, int algo) {
+  if (algo == VQSEG_SEGHEAD_AUTO) return dm_supported(K, D) ? 0 : 1;
+  if (algo == VQSEG_SEGHEAD_PIXEL) return dm_supported(K, D) ? 0 : VQSEG_EUNSUPPORTED;
+  if (algo == VQSEG_SEGHEAD_TILED) return 1;
+  return -1;
+}
+
+int vqseg_seghead_map_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
+                          const float* E, int64_t K, int cosine,
+                          float* dist_out, int64_t oB, int64_t oP, int64_t oK,
+                          int64_t* idx_out, int64_t* counts_out, float* score_out, int algo, void* stream) {
+  if (!x || !E || !dist_out || B < 0 || P < 0 || K < 1 || D < 1 || K > INT32_MAX || D > INT32_MAX ||
+      (cosine && score_out))
+    return VQSEG_EINVAL;
+  const int which = seghead_kernel(K, D, algo);
+  if (which < 0) return which == -1 ? VQSEG_EINVAL : which;
+  if (which == 0)
+    return vqseg_dist_map_f32(x, B, P, D, sB, sP, sD, E, K, cosine, dist_out, oB, oP, oK, idx_out, counts_out, score_out, stream);
+  int rc = check_arch();
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (counts_out) {
+    cudaError_t e = cudaMemsetAsync(counts_out, 0, (size_t)K * sizeof(int64_t), st);
+    if (e != cudaSuccess) return (int)e;
+  }
+  if (B * P == 0) return 0;
+  Rows xr{x, B, P, D, sB, sP, sD};
+  const long long L = cosine ? D : D + 2;
+  const int kb = auto_kblock(L) > 0 ? auto_kblock(L) : (int)L;
+  return launch_seghead_map_tiled(xr, E, (int)K, cosine != 0, kb, dist_out, oB, oP, oK, (long long*)idx_out,
+                                  (unsigned long long*)counts_out, score_out, st);
+}
+
+size_t vqseg_seghead_map_bwd_workspace_bytes(int64_t n_rows, int64_t D, int64_t K, int algo) {
+  return seghead_kernel(K, D, algo) == 1 && n_rows > 0 ? seghead_bwd_tiled_workspace_bytes(n_rows) : 0;
+}
+
+int vqseg_seghead_map_bwd_f32(const float* g, const float* map, int64_t oB, int64_t oP, int64_t oK,
+                              const float* x, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
+                              const float* E, int64_t K, int cosine, const float* score,
+                              float* gx_out, int64_t gxB, int64_t gxP, int64_t gxD, float* gE_out,
+                              int algo, void* ws, size_t ws_bytes, void* stream) {
+  if (!g || !map || !x || !E || !gx_out || !gE_out || B < 0 || P < 0 || K < 1 || D < 1 || K > INT32_MAX ||
+      D > INT32_MAX || (cosine && score))
+    return VQSEG_EINVAL;
+  const int which = seghead_kernel(K, D, algo);
+  if (which < 0) return which == -1 ? VQSEG_EINVAL : which;
+  if (which == 0) {
+    if (cosine) return vqseg_sim_map_bwd_f32(g, oB, oP, oK, x, B, P, D, sB, sP, sD, E, K, gx_out, gxB, gxP, gxD, gE_out, stream);
+    return vqseg_dist_map_bwd_f32(g, map, oB, oP, oK, x, B, P, D, sB, sP, sD, E, K, gx_out, gxB, gxP, gxD, gE_out,
+                                  score, stream);
+  }
+  if (ws_bytes < vqseg_seghead_map_bwd_workspace_bytes(B * P, D, K, algo) || (B * P > 0 && !ws)) return VQSEG_EWORKSPACE;
+  int rc = check_arch();
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMemsetAsync(gE_out, 0, (size_t)K * D * sizeof(float), st);
+  if (e != cudaSuccess) return (int)e;
+  if (B * P == 0) return 0;
+  Rows xr{x, B, P, D, sB, sP, sD};
+  RowsOut gx{gx_out, B, P, D, gxB, gxP, gxD};
+  return launch_seghead_map_bwd_tiled(xr, E, (int)K, cosine != 0, g, map, oB, oP, oK, score, gx, gE_out, ws, st);
 }
 
 }  // extern "C"

@@ -599,13 +599,132 @@ def _(grad, dist, x, codebook, score=None):
             codebook.new_empty(codebook.shape, dtype=torch.float32))
 
 
+# the head for any class count and width: vqseg_seghead_map_f32 picks the per-pixel kernels above where they apply
+# (SEGHEAD_AUTO) and the register-tiled ones otherwise; PIXEL / TILED force one of them
+SEGHEAD_AUTO, SEGHEAD_PIXEL, SEGHEAD_TILED = 0, 1, 2
+
+
+def _seghead_map_raw(x, codebook, cosine=False, with_score=False, algo=SEGHEAD_AUTO):
+    _require_cuda(x, codebook)
+    L = _native.lib()
+    if x.dtype != torch.float32:
+        x = x.float()
+    cb = codebook.detach()
+    if cb.dtype != torch.float32 or not cb.is_contiguous():
+        cb = cb.contiguous().float()
+    b, p, d, sb, sp, sd = _bpd(x)
+    k = cb.shape[0]
+    if cb.shape[1] != d:
+        raise RuntimeError(f"X1 and X2 must have the same number of columns. X1: {d} X2: {cb.shape[1]}")
+    dev = x.device
+    dist = torch.empty_strided((b, p, k), (k * p, 1, p), dtype=torch.float32, device=dev)
+    idx = torch.empty((b, p), dtype=torch.int64, device=dev)
+    counts = torch.empty(k, dtype=torch.int64, device=dev)
+    score = torch.empty_strided((b, p, k), (k * p, 1, p), dtype=torch.float32, device=dev) if with_score else None
+    with torch.cuda.device(dev):
+        _native.check(L.vqseg_seghead_map_f32(x.data_ptr(), b, p, d, sb, sp, sd, cb.data_ptr(), k, 1 if cosine else 0,
+                                              dist.data_ptr(), dist.stride(0), dist.stride(1), dist.stride(2),
+                                              idx.data_ptr(), counts.data_ptr(),
+                                              score.data_ptr() if with_score else None, algo, _stream()), "seghead_map")
+    return dist, idx, counts, score
+
+
+def _seghead_map_impl(x: torch.Tensor, codebook: torch.Tensor, cosine: bool = False,
+                      algo: int = SEGHEAD_AUTO) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """(map (B, P, K) laid out as (B, K, P), idx (B, P), counts (K,)) for any K and D: the Euclidean distance map
+    (bit-equal to ATen's CPU cdist) + first argmin, or, with cosine=True, the similarity map of rows the caller has
+    already l2-normalised + first argmax."""
+    return _seghead_map_raw(x, codebook, cosine, False, algo)[:3]
+
+
+seghead_map = torch.library.custom_op("vqseg::seghead_map", mutates_args=())(_seghead_map_impl)
+
+
+@seghead_map.register_fake
+def _(x, codebook, cosine=False, algo=SEGHEAD_AUTO):
+    b, p, d = x.shape
+    k = codebook.shape[0]
+    return (torch.empty_strided((b, p, k), (k * p, 1, p), dtype=torch.float32, device=x.device),
+            x.new_empty((b, p), dtype=torch.int64), x.new_empty((k,), dtype=torch.int64))
+
+
+def _seghead_score_map_impl(x: torch.Tensor, codebook: torch.Tensor,
+                            algo: int = SEGHEAD_AUTO) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Euclidean map plus the class scores softmax_k(1 - d_k / sum_j d_j) from the same launch, for any K and D:
+    (dist, score, idx, counts)."""
+    dist, idx, counts, score = _seghead_map_raw(x, codebook, False, True, algo)
+    return dist, score, idx, counts
+
+
+seghead_score_map = torch.library.custom_op("vqseg::seghead_score_map", mutates_args=())(_seghead_score_map_impl)
+
+
+@seghead_score_map.register_fake
+def _(x, codebook, algo=SEGHEAD_AUTO):
+    b, p, d = x.shape
+    k = codebook.shape[0]
+    mk = lambda: torch.empty_strided((b, p, k), (k * p, 1, p), dtype=torch.float32, device=x.device)  # noqa: E731
+    return mk(), mk(), x.new_empty((b, p), dtype=torch.int64), x.new_empty((k,), dtype=torch.int64)
+
+
+def _seghead_map_bwd_impl(grad: torch.Tensor, dist: torch.Tensor, x: torch.Tensor, codebook: torch.Tensor,
+                          cosine: bool = False, score: Optional[torch.Tensor] = None,
+                          algo: int = SEGHEAD_AUTO) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Backward of seghead_map / seghead_score_map: (gx with x's (B, P, D) shape in NCHW memory order, gE (K, D)).
+    `dist` is the saved map (the similarity map when cosine=True); with `score` (Euclidean only) `grad` is the
+    gradient w.r.t. the class scores."""
+    _require_cuda(grad, dist, x, codebook, score)
+    L = _native.lib()
+    if x.dtype != torch.float32:
+        x = x.float()
+    cb = codebook.detach()
+    if cb.dtype != torch.float32 or not cb.is_contiguous():
+        cb = cb.contiguous().float()
+    b, p, d, sb, sp, sd = _bpd(x)
+    k = cb.shape[0]
+    g = grad.float()
+    if g.stride() != dist.stride():
+        g2 = torch.empty_strided(dist.shape, dist.stride(), dtype=torch.float32, device=dist.device)
+        g2.copy_(g)
+        g = g2
+    gx = torch.empty_strided((b, p, d), (d * p, 1, p), dtype=torch.float32, device=x.device)
+    ge = torch.empty((k, d), dtype=torch.float32, device=x.device)
+    nws = L.vqseg_seghead_map_bwd_workspace_bytes(b * p, d, k, algo)
+    ws = torch.empty(nws, dtype=torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        _native.check(L.vqseg_seghead_map_bwd_f32(g.data_ptr(), dist.data_ptr(), dist.stride(0), dist.stride(1),
+                                                  dist.stride(2), x.data_ptr(), b, p, d, sb, sp, sd, cb.data_ptr(), k,
+                                                  1 if cosine else 0, score.data_ptr() if score is not None else None,
+                                                  gx.data_ptr(), gx.stride(0), gx.stride(1), gx.stride(2), ge.data_ptr(),
+                                                  algo, ws.data_ptr() if nws else None, nws, _stream()), "seghead_map_bwd")
+    return gx, ge
+
+
+seghead_map_bwd = torch.library.custom_op("vqseg::seghead_map_bwd", mutates_args=())(_seghead_map_bwd_impl)
+
+
+@seghead_map_bwd.register_fake
+def _(grad, dist, x, codebook, cosine=False, score=None, algo=SEGHEAD_AUTO):
+    b, p, d = x.shape
+    return (torch.empty_strided((b, p, d), (d * p, 1, p), dtype=torch.float32, device=x.device),
+            codebook.new_empty(codebook.shape, dtype=torch.float32))
+
+
+def fast_seghead_map(x, codebook, cosine=False, algo=SEGHEAD_AUTO):
+    return (_seghead_map_impl if _fast() else seghead_map)(x, codebook, cosine, algo)
+
+
+def fast_seghead_map_bwd(grad, dist, x, codebook, cosine=False, score=None, algo=SEGHEAD_AUTO):
+    return (_seghead_map_bwd_impl if _fast() else seghead_map_bwd)(grad, dist, x, codebook, cosine, score, algo)
+
+
 class _EuclideanDistMap(torch.autograd.Function):
     """torch.cdist(x, weight, p=2) + argmin + bincount with the map as a differentiable output
     (vq_segmentation_head.py:167-174): gradients to the features AND to the prototypes."""
 
     @staticmethod
     def forward(ctx, x, weight):
-        dist, idx, counts = (_dist_map_impl if _fast() else dist_map)(x, weight, False)
+        dist, idx, counts = fast_seghead_map(x, weight, False)
         ctx.save_for_backward(x, weight, dist)
         ctx.mark_non_differentiable(idx, counts)
         return dist, idx, counts
@@ -613,7 +732,7 @@ class _EuclideanDistMap(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_dist, g_idx, g_counts):
         x, weight, dist = ctx.saved_tensors
-        gx, ge = (_dist_map_bwd_impl if _fast() else dist_map_bwd)(g_dist, dist, x, weight)
+        gx, ge = fast_seghead_map_bwd(g_dist, dist, x, weight)
         return (gx if ctx.needs_input_grad[0] else None), (ge if ctx.needs_input_grad[1] else None)
 
 
@@ -627,7 +746,7 @@ class _EuclideanScoreMap(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, weight):
-        dist, score, idx, counts = (_dist_score_map_impl if _fast() else dist_score_map)(x, weight)
+        dist, score, idx, counts = (_seghead_score_map_impl if _fast() else seghead_score_map)(x, weight)
         ctx.save_for_backward(x, weight, dist, score)
         ctx.mark_non_differentiable(idx, counts)
         return score, idx, counts
@@ -635,7 +754,7 @@ class _EuclideanScoreMap(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_score, g_idx, g_counts):
         x, weight, dist, score = ctx.saved_tensors
-        gx, ge = (_dist_map_bwd_impl if _fast() else dist_map_bwd)(g_score, dist, x, weight, score)
+        gx, ge = fast_seghead_map_bwd(g_score, dist, x, weight, False, score)
         return (gx if ctx.needs_input_grad[0] else None), (ge if ctx.needs_input_grad[1] else None)
 
 

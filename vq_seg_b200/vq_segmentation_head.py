@@ -7,9 +7,10 @@ the K class prototypes is an OUTPUT (`score = activation(1 - d / sum_k d)`) and 
 to the prototypes.
 
 Euclidean: one kernel writes the exact fp32 distance map in the (B,K,H,W) score layout together with the argmin
-and the class counts (csrc/seghead.cu, bit-equal to ATen's CPU cdist); its backward is one kernel too.  Cosine: the
-rows are l2-normalised by the existing kernel, the same map kernel evaluates the similarities; the backward of that
-rarely used variant is composed from torch ops.  GPU only: there is no CPU fallback.
+and the class counts (bit-equal to ATen's CPU cdist); its backward is one kernel too.  Cosine: the rows are
+l2-normalised by the existing kernel, the same map kernel evaluates the similarities.  Any number of classes and any
+width: the per-pixel kernels (csrc/seghead.cu) serve small heads, the register-tiled ones (csrc/seghead_tiled.cu) the
+rest, chosen in C (vqseg_seghead_map_f32).  GPU only: there is no CPU fallback.
 """
 import torch
 import torch.nn.functional as F
@@ -70,12 +71,12 @@ class EuclideanSegHead(_SegHeadBase):
 class _CosineMap(torch.autograd.Function):
     """similarity = l2norm(x) @ weight^T with weight already unit-norm (:97-104); gradient through the
     normalisation to x and directly to the weight (the reference renormalises weight.data in place).  Forward: the
-    map kernel normalises on the fly; backward: one kernel (vqseg_sim_map_bwd_f32)."""
+    map kernel on the normalised rows; backward: vqseg_seghead_map_bwd_f32 in cosine mode."""
 
     @staticmethod
     def forward(ctx, x, weight):
         xn = ops.l2norm_rows(x)
-        sim, idx, counts = (ops._dist_map_impl if ops._fast() else ops.dist_map)(xn, weight, True)
+        sim, idx, counts = ops.fast_seghead_map(xn, weight, True)
         ctx.save_for_backward(x, sim, weight)
         ctx.mark_non_differentiable(idx, counts)
         return sim, idx, counts
@@ -83,7 +84,7 @@ class _CosineMap(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g, g_idx, g_counts):
         x, sim, weight = ctx.saved_tensors
-        gx, gw = (ops._sim_map_bwd_impl if ops._fast() else ops.sim_map_bwd)(g, sim, x, weight)
+        gx, gw = ops.fast_seghead_map_bwd(g, sim, x, weight, True)
         return (gx if ctx.needs_input_grad[0] else None), (gw if ctx.needs_input_grad[1] else None)
 
 
