@@ -191,10 +191,12 @@ int    vqseg_gather_rows_f32(const float* x, int64_t B, int64_t P, int64_t D,
 
 /* ---- cosine codebook helper (CosinesimCodebook, vq_img.py:93-107) -----------------------------
  * out[b,p,:] = x[b,p,:] / max(|x[b,p,:]|, 1e-12)  (F.normalize, vq_img.py:7-8,:97,:100,:54) in ATen's CPU
- * arithmetic: a contiguous last dim (sD == 1: code rows, k-means means) is reduced in ATen's vectorised last-dim order,
- * a strided one (the 'b c h w -> b (h w) c' view the cosine codebook normalises) as one sequential chain; IEEE sqrt
- * and division.  `out` may have any strides (same layout as x keeps NCHW maps TMA-loadable) and may alias x when the
- * strides are equal (in-place renormalisation of the codebook, vq_img.py:100).
+ * arithmetic, whose summation order follows the stride of x's reduced dim alone: sD == 1 (code rows, k-means means,
+ * channels-last maps and their batch slices, 1 x 1 maps) is reduced in ATen's vectorised last-dim order, any other sD
+ * (the 'b c h w -> b (h w) c' view of an NCHW map the cosine codebook normalises) as one sequential chain; IEEE sqrt
+ * and division.  Any sB and sP are accepted.  `out` may have any strides, which do not change the order (same layout
+ * as x keeps NCHW maps TMA-loadable), and may alias x when the strides are equal (in-place renormalisation of the
+ * codebook, vq_img.py:100).
  * The lookup itself (einsum + argmax, vq_img.py:104-107) is vqseg_assign_f32 with VQSEG_METRIC_IP. */
 int    vqseg_l2norm_f32(const float* x, int64_t B, int64_t P, int64_t D,
                         int64_t sB, int64_t sP, int64_t sD,

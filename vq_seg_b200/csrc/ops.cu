@@ -883,25 +883,27 @@ __global__ void __launch_bounds__(256) unpack_keys_kernel(const unsigned long lo
 }
 
 // ---- F.normalize(t, p=2, dim=-1) = t / max(||t||, 1e-12) in ATen's CPU arithmetic (vq_img.py:7-8) --------------------
-// Probed on the reference's CPU path (torch 2.11, tests/golden/make_golden_cosine.py pins it):
-//  * the norm of a CONTIGUOUS last dim (code rows, k-means means) is ATen's vectorised last-dim reduction: eight lane
-//    accumulators a_l += fl(v * v) over elements l, l + 8, ..., summed a_0 + a_1 + ... + a_7 in order, then the
-//    D % 8 tail: four separately rounded fl(v * v) adds if at least four remain, fused multiply-adds for the last <= 3;
-//  * the norm over a STRIDED dim (the 'b c h w -> b (h w) c' view of vq_img.py:232, which is what the cosine codebook
+// Probed on the reference's CPU path (torch 2.11, tests/golden/make_golden_cosine.py and tests/test_layout_rules.py
+// pin it).  ATen picks the order by the stride of the reduced dim ALONE, whatever sB, sP and the output's strides are:
+//  * sD == 1 (code rows, k-means means, channels-last maps and their batch slices, 1 x 1 maps): ATen's vectorised
+//    last-dim reduction: eight lane accumulators a_l += fl(v * v) over elements l, l + 8, ..., summed
+//    a_0 + a_1 + ... + a_7 in order, then the D % 8 tail: four separately rounded fl(v * v) adds if at least four
+//    remain, fused multiply-adds for the last <= 3;
+//  * any other sD (the 'b c h w -> b (h w) c' view of an NCHW map, vq_img.py:232, which is what the cosine codebook
 //    normalises, :97) is one sequential chain acc = fl(acc + fl(v * v)) in channel order;
 //  * sqrt and the division are IEEE round-to-nearest.
-// Eight lanes own a contiguous row (lane l = accumulator l); one thread owns a strided row (pixel-contiguous maps:
+// Eight lanes own a row with sD == 1 (lane l = accumulator l); one thread owns a strided row (pixel-contiguous maps:
 // a warp reads 32 neighbouring pixels of one channel).
-__global__ void __launch_bounds__(256) l2norm_lastdim_kernel(const float* __restrict__ x, long long n_rows, int D,
-                                                             long long row_stride, float* __restrict__ out, long long out_stride) {
+__global__ void __launch_bounds__(256) l2norm_lastdim_kernel(Rows x, RowsOut out) {
   const int l8 = threadIdx.x & 7;
   const long long n = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 3;
-  const bool on = n < n_rows;                            // (whole groups of 8 lanes are on or off together)
-  const float* row = x + (on ? n : 0) * row_stride;
+  const bool on = n < x.n_rows();                        // (whole groups of 8 lanes are on or off together)
+  const int D = (int)x.D;
+  const float* row = x.row(on ? n : 0);
   const float nrm = fmaxf(aten_norm_lastdim8(row, on ? D : 0, l8), 1e-12f);
   if (!on) return;
-  float* o = out + n * out_stride;
-  for (int d = l8; d < D; d += 8) o[d] = __fdiv_rn(row[d], nrm);       // in place is fine: each element is read by its writer
+  float* o = out.row(n);
+  for (int d = l8; d < D; d += 8) o[(long long)d * out.sD] = __fdiv_rn(row[d], nrm);   // in place is fine: each element is read by its writer
 }
 
 // pixel-contiguous maps (sP == 1): a block owns 32 neighbouring pixels of one image.  All eight warps stage 256
@@ -1409,13 +1411,12 @@ int vqseg_l2norm_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_t sB
   if (!x || !out || D <= 0 || B < 0 || P < 0 || D >= (1ll << 31)) return VQSEG_EINVAL;
   if (B * P == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
-  if (sD == 1 && oD == 1 && (B == 1 || (sB == P * sP && oB == P * oP))) {
-    // contiguous last dim, one flat row range: ATen's vectorised last-dim reduction
-    const long long n = B * P;
-    l2norm_lastdim_kernel<<<(unsigned)((n * 8 + 255) / 256), 256, 0, st>>>(x, n, (int)D, sP, out, oP);
+  Rows xr{x, B, P, D, sB, sP, sD};
+  RowsOut orow{out, B, P, D, oB, oP, oD};
+  if (sD == 1 || D == 1) {
+    // the order follows x's reduced dim only (see the kernels above); one term needs no order
+    l2norm_lastdim_kernel<<<(unsigned)((B * P * 8 + 255) / 256), 256, 0, st>>>(xr, orow);
   } else {
-    Rows xr{x, B, P, D, sB, sP, sD};
-    RowsOut orow{out, B, P, D, oB, oP, oD};
     if (sP == 1) {
       const long long groups = B * ((P + 31) / 32), cap = (long long)num_sms() * 16;
       static bool carved[kMaxDevices] = {false};        // 32 KB of static shared memory per block: ask for the large carve-out
