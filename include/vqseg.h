@@ -229,7 +229,8 @@ int    vqseg_dist_map_f32(const float* x, int64_t B, int64_t P, int64_t D, int64
                           int64_t* idx_out, int64_t* counts_out, float* score_out, void* stream);
 /* backward of the Euclidean map (autograd of torch.cdist, p=2): with w = g / dist (0 where dist == 0),
  *   gx[n,:] = sum_k w[n,k] (x[n,:] - e_k),   gE[k,:] = sum_n w[n,k] (e_k - x[n,:])   (gE zeroed by the call;
- * accumulated with fp32 atomics: sums within 1e-5 relative, not bit-reproducible).  g and dist share strides.
+ * accumulated with fp32 atomics: sums within 1e-5 relative, not bit-reproducible -- vqseg_seghead_map_bwd_f32 with
+ * VQSEG_SEGHEAD_DETERMINISTIC is).  g and dist share strides.
  * score (nullable): when given, g is the gradient w.r.t. score_out and the kernel first chains it through the
  * softmax and the 1 - d / sum(d) normalisation.                                                           */
 int    vqseg_dist_map_bwd_f32(const float* g, const float* dist, int64_t oB, int64_t oP, int64_t oK,
@@ -258,15 +259,24 @@ int    vqseg_sim_map_bwd_f32(const float* g, int64_t oB, int64_t oP, int64_t oK,
 #define VQSEG_SEGHEAD_AUTO   0
 #define VQSEG_SEGHEAD_PIXEL  1
 #define VQSEG_SEGHEAD_TILED  2
+/* OR into the algo of vqseg_seghead_map_bwd_workspace_bytes / vqseg_seghead_map_bwd_f32 (the forward map rejects it
+ * with VQSEG_EINVAL): gE bit-reproducible, see below.                                                             */
+#define VQSEG_SEGHEAD_DETERMINISTIC 0x100
 int    vqseg_seghead_map_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
                              const float* E, int64_t K, int cosine,
                              float* dist_out, int64_t oB, int64_t oP, int64_t oK,
                              int64_t* idx_out, int64_t* counts_out, float* score_out, int algo, void* stream);
 /* backward of vqseg_seghead_map_f32.  cosine == 0: as vqseg_dist_map_bwd_f32 (`map` = the distance map, `score`
  * nullable); cosine != 0: as vqseg_sim_map_bwd_f32 with `map` = the similarity map (the tiled kernels take
- * <xn, gxn> = sum_k g_k sim_k from it), score must be null.  g and map share strides; gE_out is zeroed by the call
- * and accumulated with fp32 atomics.  ws must hold vqseg_seghead_map_bwd_workspace_bytes (16 bytes per pixel for
- * the tiled kernels, 0 for the per-pixel ones).                                                                   */
+ * <xn, gxn> = sum_k g_k sim_k from it), score must be null.  g and map share strides.  ws must hold
+ * vqseg_seghead_map_bwd_workspace_bytes of the same algo.
+ * Without VQSEG_SEGHEAD_DETERMINISTIC gE_out is zeroed by the call and accumulated with fp32 atomics (not
+ * bit-reproducible); the workspace is 16 bytes per pixel for the tiled kernels, 0 for the per-pixel ones.
+ * With it gE_out is a function of the inputs and of (B*P, K, D) alone -- not of the device's SM count, the launch
+ * timing, the stream or the strides of x: the pixels are cut into S slices of consecutive rows (S from the shape
+ * only), each slice's (K, D) partial sum is formed in the kernel's fixed in-block order with tiles in ascending
+ * order and stored with plain stores, and the S partials are added in a fixed order that depends on S alone.  The
+ * workspace adds S*K*D*4 bytes of partials when S > 1, never more than 32 MiB.  gx is the same either way. */
 size_t vqseg_seghead_map_bwd_workspace_bytes(int64_t n_rows, int64_t D, int64_t K, int algo);
 int    vqseg_seghead_map_bwd_f32(const float* g, const float* map, int64_t oB, int64_t oP, int64_t oK,
                                  const float* x, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,

@@ -1,7 +1,8 @@
 """Times the VQ segmentation head (Euclidean + Softmax2d) on one GPU and prints one JSON line.
 
 Per shape: the module's eval forward (no_grad) and train forward + backward, the map kernel and its backward alone
-(replayed from a CUDA graph, with the FLOP rate of the 2NKD contraction each one runs), and the same head written
+(replayed from a CUDA graph, with the FLOP rate of the 2NKD contraction each one runs), the backward again with
+VQSEG_SEGHEAD_DETERMINISTIC (what the head runs under torch.use_deterministic_algorithms), and the same head written
 with torch ops on the same GPU (cdist, normalisation, Softmax2d, autograd).  The fp32 rate denominator is a cuBLAS SGEMM (8192^3, TF32 off) timed in
 the same call; the device name and power limit are read in the same call too.  CUDA events over --iters iterations
 after warm-up; the inputs are cycled through enough buffers to exceed the 126 MB L2.
@@ -133,6 +134,9 @@ def main():
         dm, sc, _, _ = ops._seghead_score_map_impl(views[0], e)
         g = torch.randn_like(sc)
         r["bwd_us"] = graphed(lambda v: ops._seghead_map_bwd_impl(g, dm, v, e, False, sc), views, args.iters, args.warmup)
+        det = ops.SEGHEAD_AUTO | ops.SEGHEAD_DETERMINISTIC
+        r["bwd_det_us"] = graphed(lambda v: ops._seghead_map_bwd_impl(g, dm, v, e, False, sc, det), views, args.iters,
+                                  args.warmup)
         r["map_tflops"] = flop / r["map_us"] / 1e6
         r["bwd_tflops"] = 2 * flop / r["bwd_us"] / 1e6          # gx and gE: two contractions of 2NKD each
         r["map_frac_of_sgemm"] = r["map_tflops"] / sgemm_tflops

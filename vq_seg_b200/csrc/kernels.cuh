@@ -130,10 +130,22 @@ inline int auto_kblock(long long L) {
 int launch_seghead_map_tiled(const Rows& x, const float* E, int K, bool cosine, int kb, float* dist, long long oB,
                              long long oP, long long oK, long long* idx, unsigned long long* counts, float* score,
                              cudaStream_t st);
-size_t seghead_bwd_tiled_workspace_bytes(long long n_rows);
-// gE must be zeroed by the caller; cosine: dist is the similarity map
+// Deterministic backward (VQSEG_SEGHEAD_DETERMINISTIC): the pixels are cut into slices of consecutive rows whose
+// number is a function of (n_rows, K, D) alone; each slice's (K, D) partial is stored with plain stores and the
+// partials are added in a fixed order (launch_seghead_slice_sum).  The split uses a B200's SM count as a constant, and
+// the partials never take more than kSegheadDetPartialBytes.
+constexpr long long kSegheadDetSms = 148;
+constexpr long long kSegheadDetPartialBytes = 32ll << 20;
+inline long long seghead_det_max_slices(long long K, long long D) {
+  const long long m = kSegheadDetPartialBytes / (K * D * (long long)sizeof(float));
+  return m > 1 ? m : 1;
+}
+size_t seghead_bwd_tiled_workspace_bytes(long long n_rows, int K, int D, bool det);
+// gE must be zeroed by the caller unless det (every element is stored); cosine: dist is the similarity map
 int launch_seghead_map_bwd_tiled(const Rows& x, const float* E, int K, bool cosine, const float* g, const float* dist,
                                  long long oB, long long oP, long long oK, const float* score, const RowsOut& gx,
-                                 float* gE, void* ws, cudaStream_t st);
+                                 float* gE, bool det, void* ws, cudaStream_t st);
+// out[i] = the sum of part[z n + i] over z < S, in an order that depends on S alone
+int launch_seghead_slice_sum(const float* part, long long n, int S, float* out, cudaStream_t st);
 
 }  // namespace vqseg

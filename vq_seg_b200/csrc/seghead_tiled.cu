@@ -9,7 +9,8 @@
 //              MKL's K-block boundaries, |x|^2 and |e|^2 entering as the last two augmented terms -- the map is an
 //              output and stays bit-equal to ATen's CPU cdist.
 //   gx       : acc[pixel][dim]  += w[pixel][class] e[class][dim], rows = classes.
-//   gE       : acc[dim][class]  += x[pixel][dim] w[pixel][class], rows = pixels (split over blocks, fp32 atomics).
+//   gE       : acc[dim][class]  += x[pixel][dim] w[pixel][class], rows = pixels (split over blocks, fp32 atomics;
+//              deterministic mode: per-split partials with plain stores, added in a fixed order by seghead_slice_sum).
 // The backward weight w (g / d, chained through the softmax and the normalisation when the class scores are
 // given) is derived on the fly from g, d, the score and four per-pixel scalars: no N x K matrix is materialised.
 #include "common.cuh"
@@ -432,7 +433,9 @@ seghead_bwd_gx_kernel(Rows x, const float* __restrict__ E, int K, const float* _
 // gE[k, :] += sum_{n in this block's pixels} w[n, k] (e_k - x[n, :])   (Euclidean)
 //          += sum_n g[n, k] xn[n, :]                                    (cosine)
 // Block tile: 128 dims x 64 classes, contraction over a range of pixels (grid.z splits the pixels), fp32 atomics.
-template <bool COSINE>
+// DET: split z stores its sum (zeros included) to gE + z K D instead: the caller's partials, or gE itself when
+// there is one split.
+template <bool COSINE, bool DET>
 __global__ void __launch_bounds__(kTThreads, 2)
 seghead_bwd_ge_kernel(Rows x, const float* __restrict__ E, int K, const float* __restrict__ g, const float* __restrict__ dist,
                       long long oB, long long oP, long long oK, const float* __restrict__ score,
@@ -510,16 +513,79 @@ seghead_bwd_ge_kernel(Rows x, const float* __restrict__ E, int K, const float* _
       if (k >= K) continue;
       const long long o = (long long)k * D + d;
       const float r = COSINE ? acc[i][j] : __ldg(E + o) * s_ws[4 * tb + j] - acc[i][j];
-      if (r != 0.f) atomicAdd(gE + o, r);
+      if (DET) gE[(long long)blockIdx.z * K * D + o] = r;
+      else if (r != 0.f) atomicAdd(gE + o, r);
     }
   }
 }
 
-size_t seghead_bwd_tiled_workspace_bytes(long long n_rows) { return (size_t)n_rows * sizeof(float4); }
+// The pixel split of the gE kernel: ~4 blocks per SM over the (dims x classes) tiles, at most `max_splits` splits.
+// (splits, chunks per split) with every split non-empty.
+static void ge_split(long long N, int K, int D, long long sms, long long max_splits, long long& splits, long long& cps) {
+  const long long tiles = (long long)((D + kTA - 1) / kTA) * ((K + kTB - 1) / kTB);
+  const long long n_chunks = (N + kTR - 1) / kTR;
+  splits = (4ll * sms + tiles - 1) / tiles;
+  if (splits > n_chunks) splits = n_chunks;
+  if (splits > 65535) splits = 65535;
+  if (splits > max_splits) splits = max_splits;
+  cps = (n_chunks + splits - 1) / splits;
+  splits = (n_chunks + cps - 1) / cps;
+}
+
+// Deterministic mode: the split is a function of the shape alone (a B200's SM count in place of the device's), and
+// the partials stay within kSegheadDetPartialBytes.
+static void ge_split_det(long long N, int K, int D, long long& splits, long long& cps) {
+  ge_split(N, K, D, kSegheadDetSms, seghead_det_max_slices(K, D), splits, cps);
+}
+
+size_t seghead_bwd_tiled_workspace_bytes(long long n_rows, int K, int D, bool det) {
+  size_t bytes = (size_t)n_rows * sizeof(float4);
+  if (det && n_rows > 0 && K > 0 && D > 0) {
+    long long splits, cps;
+    ge_split_det(n_rows, K, D, splits, cps);
+    if (splits > 1) bytes += (size_t)splits * K * D * sizeof(float);
+  }
+  return bytes;
+}
+
+// out[i] = sum_z part[z n + i] over the S slices in a fixed order that depends on S alone: group j of G = min(S, 32)
+// adds its run of consecutive slices [j R, (j + 1) R) in ascending order (R = ceil(S / G)), then the G run sums are
+// added in ascending j.  (One ascending chain of S dependent loads per element would be latency-bound when K D is
+// small and S large: the 3-class head has 96 elements and 2048 slices.)
+__global__ void seghead_slice_sum_kernel(const float* __restrict__ part, long long n, int S, int R, float* __restrict__ out) {
+  extern __shared__ float ss_run[];                       // [G][32]
+  const int e = threadIdx.x & 31, j = threadIdx.x >> 5, G = blockDim.x >> 5;
+  const long long i = (long long)blockIdx.x * 32 + e;
+  float s = 0.f;
+  if (i < n) {
+    const int z0 = j * R, z1 = min(z0 + R, S);
+    if (z0 < z1) {
+      s = part[(long long)z0 * n + i];
+#pragma unroll 8
+      for (int z = z0 + 1; z < z1; ++z) s = __fadd_rn(s, part[(long long)z * n + i]);
+    }
+  }
+  ss_run[j * 32 + e] = s;
+  __syncthreads();
+  if (j == 0 && i < n) {
+    float t = ss_run[e];
+    for (int q = 1; q < G; ++q)
+      if (q * R < S) t = __fadd_rn(t, ss_run[q * 32 + e]);
+    out[i] = t;
+  }
+}
+
+int launch_seghead_slice_sum(const float* part, long long n, int S, float* out, cudaStream_t st) {
+  const int G = S < 32 ? S : 32, R = (S + G - 1) / G;
+  const long long blocks = (n + 31) / 32;
+  seghead_slice_sum_kernel<<<(unsigned)blocks, 32 * G, (size_t)G * 32 * sizeof(float), st>>>(part, n, S, R, out);
+  VQSEG_LAUNCH_CHECK();
+  return 0;
+}
 
 int launch_seghead_map_bwd_tiled(const Rows& x, const float* E, int K, bool cosine, const float* g, const float* dist,
                                  long long oB, long long oP, long long oK, const float* score, const RowsOut& gx,
-                                 float* gE, void* ws, cudaStream_t st) {
+                                 float* gE, bool det, void* ws, cudaStream_t st) {
   const long long N = x.n_rows();
   const int D = (int)x.D;
   float4* scal = static_cast<float4*>(ws);
@@ -530,19 +596,22 @@ int launch_seghead_map_bwd_tiled(const Rows& x, const float* E, int K, bool cosi
   if (cosine) seghead_bwd_gx_kernel<true><<<ggx, kTThreads, 0, st>>>(x, E, K, g, dist, oB, oP, oK, nullptr, scal, gx);
   else seghead_bwd_gx_kernel<false><<<ggx, kTThreads, 0, st>>>(x, E, K, g, dist, oB, oP, oK, score, scal, gx);
   VQSEG_LAUNCH_CHECK();
-  // split the pixels so that ~4 blocks per SM cover the (dims x classes) tiles
-  const long long tiles = (long long)((D + kTA - 1) / kTA) * ((K + kTB - 1) / kTB);
-  const long long n_chunks = (N + kTR - 1) / kTR;
-  long long splits = (4ll * num_sms() + tiles - 1) / tiles;
-  if (splits > n_chunks) splits = n_chunks;
-  if (splits > 65535) splits = 65535;
-  const long long cps = (n_chunks + splits - 1) / splits;
-  splits = (n_chunks + cps - 1) / cps;
+  long long splits, cps;
+  if (det) ge_split_det(N, K, D, splits, cps);
+  else ge_split(N, K, D, num_sms(), 65535, splits, cps);
   const dim3 gge((unsigned)((D + kTA - 1) / kTA), (unsigned)((K + kTB - 1) / kTB), (unsigned)splits);
-  if (cosine) seghead_bwd_ge_kernel<true><<<gge, kTThreads, 0, st>>>(x, E, K, g, dist, oB, oP, oK, nullptr, scal, gE, (int)cps);
-  else seghead_bwd_ge_kernel<false><<<gge, kTThreads, 0, st>>>(x, E, K, g, dist, oB, oP, oK, score, scal, gE, (int)cps);
+  const float* sc = cosine ? nullptr : score;
+  if (!det) {
+    if (cosine) seghead_bwd_ge_kernel<true, false><<<gge, kTThreads, 0, st>>>(x, E, K, g, dist, oB, oP, oK, sc, scal, gE, (int)cps);
+    else seghead_bwd_ge_kernel<false, false><<<gge, kTThreads, 0, st>>>(x, E, K, g, dist, oB, oP, oK, sc, scal, gE, (int)cps);
+    VQSEG_LAUNCH_CHECK();
+    return 0;
+  }
+  float* part = splits > 1 ? reinterpret_cast<float*>(scal + N) : gE;
+  if (cosine) seghead_bwd_ge_kernel<true, true><<<gge, kTThreads, 0, st>>>(x, E, K, g, dist, oB, oP, oK, sc, scal, part, (int)cps);
+  else seghead_bwd_ge_kernel<false, true><<<gge, kTThreads, 0, st>>>(x, E, K, g, dist, oB, oP, oK, sc, scal, part, (int)cps);
   VQSEG_LAUNCH_CHECK();
-  return 0;
+  return splits > 1 ? launch_seghead_slice_sum(part, (long long)K * D, (int)splits, gE, st) : 0;
 }
 
 }  // namespace vqseg

@@ -298,9 +298,11 @@ def _(grad_q, idx, num_codes):
 
 
 def _code_stats_impl(x: torch.Tensor, idx: torch.Tensor, num_codes: int, deterministic: bool = True) -> Tuple[torch.Tensor, torch.Tensor]:
-    """(counts (K,) int64, sums (K, D) fp32) of the rows assigned to each code."""
+    """(counts (K,) int64, sums (K, D) fp32) of the rows assigned to each code.  The sums are ordered (ascending rows)
+    when `deterministic` is set or torch.use_deterministic_algorithms(True) is in force."""
     _require_cuda(x, idx)
     L = _native.lib()
+    deterministic = deterministic or torch.are_deterministic_algorithms_enabled()
     if x.dtype != torch.float32:
         x = x.float()
     b, p, d, sb, sp, sd = _bpd(x)
@@ -602,6 +604,7 @@ def _(grad, dist, x, codebook, score=None):
 # the head for any class count and width: vqseg_seghead_map_f32 picks the per-pixel kernels above where they apply
 # (SEGHEAD_AUTO) and the register-tiled ones otherwise; PIXEL / TILED force one of them
 SEGHEAD_AUTO, SEGHEAD_PIXEL, SEGHEAD_TILED = 0, 1, 2
+SEGHEAD_DETERMINISTIC = 0x100   # OR into the algo of seghead_map_bwd: prototype gradient in a fixed summation order
 
 
 def _seghead_map_raw(x, codebook, cosine=False, with_score=False, algo=SEGHEAD_AUTO):
@@ -715,6 +718,9 @@ def fast_seghead_map(x, codebook, cosine=False, algo=SEGHEAD_AUTO):
 
 
 def fast_seghead_map_bwd(grad, dist, x, codebook, cosine=False, score=None, algo=SEGHEAD_AUTO):
+    """seghead_map_bwd for the head's autograd functions: deterministic under torch.use_deterministic_algorithms(True)"""
+    if torch.are_deterministic_algorithms_enabled():
+        algo |= SEGHEAD_DETERMINISTIC
     return (_seghead_map_bwd_impl if _fast() else seghead_map_bwd)(grad, dist, x, codebook, cosine, score, algo)
 
 
@@ -843,6 +849,15 @@ class _StraightThrough(torch.autograd.Function):
         return gx, None, None, None
 
 
+def _codebook_grad(grad_q, idx, num_codes):
+    """gE[k] = sum of grad_q over the rows assigned to k.  Under torch.use_deterministic_algorithms(True): the ordered
+    per-code sums of code_stats (one fp32 chain per (code, dim) in ascending rows, the order of CPU index_add_)
+    instead of the atomic kernel."""
+    if torch.are_deterministic_algorithms_enabled():
+        return (_code_stats_impl if _fast() else code_stats)(grad_q, idx, num_codes, True)[1]
+    return (_gather_bwd_codebook_impl if _fast() else gather_bwd_codebook)(grad_q, idx, num_codes)
+
+
 class _EvalGather(torch.autograd.Function):
     """Eval forward: q = E[idx].  Like the reference's one_hot matmul (vq_img.py:169-170) the gradient
     goes to the codebook only."""
@@ -857,8 +872,7 @@ class _EvalGather(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_q):
         (idx,) = ctx.saved_tensors
-        ge = ((_gather_bwd_codebook_impl if _fast() else gather_bwd_codebook)(grad_q, idx, ctx.num_codes)
-              if ctx.needs_input_grad[0] else None)
+        ge = _codebook_grad(grad_q, idx, ctx.num_codes) if ctx.needs_input_grad[0] else None
         return ge, None, None, None
 
 
@@ -896,8 +910,7 @@ class _FusedEvalForward(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_q, _gi, _gm, _gu):
         (idx,) = ctx.saved_tensors
-        ge = ((_gather_bwd_codebook_impl if _fast() else gather_bwd_codebook)(grad_q, idx, ctx.num_codes)
-              if ctx.needs_input_grad[0] else None)
+        ge = _codebook_grad(grad_q, idx, ctx.num_codes) if ctx.needs_input_grad[0] else None
         return ge, None, None, None, None
 
 
