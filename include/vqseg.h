@@ -211,6 +211,23 @@ int    vqseg_ema_update_f32(const int64_t* counts, const float* sums, float* clu
                             float* embed_avg_inout, float* weight_out, int64_t K, int64_t D,
                             float decay, float eps, void* ws, void* stream);
 
+/* ---- EMA update with dead-code expiry: OPT-IN EXTENSION, no reference counterpart (threshold_ema_dead_code of
+ * lucidrains/vector-quantize-pytorch, expire_codes_ / replace).  The update of vqseg_ema_update_f32, then:
+ *   expired[k] = cluster_size[k] < threshold   (strict fp32 comparison on the cluster sizes just updated);
+ *   the r-th expired code in ascending k takes candidate row r of cand_rows ((K, D) packed: the caller samples K rows
+ *   of the batch, randperm(N)[:K] for N >= K, else randint(0, N, (K,))):
+ *     weight[k] = cand[r];  embed_avg[k] = cand[r] * reset (one fp32 multiply);  cluster_size[k] = reset.
+ * The Laplace smoothing uses n = sum(cluster_size) BEFORE any reset, so every output of a code that did not expire is
+ * bit-identical to what vqseg_ema_update_f32 writes on the same inputs.  expired_out (nullable) = int64 [last, total]:
+ * [0] is set to this call's expired count and [1] accumulates it (counters for logging without a host sync).
+ * Two launches like vqseg_ema_update_f32; K < 2^26.  ws: >= vqseg_ema_expire_workspace_bytes(K).              */
+size_t vqseg_ema_expire_workspace_bytes(int64_t K);
+int    vqseg_ema_update_expire_f32(const int64_t* counts, const float* sums, float* cluster_size_inout,
+                                   float* embed_avg_inout, float* weight_out, int64_t K, int64_t D,
+                                   float decay, float eps, float threshold, float reset,
+                                   const float* cand_rows, int64_t* expired_out,
+                                   void* ws, size_t ws_bytes, void* stream);
+
 /* ---- VQ segmentation head (models/modules/vq_segmentation_head.py) ------------------------------
  * The head classifies every decoder pixel by its distance to K class prototypes and RETURNS the distance map.
  * dist_out[b, p, k] (element strides oB, oP, oK; (K*P, 1, P) gives the (B, K, H, W) score layout directly):

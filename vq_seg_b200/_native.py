@@ -41,6 +41,8 @@ SIGNATURES = {
     "vqseg_gather_rows_f32": (ci, [vp, i64, i64, i64, i64, i64, i64, vp, i64, vp, vp]),
     "vqseg_l2norm_f32": (ci, [vp, i64, i64, i64, i64, i64, i64, vp, i64, i64, i64, vp]),
     "vqseg_ema_update_f32": (ci, [vp, vp, vp, vp, vp, i64, i64, f32, f32, vp, vp]),
+    "vqseg_ema_expire_workspace_bytes": (sz, [i64]),
+    "vqseg_ema_update_expire_f32": (ci, [vp, vp, vp, vp, vp, i64, i64, f32, f32, f32, f32, vp, vp, vp, sz, vp]),
     "vqseg_dist_map_f32": (ci, [vp, i64, i64, i64, i64, i64, i64, vp, i64, ci, vp, i64, i64, i64, vp, vp, vp, vp]),
     "vqseg_dist_map_bwd_f32": (ci, [vp, vp, i64, i64, i64, vp, i64, i64, i64, i64, i64, i64, vp, i64,
                                     vp, i64, i64, i64, vp, vp, vp]),

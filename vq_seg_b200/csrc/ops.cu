@@ -1,6 +1,8 @@
 // HBM-bound kernels of the VQ bottleneck: codebook gather + straight-through estimator + commitment
 // loss, its backward, per-code statistics for k-means, and small helpers.
 // Reference call sites are cited per kernel (paths relative to the reference root).
+#include <climits>
+
 #include "common.cuh"
 
 namespace vqseg {
@@ -978,14 +980,47 @@ static inline unsigned grid_for(long long total, int threads, int waves = 8) {
 // reference derives):  cluster_size <- decay cluster_size + (1 - decay) counts;  embed_avg <- decay embed_avg +
 // (1 - decay) sums;  n = sum(cluster_size);  cs = (cluster_size + eps) / (n + K eps) n;  weight = embed_avg / cs.
 // =================================================================================================
+// Dead-code expiry (EXPIRE, vqseg_ema_update_expire_f32): a code whose updated cluster_size is < threshold takes the
+// next candidate row in ascending k (slot = exclusive prefix of the expired mask), as lucidrains's boolean-mask
+// `replace`.  The smoothing's n is summed before any reset, so live codes get exactly what the EXPIRE=false
+// instantiation (vqseg_ema_update_f32) writes.
+template <bool EXPIRE>
 __global__ void __launch_bounds__(256) ema_cluster_kernel(const long long* __restrict__ counts, float* __restrict__ cluster_size,
-                                                          int K, float decay, float* __restrict__ total_out) {
+                                                          int K, float decay, float* __restrict__ total_out,
+                                                          float threshold, int* __restrict__ slot,
+                                                          long long* __restrict__ expired_out) {
   __shared__ double s_red[256];
+  __shared__ int s_warp[2][8];                   // per-warp expired counts, double-buffered: one barrier per 256 codes
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   double s = 0.0;
-  for (int k = threadIdx.x; k < K; k += 256) {
+  int offset = 0;                                // expired codes below this chunk
+  auto update = [&](int k) {
     const float cs = __fadd_rn(__fmul_rn(cluster_size[k], decay), __fmul_rn(1.f - decay, (float)counts[k]));
     cluster_size[k] = cs;
     s += (double)cs;
+    return cs;
+  };
+  if constexpr (!EXPIRE) {
+    for (int k = threadIdx.x; k < K; k += 256) update(k);
+  } else {
+    // chunks of 256 codes: thread t still owns k = t, t + 256, ... in increasing order, so s sums in the same order
+    for (int k0 = 0; k0 < K; k0 += 256) {
+      const int k = k0 + threadIdx.x;
+      const bool dead = k < K && update(k) < threshold;
+      const unsigned ballot = __ballot_sync(0xffffffffu, dead);
+      const int buf = (k0 >> 8) & 1;
+      if (lane == 0) s_warp[buf][wid] = __popc(ballot);
+      __syncthreads();
+      int below = 0, chunk = 0;
+#pragma unroll
+      for (int w = 0; w < 8; ++w) {
+        const int c = s_warp[buf][w];
+        below += w < wid ? c : 0;
+        chunk += c;
+      }
+      if (k < K) slot[k] = dead ? offset + below + __popc(ballot & ((1u << lane) - 1u)) : -1;
+      offset += chunk;
+    }
   }
   s_red[threadIdx.x] = s;
   __syncthreads();
@@ -993,14 +1028,39 @@ __global__ void __launch_bounds__(256) ema_cluster_kernel(const long long* __res
     if ((int)threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o];
     __syncthreads();
   }
-  if (threadIdx.x == 0) *total_out = (float)s_red[0];
+  if (threadIdx.x == 0) {
+    *total_out = (float)s_red[0];
+    if constexpr (EXPIRE) {
+      if (expired_out) {
+        expired_out[0] = offset;
+        expired_out[1] += offset;
+      }
+    }
+  }
 }
 
-__global__ void __launch_bounds__(256) ema_embed_kernel(const float* __restrict__ sums, const float* __restrict__ cluster_size,
+template <bool EXPIRE>
+__global__ void __launch_bounds__(256) ema_embed_kernel(const float* __restrict__ sums, float* __restrict__ cluster_size,
                                                         const float* __restrict__ total, float* __restrict__ embed_avg,
-                                                        float* __restrict__ weight, int K, int D, float decay, float eps) {
+                                                        float* __restrict__ weight, int K, int D, float decay, float eps,
+                                                        const int* __restrict__ slot, const float* __restrict__ cand,
+                                                        float reset) {
   const int k = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (k >= K) return;
+  if constexpr (EXPIRE) {
+    const int r = __ldg(slot + k);
+    if (r >= 0) {                                // this warp owns code k: nothing else reads or writes its rows
+      const float* c = cand + (long long)r * D;
+      for (int d = lane; d < D; d += 32) {
+        const long long i = (long long)k * D + d;
+        const float v = __ldg(c + d);
+        weight[i] = v;
+        embed_avg[i] = __fmul_rn(v, reset);
+      }
+      if (lane == 0) cluster_size[k] = reset;
+      return;
+    }
+  }
   const float n = __ldg(total);
   const float cs = __fmul_rn(__fdiv_rn(__fadd_rn(cluster_size[k], eps), __fadd_rn(n, __fmul_rn((float)K, eps))), n);
   for (int d = lane; d < D; d += 32) {
@@ -1371,10 +1431,40 @@ int vqseg_ema_update_f32(const int64_t* counts, const float* sums, float* cluste
                          float* weight_out, int64_t K, int64_t D, float decay, float eps, void* ws, void* stream) {
   if (!counts || !sums || !cluster_size_inout || !embed_avg_inout || !weight_out || !ws || K <= 0 || D <= 0) return VQSEG_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
-  ema_cluster_kernel<<<1, 256, 0, st>>>((const long long*)counts, cluster_size_inout, (int)K, decay, (float*)ws);
+  ema_cluster_kernel<false><<<1, 256, 0, st>>>((const long long*)counts, cluster_size_inout, (int)K, decay, (float*)ws,
+                                               0.f, nullptr, nullptr);
   VQSEG_LAUNCH_CHECK();
-  ema_embed_kernel<<<(unsigned)((K * 32 + 255) / 256), 256, 0, st>>>(sums, cluster_size_inout, (const float*)ws, embed_avg_inout,
-                                                                    weight_out, (int)K, (int)D, decay, eps);
+  ema_embed_kernel<false><<<(unsigned)((K * 32 + 255) / 256), 256, 0, st>>>(sums, cluster_size_inout, (const float*)ws,
+                                                                           embed_avg_inout, weight_out, (int)K, (int)D,
+                                                                           decay, eps, nullptr, nullptr, 0.f);
+  VQSEG_LAUNCH_CHECK();
+  return 0;
+}
+
+// ws: the fp32 n, then one int32 slot per code
+static constexpr size_t kExpireSlotOffset = 16;
+
+size_t vqseg_ema_expire_workspace_bytes(int64_t K) {
+  return K > 0 ? kExpireSlotOffset + (size_t)K * sizeof(int) : 0;
+}
+
+int vqseg_ema_update_expire_f32(const int64_t* counts, const float* sums, float* cluster_size_inout,
+                                float* embed_avg_inout, float* weight_out, int64_t K, int64_t D, float decay, float eps,
+                                float threshold, float reset, const float* cand_rows, int64_t* expired_out, void* ws,
+                                size_t ws_bytes, void* stream) {
+  if (!counts || !sums || !cluster_size_inout || !embed_avg_inout || !weight_out || !cand_rows || !ws || K <= 0 ||
+      D <= 0 || K > INT_MAX / 32)
+    return VQSEG_EINVAL;
+  if (ws_bytes < vqseg_ema_expire_workspace_bytes(K)) return VQSEG_EWORKSPACE;
+  cudaStream_t st = (cudaStream_t)stream;
+  float* total = (float*)ws;
+  int* slot = (int*)((char*)ws + kExpireSlotOffset);
+  ema_cluster_kernel<true><<<1, 256, 0, st>>>((const long long*)counts, cluster_size_inout, (int)K, decay, total,
+                                              threshold, slot, (long long*)expired_out);
+  VQSEG_LAUNCH_CHECK();
+  ema_embed_kernel<true><<<(unsigned)((K * 32 + 255) / 256), 256, 0, st>>>(sums, cluster_size_inout, total,
+                                                                          embed_avg_inout, weight_out, (int)K, (int)D,
+                                                                          decay, eps, slot, cand_rows, reset);
   VQSEG_LAUNCH_CHECK();
   return 0;
 }

@@ -40,6 +40,16 @@ def allreduce_code_stats(counts: torch.Tensor, sums: torch.Tensor, group=None) -
     h2.wait()
 
 
+def broadcast_rows(rows: torch.Tensor, group=None) -> None:
+    """In-place broadcast of rank 0's packed (K, D) rows: the `expire_sync_fn` of enable_ema(threshold_ema_dead_code=...).
+    Every rank draws its own dead-code candidates from its own batch; with `allreduce_code_stats` as the EMA's
+    `reduce_fn` the cluster sizes, hence the expired codes, are the same on every rank, and rank 0's candidates keep
+    the codebooks identical (K * D * 4 bytes per training forward)."""
+    if _world(group)[1] == 1:
+        return
+    dist.broadcast(rows, src=dist.get_global_rank(group, 0) if group is not None else 0, group=group)
+
+
 def global_code_usage(counts: torch.Tensor, group=None, usage_fn: Optional[Callable] = None) -> torch.Tensor:
     """code_usage over ALL ranks' pixels: all-reduce the K counts, then 100 * (#zero / K) (vq_img.py:173-175)."""
     counts = counts.clone()

@@ -463,6 +463,38 @@ def _ema_update_impl(counts: torch.Tensor, sums: torch.Tensor, cluster_size: tor
 ema_update = torch.library.custom_op("vqseg::ema_update", mutates_args=("cluster_size", "embed_avg", "weight"))(_ema_update_impl)
 
 
+def _ema_update_expire_impl(counts: torch.Tensor, sums: torch.Tensor, cluster_size: torch.Tensor, embed_avg: torch.Tensor,
+                            weight: torch.Tensor, decay: float, eps: float, threshold: float, reset: float,
+                            cand: torch.Tensor, expired: torch.Tensor) -> None:
+    """ema_update, then dead-code expiry (vqseg.h, vqseg_ema_update_expire_f32): the r-th code in ascending k whose
+    updated cluster_size is < threshold takes row r of `cand` (K, D) as its weight, cand * reset as its embed_avg and
+    `reset` as its cluster_size.  expired: int64 (2,) counters [last, total], updated on the device."""
+    _require_cuda(counts, sums, cluster_size, embed_avg, weight, cand, expired)
+    L = _native.lib()
+    k, d = weight.shape
+    assert counts.dtype == torch.int64 and counts.is_contiguous() and counts.numel() == k
+    for t in (sums, cluster_size, embed_avg, weight, cand):
+        assert t.dtype == torch.float32 and t.is_contiguous()
+    assert cand.shape == (k, d), "cand must hold K packed rows"
+    assert expired.dtype == torch.int64 and expired.is_contiguous() and expired.numel() == 2
+    nws = L.vqseg_ema_expire_workspace_bytes(k)
+    ws = torch.empty(nws, dtype=torch.uint8, device=weight.device)
+    with torch.cuda.device(weight.device):
+        _native.check(L.vqseg_ema_update_expire_f32(counts.data_ptr(), sums.data_ptr(), cluster_size.data_ptr(),
+                                                    embed_avg.data_ptr(), weight.data_ptr(), k, d, float(decay),
+                                                    float(eps), float(threshold), float(reset), cand.data_ptr(),
+                                                    expired.data_ptr(), ws.data_ptr(), nws, _stream()), "ema_update_expire")
+
+
+ema_update_expire = torch.library.custom_op(
+    "vqseg::ema_update_expire", mutates_args=("cluster_size", "embed_avg", "weight", "expired"))(_ema_update_expire_impl)
+
+
+@ema_update_expire.register_fake
+def _(counts, sums, cluster_size, embed_avg, weight, decay, eps, threshold, reset, cand, expired):
+    return None
+
+
 # -------------------------------------------------------------------------------------------------
 # distance map of the VQ segmentation head (models/modules/vq_segmentation_head.py:167-176 / :104-111)
 def _dist_map_raw(x, codebook, cosine=False, with_score=False):

@@ -118,6 +118,8 @@ class _CodebookBase(nn.Module):
         self.algo = ops.ALGO_AUTO
         self.kmeans_init_indices = None         # test hook: inject the k-means init rows
         self.kmeans_reduce_fn = None            # data-parallel hook: all-reduce (counts, sums)
+        self.threshold_ema_dead_code = 0.0      # dead-code expiry of the EMA update (enable_ema); 0 = off
+        self.expire_indices = None              # test hook: inject the K candidate rows of the expiry
         self._blob = None
         self._blob_key = None
 
@@ -135,7 +137,8 @@ class _CodebookBase(nn.Module):
         self._blob = None
 
     # ---- opt-in EMA codebook update (extension, SURVEY.md 8f-4; the reference never reads decay / eps) ----
-    def enable_ema(self, decay=None, eps=1e-5, reduce_fn=None, deterministic=False, persistent=False):
+    def enable_ema(self, decay=None, eps=1e-5, reduce_fn=None, deterministic=False, persistent=False,
+                   threshold_ema_dead_code=0.0, reset_cluster_size=None, expire_sync_fn=None):
         """After every TRAINING forward move the codebook towards the per-code means of that batch with the
         standard VQ-VAE EMA rule (include/vqseg.h, vqseg_ema_update_f32), using the `decay` the constructor stored
         (VectorQuantizer.enable_ema() also passes its stored `eps`).  `reduce_fn(counts, sums)` all-reduces the statistics in data-parallel training
@@ -143,7 +146,19 @@ class _CodebookBase(nn.Module):
         state_dict keys stay the reference's; `persistent=True` puts `cluster_size` / `embed_avg` into the state_dict so
         a resumed run continues the averages instead of restarting them.  They start as if every code had been used
         once (cluster_size = 1, embed_avg = weight): a code that gets no vector in the first steps keeps its weight
-        instead of being divided by ~eps."""
+        instead of being divided by ~eps.
+
+        `threshold_ema_dead_code > 0` replaces dead codes on the device after each EMA update (threshold_ema_dead_code
+        of lucidrains/vector-quantize-pytorch): every code whose updated cluster_size is below the threshold takes a
+        row of the batch (K rows drawn like sample_vectors; the r-th dead code in ascending k gets row r) as its
+        weight, that row * `reset_cluster_size` (default: the threshold) as its embed_avg and `reset_cluster_size` as
+        its cluster_size (vqseg_ema_update_expire_f32).  No host sync and no data-dependent shapes, so a training
+        forward with expiry can be captured as a CUDA graph.  `expire_sync_fn(rows)` makes the K candidate rows
+        identical on every rank in data-parallel training (vq_seg_b200.distributed.broadcast_rows).  The int64 device
+        counters `codes_expired_last` / `codes_expired_total` count the replaced codes; they are not in the state_dict."""
+        threshold_ema_dead_code = float(threshold_ema_dead_code)
+        if not threshold_ema_dead_code >= 0:
+            raise ValueError(f"threshold_ema_dead_code must be >= 0, got {threshold_ema_dead_code}")
         if decay is not None:
             self.decay = decay
         self.ema_eps = eps
@@ -153,8 +168,22 @@ class _CodebookBase(nn.Module):
         self.register_buffer("embed_avg", w.detach().clone().float().contiguous(), persistent=persistent)
         self.ema_reduce_fn = reduce_fn
         self.ema_deterministic = deterministic
+        self.threshold_ema_dead_code = threshold_ema_dead_code
+        self.reset_cluster_size = threshold_ema_dead_code if reset_cluster_size is None else float(reset_cluster_size)
+        self.expire_sync_fn = expire_sync_fn
+        self.register_buffer("codes_expired", torch.zeros(2, dtype=torch.int64, device=w.device), persistent=False)
         self.ema_enabled = True
         return self
+
+    @property
+    def codes_expired_last(self) -> torch.Tensor:
+        """Codes replaced by the last training forward (0-d int64 on the device)."""
+        return self.codes_expired[0]
+
+    @property
+    def codes_expired_total(self) -> torch.Tensor:
+        """Codes replaced since enable_ema() (0-d int64 on the device)."""
+        return self.codes_expired[1]
 
     @torch.no_grad()
     def _ema_step(self, x, idx):
@@ -164,7 +193,14 @@ class _CodebookBase(nn.Module):
         if self.ema_reduce_fn is not None:
             self.ema_reduce_fn(counts, sums)
         w = self.embedding.weight
-        ops.ema_update(counts, sums, self.cluster_size, self.embed_avg, w.data, self.decay, self.ema_eps)
+        if self.threshold_ema_dead_code > 0:
+            cand = _sample_rows(x, self.num_embeddings, self.expire_indices)
+            if self.expire_sync_fn is not None:
+                self.expire_sync_fn(cand)
+            ops.ema_update_expire(counts, sums, self.cluster_size, self.embed_avg, w.data, self.decay, self.ema_eps,
+                                  self.threshold_ema_dead_code, self.reset_cluster_size, cand, self.codes_expired)
+        else:
+            ops.ema_update(counts, sums, self.cluster_size, self.embed_avg, w.data, self.decay, self.ema_eps)
         self.invalidate()                       # the prepared fp16 image of the codebook is stale now
 
     def _kmeans_init(self, flatten_x, cosine):
@@ -286,7 +322,8 @@ class VectorQuantizer(nn.Module):
         return ent[1]
 
     def enable_ema(self, **kw):
-        """Opt-in EMA codebook update with the stored `decay` and `eps` (extension; see the codebook's enable_ema)."""
+        """Opt-in EMA codebook update with the stored `decay` and `eps`, optionally with dead-code expiry
+        (`threshold_ema_dead_code`, `reset_cluster_size`, `expire_sync_fn`; extension; see the codebook's enable_ema)."""
         kw.setdefault("eps", self.eps)
         self.codebook.enable_ema(**kw)
         return self
@@ -294,6 +331,8 @@ class VectorQuantizer(nn.Module):
     def forward(self, x):
         if x.dim() != 4:
             raise ValueError(f"VectorQuantizer expects a (B, C, H, W) tensor, got shape {tuple(x.shape)}")
+        if self.training and self.codebook.threshold_ema_dead_code > 0 and not self.codebook.ema_enabled:
+            raise ValueError("threshold_ema_dead_code replaces codes after the EMA update: enable it through enable_ema()")
         if not x.is_cuda:
             raise RuntimeError("vq_seg_b200.VectorQuantizer runs on a B200 GPU only (no CPU fallback); "
                                "move the module and its input to cuda")
@@ -339,7 +378,9 @@ class VectorQuantizer(nn.Module):
             loss = torch.zeros(1, device=device, dtype=torch.float32, requires_grad=self.training)
         if self.training and cb.ema_enabled:
             if cb.embed_avg.device != device:    # enable_ema() ran before .to(device)
-                cb.enable_ema(eps=cb.ema_eps, reduce_fn=cb.ema_reduce_fn, deterministic=cb.ema_deterministic)
+                cb.enable_ema(eps=cb.ema_eps, reduce_fn=cb.ema_reduce_fn, deterministic=cb.ema_deterministic,
+                              threshold_ema_dead_code=cb.threshold_ema_dead_code,
+                              reset_cluster_size=cb.reset_cluster_size, expire_sync_fn=cb.expire_sync_fn)
             cb._ema_step(ops.l2norm_rows(xv) if cosine else xv, idx)
         quantize = quantize.permute(0, 2, 1).reshape(b, c, h, w)     # memory is already (B, C, H*W): a view
         embed_index = idx.reshape(b, h, w)
