@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libvqseg.so")
 DEV_LIB = os.path.join(HERE, "libvqseg_dev.so")
 SOURCES = ["api.cu", "exact.cu", "assign_tc.cu", "assign_tc2.cu", "assign_tc3.cu", "assign_tc4.cu", "ops.cu", "seghead.cu", "seghead_tiled.cu"]
-HEADERS = ["common.cuh", "tc_common.cuh", "kernels.cuh", "codebook_prep.cuh", "exact_chain.cuh", os.path.join("..", "..", "include", "vqseg.h")]
+HEADERS = ["common.cuh", "tc_common.cuh", "kernels.cuh", "codebook_prep.cuh", "filter_epilogue.cuh", "exact_chain.cuh", os.path.join("..", "..", "include", "vqseg.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr"]
 

@@ -318,6 +318,8 @@ static int assign_internal(const float* x, int64_t B, int64_t P, int64_t D, int6
   const long long chain_len = ip ? D : D + 2;
   const long long kb_eff = (kblock <= 0 || kblock > chain_len) ? chain_len : kblock;
   const float slack_t2 = (float)(3 * ((chain_len + kb_eff - 1) / kb_eff) + 9) * 5.97e-8f;
+  const FilterOut out{(int)K, (long long*)idx_out, (unsigned long long*)counts_out, code_base, force ? 1 : 0, slack_t2,
+                      work, work_count};
   prof_record(prof_events, 0, st);
   if (kernel == 3) {
     Tc3Args t3;
@@ -326,10 +328,8 @@ static int assign_internal(const float* x, int64_t B, int64_t P, int64_t D, int6
     t3.tiles_per_image = (int)((P + 127) / 128);
     t3.n_tiles = (int)(B * t3.tiles_per_image);
     t3.n_ptiles = (t3.n_tiles + 1) / 2; t3.n_cc = n_cc; t3.n_dc = n_dc;
-    t3.K = (int)K; t3.K_pad = (int)kp; t3.off_image = oi; t3.off_aug = oa; t3.off_enorm = oe;
-    t3.idx_out = (long long*)idx_out; t3.counts_out = (unsigned long long*)counts_out; t3.code_base = code_base;
-    t3.force_rescore = force ? 1 : 0; t3.slack_t2 = slack_t2;
-    t3.work = work; t3.work_count = work_count;
+    t3.K_pad = (int)kp; t3.off_image = oi; t3.off_aug = oa; t3.off_enorm = oe;
+    t3.out = out;
     t3.trace = dev_trace();
     rc = launch_assign_tc3(xr, t3, st);
   } else if (kernel == 4 || kernel == 5) {
@@ -350,20 +350,16 @@ static int assign_internal(const float* x, int64_t B, int64_t P, int64_t D, int6
       t4.n_dc = slice_dc; t4.n_slices = n_slices;
       t4.part_scores = part_scores; t4.part_norms = part_norms;
     }
-    t4.K = (int)K; t4.K_pad = (int)kp; t4.off_image = oi; t4.off_aug = oa; t4.off_enorm = oe;
-    t4.idx_out = (long long*)idx_out; t4.counts_out = (unsigned long long*)counts_out; t4.code_base = code_base;
-    t4.force_rescore = force ? 1 : 0; t4.slack_t2 = slack_t2;
-    t4.work = work; t4.work_count = work_count;
+    t4.K_pad = (int)kp; t4.off_image = oi; t4.off_aug = oa; t4.off_enorm = oe;
+    t4.out = out;
     t4.trace = dev_trace();
     rc = launch_assign_tc4(xr, t4, lay4, st);
     if (!rc && kernel == 5) {
       ShortlistArgs sl;
       memset(&sl, 0, sizeof(sl));
-      sl.scores = part_scores; sl.norms = part_norms; sl.n_rows = n_rows; sl.K = (int)K; sl.K_pad = (int)kp; sl.D = (int)D;
+      sl.scores = part_scores; sl.norms = part_norms; sl.n_rows = n_rows; sl.K_pad = (int)kp; sl.D = (int)D;
       sl.blob = (const unsigned char*)blob;
-      sl.idx_out = (long long*)idx_out; sl.counts_out = (unsigned long long*)counts_out; sl.code_base = code_base;
-      sl.force_rescore = force ? 1 : 0; sl.slack_t2 = slack_t2;
-      sl.work = work; sl.work_count = work_count;
+      sl.out = out;
       rc = launch_shortlist(sl, st);
     }
   } else if (kernel == 2) {
@@ -371,11 +367,8 @@ static int assign_internal(const float* x, int64_t B, int64_t P, int64_t D, int6
     memset(&t2, 0, sizeof(t2));
     t2.x = xr; t2.blob = (const unsigned char*)blob; t2.n_rows = n_rows;
     t2.n_ptiles = (int)((n_rows + 255) / 256); t2.n_cc = n_cc; t2.n_dc = n_dc;
-    t2.K = (int)K; t2.K_pad = (int)kp; t2.off_image = oi; t2.off_aug = oa; t2.off_enorm = oe;
-    t2.tau = 0.f;
-    t2.idx_out = (long long*)idx_out; t2.counts_out = (unsigned long long*)counts_out; t2.code_base = code_base;
-    t2.force_rescore = force ? 1 : 0; t2.slack_t2 = slack_t2;
-    t2.work = work; t2.work_count = work_count;
+    t2.K_pad = (int)kp; t2.off_image = oi; t2.off_aug = oa; t2.off_enorm = oe;
+    t2.out = out;
     t2.trace = dev_trace();
     rc = launch_assign_tc2(t2, st);
   } else {
@@ -383,11 +376,7 @@ static int assign_internal(const float* x, int64_t B, int64_t P, int64_t D, int6
     memset(&ta, 0, sizeof(ta));
     ta.x = xr; ta.blob = (const unsigned char*)blob; ta.n_rows = n_rows;
     ta.n_tiles = (int)((n_rows + 127) / 128); ta.n_cc = n_cc; ta.n_dc = n_dc;
-    ta.K = (int)K;
-    ta.tau = 0.f;
-    ta.idx_out = (long long*)idx_out; ta.counts_out = (unsigned long long*)counts_out; ta.code_base = code_base;
-    ta.force_rescore = force ? 1 : 0; ta.slack_t2 = slack_t2;
-    ta.work = work; ta.work_count = work_count;
+    ta.out = out;
     ta.trace = dev_trace();
     rc = launch_assign_tc(ta, st);
   }

@@ -20,7 +20,7 @@
 // Pipelines: smem full/empty mbarriers (3 stages), TMEM full/empty (2 x 256 columns), limb-tile full/empty (2);
 // setmaxnreg moves the register budget to the producers (144 / 72 / 40).
 #include "tc_common.cuh"
-#include "kernels.cuh"
+#include "filter_epilogue.cuh"
 #include "codebook_prep.cuh"
 
 namespace vqseg {
@@ -33,7 +33,6 @@ constexpr int kBStageBytes = kUnitN * kDChunk * 2;        // 32 KiB
 constexpr int kProducerWarps = 8;
 constexpr int kMmaWarp = 16;          // warps 8-15: epilogue, 16: MMA issuer + TMEM alloc, 17: B loader, 18-19: idle
 constexpr int kTcThreads = 20 * 32;
-constexpr int kCandCap = 8;           // short-list entries kept per row before falling back to "all codes"
 constexpr int kXsqBufs = 8;
 constexpr int kAugTileBytes = 128 * 16 * 2;               // 4 KiB: 128 codes x 16 fp16, SWIZZLE_NONE core matrices
 constexpr uint32_t kIdesc = make_idesc_f16(kTileM, kUnitN);
@@ -45,7 +44,7 @@ struct TcSmem {
   static constexpr int off_baug = off_b + kStages * kBStageBytes;             // [2] 8 KiB: limb tiles of 256 codes
   static constexpr int off_aaug = off_baug + 2 * 2 * kAugTileBytes;           // 4 KiB
   static constexpr int off_cand = off_aaug + kAugTileBytes;                   // [2 halves][128][cap] code indices
-  static constexpr int off_xchg = off_cand + 2 * kTileM * kCandCap * 4;       // [128] {m_run, cnt|overflow} of the upper half
+  static constexpr int off_xchg = off_cand + 2 * kTileM * kWorkCandCap * 4;   // [128] {m_run, cnt|overflow} of the upper half
   static constexpr int off_xsq = off_xchg + kTileM * 8;                       // [kXsqBufs][128] float2 {|x|^2, |fp16(x)-x|^2}
   static constexpr int off_bar = off_xsq + kXsqBufs * kTileM * 8;             // mbarriers
   static constexpr int off_tmem = off_bar + 8 * (2 * kStages + 8);
@@ -226,21 +225,13 @@ __global__ void __launch_bounds__(kTcThreads, 1) assign_tc_kernel(TcArgs a) {
     const int half = (warp - kProducerWarps) >> 2;
     const int r = quarter * 32 + lane;
     const uint32_t lane_addr = tmem_base + ((uint32_t)(quarter * 32) << 16) + half * 128;
-    int* cand = reinterpret_cast<int*>(smem + TcSmem::off_cand) + (half * kTileM + r) * kCandCap;
-    const int* cand_hi = reinterpret_cast<const int*>(smem + TcSmem::off_cand) + (kTileM + r) * kCandCap;
+    const ShortList<int>::Slots lists(reinterpret_cast<int*>(smem + TcSmem::off_cand), kTileM, half, r);
     float2* xchg = reinterpret_cast<float2*>(smem + TcSmem::off_xchg) + r;
-    const float scale = hdr->scale;
-    const float emax = sqrtf(hdr->max_enorm) * 1.0001f;
-    const float de_max = sqrtf(__uint_as_float(hdr->max_de2_bits)) * 1.0001f;
-    const bool bad_blob = (hdr->flags & 1u) != 0;
+    const FilterBound bound(hdr);
     int u = 0;
     for (int t = 0; t < my_tiles; ++t) {
       const long long n = ((long long)blockIdx.x + (long long)t * gridDim.x) * kTileM + r;
-      float m_run = __int_as_float(0x7f800000);
-      float slack = 0.f;
-      int cnt = 0;
-      bool overflow = false;          // the short-list of this half ran over its capacity (cleared when a new minimum drops the list)
-      bool bad = false;               // the row cannot be bounded at all (non-finite slack, unusable blob): every code is rescored
+      ShortList<int> sl(lists);
       for (int cc = 0; cc < a.n_cc; ++cc, ++u) {
         const int buf = u & 1;
         if (warp == kProducerWarps) VQ_TRACE(2, 4 * u);
@@ -250,93 +241,21 @@ __global__ void __launch_bounds__(kTcThreads, 1) assign_tc_kernel(TcArgs a) {
         if (cc == 0) {
           // all A chunks of this tile's first unit are in: the row's |x|^2 and |fp16(x)-x|^2 have been published
           const float2 nr = reinterpret_cast<const float2*>(xsq)[(t & (kXsqBufs - 1)) * kTileM + r];
-          const float xn = sqrtf(nr.x) * 1.0001f, dn = sqrtf(nr.y) * 1.0001f;
-          // |approx - exact| <= |dx| |e^| + |x| |de|  (Cauchy-Schwarz on the ACTUAL operand rounding errors, both
-          // measured exactly: dx by the producers, de by codebook_rounding_error_kernel), two-sided, plus the fp32
-          // accumulation error of the tensor core and of the exact scorer's chain and the |e|^2 limb residual
-          slack = filter_slack(xn, dn, emax, de_max, scale, (int)a.x.D, a.slack_t2);
-          if (!(slack < 3.0e38f) || bad_blob) bad = true;
+          sl.start(bound, nr.x, nr.y, (int)a.x.D, a.out.slack_t2);
         }
         const uint32_t tb = lane_addr + buf * kUnitN;
 #pragma unroll 1
         for (int c = 0; c < 128; c += 32) {
           uint32_t v[32];
           tmem_ld32(tb + c, v);
-          float m0 = __uint_as_float(v[0]), m1 = __uint_as_float(v[1]);
-#pragma unroll
-          for (int j = 0; j < 32; j += 4) {
-            m0 = fminf(m0, fminf(__uint_as_float(v[j]), __uint_as_float(v[j + 2])));
-            m1 = fminf(m1, fminf(__uint_as_float(v[j + 1]), __uint_as_float(v[j + 3])));
-          }
-          const float m_new = fminf(m_run, fminf(m0, m1));
-          if (m_run > m_new + slack) { cnt = 0; overflow = false; }   // every earlier entry (listed or dropped) scored >= the old minimum
-          m_run = m_new;
-          const float thr = m_run + slack;
-          // bit (31 - j) of ~mk <=> v[j] <= thr: one FADD + one funnel shift per score, four independent chains
-          uint32_t mka = 0u, mkb = 0u, mkc = 0u, mkd = 0u;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            mka = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j])), mka, 1);
-            mkb = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j + 8])), mkb, 1);
-            mkc = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j + 16])), mkc, 1);
-            mkd = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j + 24])), mkd, 1);
-          }
-          uint32_t mk = ~((mka << 24) | ((mkb & 0xffu) << 16) | ((mkc & 0xffu) << 8) | (mkd & 0xffu));
-          if (overflow || bad) mk = 0u;
-          while (mk) {
-            const int j = __clz(mk);
-            mk &= ~(0x80000000u >> j);
-            if (cnt < kCandCap) cand[cnt++] = cc * kUnitN + half * 128 + c + j;
-            else { overflow = true; mk = 0u; }
-          }
+          sl.scan32(v, cc * kUnitN + half * 128 + c);
         }
         if (warp == kProducerWarps) VQ_TRACE(2, 4 * u + 2);
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar_tempty + 8 * buf);              // this warp's columns are drained
       }
-      // ---- tile done: the two column halves of each row meet (named barrier per lane quarter) ----
-      if (half == 1) *xchg = make_float2(m_run, __int_as_float(bad ? -2 : (overflow ? -1 : cnt)));
-      asm volatile("bar.sync %0, 64;" ::"r"(1 + quarter) : "memory");
-      if (half == 0) {
-        const float2 o = *xchg;
-        int cnt1 = __float_as_int(o.y);
-        const float m = fminf(m_run, o.x);
-        bool ov1 = cnt1 == -1;
-        if (cnt1 == -2) bad = true;
-        // a half whose own minimum is out of range contributes nothing (all its entries scored >= that minimum)
-        if (m_run > m + slack) { cnt = 0; overflow = false; }
-        if (o.x > m + slack) { cnt1 = 0; ov1 = false; }
-        if (cnt1 < 0) cnt1 = 0;
-        overflow = overflow || ov1 || bad;
-        const bool in_range = n < a.n_rows;
-        const int tot = overflow ? 0 : cnt + cnt1;
-        const int last = (!overflow && tot == 1) ? (cnt == 1 ? cand[0] : cand_hi[0]) : 0;
-        const bool unique = !overflow && tot == 1 && !a.force_rescore && last < a.K;
-        if (in_range && unique) {
-          a.idx_out[n] = (long long)last + a.code_base;
-          if (a.counts_out) atomicAdd(a.counts_out + last, 1ull);
-        }
-        const bool flagged = in_range && !unique;
-        const uint32_t fm = __ballot_sync(0xffffffffu, flagged);
-        if (fm) {                                            // one atomic per warp on the work counter
-          int base = 0;
-          if (lane == 0) base = atomicAdd(a.work_count, __popc(fm));
-          base = __shfl_sync(0xffffffffu, base, 0);
-          if (flagged) {
-            // one 48-byte record per undecided row (cnt > cap => the exact pass scans all codes)
-            int* rec = reinterpret_cast<int*>(a.work + (base + __popc(fm & ((1u << lane) - 1))));
-            int nc = 0;
-            if (!overflow) {
-              for (int e = 0; e < cnt; ++e) { int k = cand[e]; if (k < a.K && nc < kCandCap) rec[4 + nc++] = k; else if (k < a.K) overflow = true; }
-              for (int e = 0; e < cnt1; ++e) { int k = cand_hi[e]; if (k < a.K && nc < kCandCap) rec[4 + nc++] = k; else if (k < a.K) overflow = true; }
-            }
-            rec[0] = (int)n;
-            rec[1] = (overflow || nc == 0) ? kCandCap + 1 : nc;
-          }
-        }
-      }
-      asm volatile("bar.sync %0, 64;" ::"r"(1 + quarter) : "memory");   // lists / xchg free for the next tile
+      sl.finish(half, 1 + quarter, xchg, n < a.n_rows, n, a.out);
     }
   } else {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 40;");

@@ -19,7 +19,7 @@
 // 17 codebook loader (cp.async.bulk) then x loader, 18-19 x loaders (one TMA-issuing thread per stage).
 #include <cuda.h>
 #include "tc_common.cuh"
-#include "kernels.cuh"
+#include "filter_epilogue.cuh"
 
 namespace vqseg {
 
@@ -32,7 +32,6 @@ constexpr int k3StageBytes = k3StageCh * k3Rows * 4;    // 16 KiB
 constexpr int k3Issuers = 3;                 // one TMA-issuing thread per stage (each stage barrier has ONE waiter)
 constexpr int k3MaxBTiles = 8;               // resident 16 KiB codebook tiles per CTA
 constexpr int k3MaxCC = 2;
-constexpr int k3CandCap = kWorkCandCap;
 constexpr int k3AugBytes = 128 * 16 * 2;     // 4 KiB: 128 codes x 16 fp16, SWIZZLE_NONE core matrices
 constexpr uint32_t k3Idesc = make_idesc_f16(256, 256);
 
@@ -43,7 +42,7 @@ struct Tc3Smem {
   static constexpr int off_baug = off_stage + k3Stages * k3StageBytes;      // [k3MaxCC] 4 KiB
   static constexpr int off_aaug = off_baug + k3MaxCC * k3AugBytes;          // 256 B: ONE 8-row group, reused by all 16 (SBO = 0)
   static constexpr int off_cand = off_aaug + 256;                           // [2 halves][128][cap] uint16
-  static constexpr int off_xchg = off_cand + 2 * k3Rows * k3CandCap * 2;     // [128] {m_run, cnt|overflow} of the upper-half warp
+  static constexpr int off_xchg = off_cand + 2 * k3Rows * kWorkCandCap * 2;  // [128] {m_run, cnt|overflow} of the upper-half warp
   static constexpr int off_xsq = off_xchg + k3Rows * 8;                      // [2 tiles][2 groups][128] float2 {|x|^2, |fp16(x)-x|^2}
   static constexpr int off_bar = off_xsq + 2 * 2 * k3Rows * 8;
   static constexpr int n_bars = 2 * k3Stages + 2 * k3ASlots + 4 + 2 * k3MaxCC;
@@ -208,13 +207,9 @@ assign_tc3_kernel(const __grid_constant__ CUtensorMap tmap, Tc3Args a) {
     const int half = (warp - 8) >> 2;                     // which 128 of the unit's 256 columns
     const int r = quarter * 32 + lane;
     const uint32_t lane_addr = tmem_base + ((uint32_t)(quarter * 32) << 16) + half * 128;
-    unsigned short* cand = reinterpret_cast<unsigned short*>(smem + Tc3Smem::off_cand) + (half * k3Rows + r) * k3CandCap;
-    const unsigned short* cand_hi = reinterpret_cast<const unsigned short*>(smem + Tc3Smem::off_cand) + (k3Rows + r) * k3CandCap;
+    const ShortList<unsigned short>::Slots lists(reinterpret_cast<unsigned short*>(smem + Tc3Smem::off_cand), k3Rows, half, r);
     float2* xchg = reinterpret_cast<float2*>(smem + Tc3Smem::off_xchg) + r;
-    const float scale = hdr->scale;
-    const float emax = sqrtf(hdr->max_enorm) * 1.0001f;
-    const float de_max = sqrtf(__uint_as_float(hdr->max_de2_bits)) * 1.0001f;
-    const bool bad_blob = (hdr->flags & 1u) != 0;
+    const FilterBound bound(hdr);
     if (warp == 8) {
       // relay: this CTA's half of each code chunk has landed -> tell the leader's MMA issuer (the loader thread goes
       // straight on to issuing x boxes and must not sit in this wait)
@@ -229,11 +224,7 @@ assign_tc3_kernel(const __grid_constant__ CUtensorMap tmap, Tc3Args a) {
       tile_coords(tt, img, p0);
       const bool in_range = img < (int)a.B && p0 + r < (int)a.P;
       const long long n = (long long)img * a.P + p0 + r;
-      float m_run = __int_as_float(0x7f800000);
-      float slack = 0.f;
-      int cnt = 0;
-      bool overflow = false;          // the short-list of this half ran over its capacity (cleared when a new minimum drops the list)
-      bool bad = false;               // the row cannot be bounded at all (non-finite slack, unusable blob): every code is rescored
+      ShortList<unsigned short> sl(lists);
       for (int cc = 0; cc < a.n_cc; ++cc, ++u) {
         if (warp == 8) VQ3_TRACE(2, 4 * u);
         mbar_wait(bar_tfull + 8 * cc, (uint32_t)tt & 1);
@@ -241,90 +232,21 @@ assign_tc3_kernel(const __grid_constant__ CUtensorMap tmap, Tc3Args a) {
         if (warp == 8) VQ3_TRACE(2, 4 * u + 1);
         if (cc == 0) {
           const float2 n0 = xsq[((tt & 1) * 2 + 0) * k3Rows + r], n1 = xsq[((tt & 1) * 2 + 1) * k3Rows + r];
-          const float xn = sqrtf(n0.x + n1.x) * 1.0001f, dn = sqrtf(n0.y + n1.y) * 1.0001f;
-          // |approx - exact| <= |dx| |e^| + |x| |de| (Cauchy-Schwarz on the ACTUAL operand rounding errors, see
-          // assign_tc.cu), two-sided, + fp32 accumulation / exact-chain error + limb residual of |e|^2
-          slack = filter_slack(xn, dn, emax, de_max, scale, (int)a.D, a.slack_t2);
-          if (!(slack < 3.0e38f) || bad_blob) bad = true;
+          sl.start(bound, n0.x + n1.x, n0.y + n1.y, (int)a.D, a.out.slack_t2);
         }
         const uint32_t tb = lane_addr + cc * 256;
 #pragma unroll 1
         for (int c = 0; c < 128; c += 32) {
           uint32_t v[32];
           tmem_ld32(tb + c, v);
-          float m0 = __uint_as_float(v[0]), m1 = __uint_as_float(v[1]);
-#pragma unroll
-          for (int j = 0; j < 32; j += 4) {
-            m0 = fminf(m0, fminf(__uint_as_float(v[j]), __uint_as_float(v[j + 2])));
-            m1 = fminf(m1, fminf(__uint_as_float(v[j + 1]), __uint_as_float(v[j + 3])));
-          }
-          const float m_new = fminf(m_run, fminf(m0, m1));
-          if (m_run > m_new + slack) { cnt = 0; overflow = false; }   // every earlier entry (listed or dropped) scored >= the old minimum
-          m_run = m_new;
-          const float thr = m_run + slack;
-          uint32_t mka = 0u, mkb = 0u, mkc = 0u, mkd = 0u;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            mka = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j])), mka, 1);
-            mkb = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j + 8])), mkb, 1);
-            mkc = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j + 16])), mkc, 1);
-            mkd = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j + 24])), mkd, 1);
-          }
-          uint32_t mk = ~((mka << 24) | ((mkb & 0xffu) << 16) | ((mkc & 0xffu) << 8) | (mkd & 0xffu));
-          if (overflow || bad) mk = 0u;
-          while (mk) {
-            const int j = __clz(mk);
-            mk &= ~(0x80000000u >> j);
-            if (cnt < k3CandCap) cand[cnt++] = (unsigned short)(cc * 256 + half * 128 + c + j);
-            else { overflow = true; mk = 0u; }
-          }
+          sl.scan32(v, cc * 256 + half * 128 + c);
         }
         if (warp == 8) VQ3_TRACE(2, 4 * u + 2);
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_cluster(lead_tempty + 8 * cc);      // this warp's columns are drained
       }
-      // ---- tile done: the two column halves of each row meet (named barrier per lane quarter) ----
-      if (half == 1) *xchg = make_float2(m_run, __int_as_float(bad ? -2 : (overflow ? -1 : cnt)));
-      asm volatile("bar.sync %0, 64;" ::"r"(1 + quarter) : "memory");
-      if (half == 0) {
-        const float2 o = *xchg;
-        int cnt1 = __float_as_int(o.y);
-        const float m = fminf(m_run, o.x);
-        bool ov1 = cnt1 == -1;
-        if (cnt1 == -2) bad = true;
-        // a half whose own minimum is out of range contributes nothing (all its entries scored >= that minimum)
-        if (m_run > m + slack) { cnt = 0; overflow = false; }
-        if (o.x > m + slack) { cnt1 = 0; ov1 = false; }
-        if (cnt1 < 0) cnt1 = 0;
-        overflow = overflow || ov1 || bad;
-        const int tot = overflow ? 0 : cnt + cnt1;
-        const int last = (!overflow && tot == 1) ? (cnt == 1 ? (int)cand[0] : (int)cand_hi[0]) : 0;
-        const bool unique = !overflow && tot == 1 && !a.force_rescore && last < a.K;
-        if (in_range && unique) {
-          a.idx_out[n] = (long long)last + a.code_base;
-          if (a.counts_out) atomicAdd(a.counts_out + last, 1ull);
-        }
-        const bool flagged = in_range && !unique;
-        const uint32_t fm = __ballot_sync(0xffffffffu, flagged);
-        if (fm) {
-          int base = 0;
-          if (lane == 0) base = atomicAdd(a.work_count, __popc(fm));
-          base = __shfl_sync(0xffffffffu, base, 0);
-          if (flagged) {
-            // one 48-byte record per undecided row (cnt > cap => the exact pass scans all codes)
-            int* rec = reinterpret_cast<int*>(a.work + (base + __popc(fm & ((1u << lane) - 1))));
-            int nc = 0;
-            if (!overflow) {
-              for (int e = 0; e < cnt; ++e) { int k = cand[e]; if (k < a.K && nc < k3CandCap) rec[4 + nc++] = k; else if (k < a.K) overflow = true; }
-              for (int e = 0; e < cnt1; ++e) { int k = cand_hi[e]; if (k < a.K && nc < k3CandCap) rec[4 + nc++] = k; else if (k < a.K) overflow = true; }
-            }
-            rec[0] = (int)n;
-            rec[1] = (overflow || nc == 0) ? k3CandCap + 1 : nc;
-          }
-        }
-      }
-      asm volatile("bar.sync %0, 64;" ::"r"(1 + quarter) : "memory");   // lists / xchg free for the next tile
+      sl.finish(half, 1 + quarter, xchg, in_range, n, a.out);
     }
   } else if (warp == 16) {
     if (rank == 0 && elect_one()) {

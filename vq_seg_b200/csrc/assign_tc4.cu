@@ -20,7 +20,7 @@
 #include <cuda.h>
 #include <string.h>
 #include "tc_common.cuh"
-#include "kernels.cuh"
+#include "filter_epilogue.cuh"
 
 namespace vqseg {
 
@@ -31,7 +31,6 @@ constexpr int k4BStages = 3;                 // ring of 128-code x 64-dim codebo
 constexpr int k4XStages = 2;                 // ring of fp32 x boxes (16 KiB each), one issuing thread per stage (power of two)
 constexpr int k4BoxDims = 32;                // dims per x box
 constexpr int k4XBytes = k4BoxDims * k4Rows * 4;
-constexpr int k4CandCap = kWorkCandCap;
 constexpr int k4AugBytes = 128 * 16 * 2;     // 4 KiB: 128 codes x 16 fp16, SWIZZLE_NONE core matrices
 constexpr uint32_t k4Idesc = make_idesc_f16(256, 256);
 
@@ -42,7 +41,7 @@ struct Tc4Smem {
   static constexpr int off_baug = off_x + k4XStages * k4XBytes;             // [2] 4 KiB: |e|^2 limb tiles, by unit parity
   static constexpr int off_aaug = off_baug + 2 * k4AugBytes;                // 256 B: ONE 8-row group, reused by all 16 (SBO = 0)
   static constexpr int off_cand = off_aaug + 256;                           // [2 halves][128][cap] uint16
-  static constexpr int off_xchg = off_cand + 2 * k4Rows * k4CandCap * 2;     // [128] {m_run, cnt|overflow} of the upper-half warp
+  static constexpr int off_xchg = off_cand + 2 * k4Rows * kWorkCandCap * 2;  // [128] {m_run, cnt|overflow} of the upper-half warp
   static constexpr int off_xsq = off_xchg + k4Rows * 8;                      // [2 tiles][2 halves of a box][128] float2
   static constexpr int off_bar = off_xsq + 2 * 2 * k4Rows * 8;
   static constexpr int n_bars = 2 * k4ASlots + 3 * k4BStages + 2 * k4XStages + 4 + 2 + 2 + k4ASlots;
@@ -236,13 +235,9 @@ assign_tc4_kernel(const __grid_constant__ CUtensorMap tmap, Tc4Args a) {
     const int half = (warp - 8) >> 2;
     const int r = quarter * 32 + lane;
     const uint32_t lane_addr = tmem_base + ((uint32_t)(quarter * 32) << 16) + half * 128;
-    unsigned short* cand = reinterpret_cast<unsigned short*>(smem + Tc4Smem::off_cand) + (half * k4Rows + r) * k4CandCap;
-    const unsigned short* cand_hi = reinterpret_cast<const unsigned short*>(smem + Tc4Smem::off_cand) + (k4Rows + r) * k4CandCap;
+    const ShortList<unsigned short>::Slots lists(reinterpret_cast<unsigned short*>(smem + Tc4Smem::off_cand), k4Rows, half, r);
     float2* xchg = reinterpret_cast<float2*>(smem + Tc4Smem::off_xchg) + r;
-    const float scale = hdr->scale;
-    const float emax = sqrtf(hdr->max_enorm) * 1.0001f;
-    const float de_max = sqrtf(__uint_as_float(hdr->max_de2_bits)) * 1.0001f;
-    const bool bad_blob = (hdr->flags & 1u) != 0;
+    const FilterBound bound(hdr);
     int u = 0;
     for (int tt = 0; tt < my_tiles; ++tt) {
       const int t = tile_id(tt);
@@ -289,11 +284,7 @@ assign_tc4_kernel(const __grid_constant__ CUtensorMap tmap, Tc4Args a) {
         }
         continue;
       }
-      float m_run = __int_as_float(0x7f800000);
-      float slack = 0.f;
-      int cnt = 0;
-      bool overflow = false;          // the short-list of this half ran over its capacity (cleared when a new minimum drops the list)
-      bool bad = false;               // the row cannot be bounded at all (non-finite slack, unusable blob): every code is rescored
+      ShortList<unsigned short> sl(lists);
       for (int cc = 0; cc < a.n_cc; ++cc, ++u) {
         const int buf = u & 1;
         if (warp == 8) VQ4_TRACE(2, 4 * u);
@@ -307,11 +298,7 @@ assign_tc4_kernel(const __grid_constant__ CUtensorMap tmap, Tc4Args a) {
           } else {
             n0 = xsq[((tt & 1) * 2 + 0) * k4Rows + r]; n1 = xsq[((tt & 1) * 2 + 1) * k4Rows + r];
           }
-          const float xn = sqrtf(n0.x + n1.x) * 1.0001f, dn = sqrtf(n0.y + n1.y) * 1.0001f;
-          // |approx - exact| <= |dx| |e^| + |x| |de| (Cauchy-Schwarz on the ACTUAL operand rounding errors, see
-          // assign_tc.cu), two-sided, + fp32 accumulation / exact-chain error + limb residual of |e|^2
-          slack = filter_slack(xn, dn, emax, de_max, scale, (int)a.D, a.slack_t2);
-          if (!(slack < 3.0e38f) || bad_blob) bad = true;
+          sl.start(bound, n0.x + n1.x, n0.y + n1.y, (int)a.D, a.out.slack_t2);
           __syncwarp();
           if (!PRE && lane == 0) mbar_arrive(bar_nempty + 8 * (tt & 1));  // the converters may reuse this norm buffer
         }
@@ -320,78 +307,14 @@ assign_tc4_kernel(const __grid_constant__ CUtensorMap tmap, Tc4Args a) {
         for (int c = 0; c < 128; c += 32) {
           uint32_t v[32];
           tmem_ld32(tb + c, v);
-          float m0 = __uint_as_float(v[0]), m1 = __uint_as_float(v[1]);
-#pragma unroll
-          for (int j = 0; j < 32; j += 4) {
-            m0 = fminf(m0, fminf(__uint_as_float(v[j]), __uint_as_float(v[j + 2])));
-            m1 = fminf(m1, fminf(__uint_as_float(v[j + 1]), __uint_as_float(v[j + 3])));
-          }
-          const float m_new = fminf(m_run, fminf(m0, m1));
-          if (m_run > m_new + slack) { cnt = 0; overflow = false; }   // every earlier entry (listed or dropped) scored >= the old minimum
-          m_run = m_new;
-          const float thr = m_run + slack;
-          uint32_t mka = 0u, mkb = 0u, mkc = 0u, mkd = 0u;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            mka = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j])), mka, 1);
-            mkb = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j + 8])), mkb, 1);
-            mkc = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j + 16])), mkc, 1);
-            mkd = __funnelshift_l(__float_as_uint(thr - __uint_as_float(v[j + 24])), mkd, 1);
-          }
-          uint32_t mk = ~((mka << 24) | ((mkb & 0xffu) << 16) | ((mkc & 0xffu) << 8) | (mkd & 0xffu));
-          if (overflow || bad) mk = 0u;
-          while (mk) {
-            const int j = __clz(mk);
-            mk &= ~(0x80000000u >> j);
-            if (cnt < k4CandCap) cand[cnt++] = (unsigned short)(cc * 256 + half * 128 + c + j);
-            else { overflow = true; mk = 0u; }
-          }
+          sl.scan32(v, cc * 256 + half * 128 + c);
         }
         if (warp == 8) VQ4_TRACE(2, 4 * u + 2);
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_cluster(lead_tempty + 8 * buf);     // this warp's columns are drained
       }
-      // ---- tile done: the two column halves of each row meet (named barrier per lane quarter) ----
-      if (half == 1) *xchg = make_float2(m_run, __int_as_float(bad ? -2 : (overflow ? -1 : cnt)));
-      asm volatile("bar.sync %0, 64;" ::"r"(1 + quarter) : "memory");
-      if (half == 0) {
-        const float2 o = *xchg;
-        int cnt1 = __float_as_int(o.y);
-        const float m = fminf(m_run, o.x);
-        bool ov1 = cnt1 == -1;
-        if (cnt1 == -2) bad = true;
-        if (m_run > m + slack) { cnt = 0; overflow = false; }
-        if (o.x > m + slack) { cnt1 = 0; ov1 = false; }
-        if (cnt1 < 0) cnt1 = 0;
-        overflow = overflow || ov1 || bad;
-        const int tot = overflow ? 0 : cnt + cnt1;
-        const int last = (!overflow && tot == 1) ? (cnt == 1 ? (int)cand[0] : (int)cand_hi[0]) : 0;
-        const bool unique = !overflow && tot == 1 && !a.force_rescore && last < a.K;
-        if (in_range && unique) {
-          a.idx_out[n] = (long long)last + a.code_base;
-          if (a.counts_out) atomicAdd(a.counts_out + last, 1ull);
-        }
-        const bool flagged = in_range && !unique;
-        const uint32_t fm = __ballot_sync(0xffffffffu, flagged);
-        if (fm) {
-          int base = 0;
-          if (lane == 0) base = atomicAdd(a.work_count, __popc(fm));
-          base = __shfl_sync(0xffffffffu, base, 0);
-          if (flagged) {
-            // one 48-byte record per undecided row (cnt > cap => the exact pass scans all codes)
-            int* rec = reinterpret_cast<int*>(a.work + (base + __popc(fm & ((1u << lane) - 1))));
-            int nc = 0;
-            if (!overflow) {
-              for (int e = 0; e < cnt; ++e) { int k = cand[e]; if (k < a.K && nc < k4CandCap) rec[4 + nc++] = k; else if (k < a.K) overflow = true; }
-              for (int e = 0; e < cnt1; ++e) { int k = cand_hi[e]; if (k < a.K && nc < k4CandCap) rec[4 + nc++] = k; else if (k < a.K) overflow = true; }
-            }
-            rec[0] = (int)n;
-            rec[1] = (overflow || nc == 0) ? k4CandCap + 1 : nc;
-          }
-        }
-      }
-      asm volatile("bar.sync %0, 64;" ::"r"(1 + quarter) : "memory");   // lists / xchg free for the next tile
+      sl.finish(half, 1 + quarter, xchg, in_range, n, a.out);
     }
   } else if (warp == 16) {
     if (rank == 0 && elect_one()) {
@@ -581,17 +504,12 @@ int launch_samples_prepare(const Rows& x, long long rows_padded, int D_pad, unsi
 // |fp16(x) - x|^2 and the blob's header), the codes within the bound in ascending order.  One survivor: final index;
 // otherwise a work record for the rescoring pass (more than kWorkCandCap survivors: "score every code").
 __global__ void __launch_bounds__(256) shortlist_kernel(ShortlistArgs a) {
-  const BlobHeader* hdr = reinterpret_cast<const BlobHeader*>(a.blob);
+  const FilterBound bound(reinterpret_cast<const BlobHeader*>(a.blob));
   const int lane = threadIdx.x & 31;
-  const float scale = hdr->scale;
-  const float emax = sqrtf(hdr->max_enorm) * 1.0001f;
-  const float de_max = sqrtf(__uint_as_float(hdr->max_de2_bits)) * 1.0001f;
-  const bool bad_blob = (hdr->flags & 1u) != 0;
   const long long w0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = ((long long)gridDim.x * blockDim.x) >> 5;
   for (long long n = w0; n < a.n_rows; n += nw) {
-    const float xn = sqrtf(a.norms[2 * n]) * 1.0001f, dn = sqrtf(a.norms[2 * n + 1]) * 1.0001f;
-    const float slack = filter_slack(xn, dn, emax, de_max, scale, (int)a.D, a.slack_t2);   // (common.cuh)
-    bool overflow = !(slack < 3.0e38f) || bad_blob;
+    const float slack = bound.slack(a.norms[2 * n], a.norms[2 * n + 1], a.D, a.out.slack_t2);
+    bool overflow = !(slack < 3.0e38f) || bound.defer_all;
     const float* sc = a.scores + n * (long long)a.K_pad;
     float m = __int_as_float(0x7f800000);
     for (int k = 4 * lane; k < a.K_pad; k += 128) {
@@ -603,7 +521,7 @@ __global__ void __launch_bounds__(256) shortlist_kernel(ShortlistArgs a) {
     int cnt = 0, mine = -1;                                 // lane l keeps the l-th survivor (l < kWorkCandCap)
     for (int k0 = 0; k0 < a.K_pad && !overflow; k0 += 32) {
       const int k = k0 + lane;
-      const bool hit = k < a.K && !(thr - sc[k] < 0.f);     // the epilogues' sign-bit test: a NaN score is a survivor
+      const bool hit = k < a.out.K && !(thr - sc[k] < 0.f); // the epilogues' sign-bit test: a NaN score is a survivor
       const uint32_t hm = __ballot_sync(0xffffffffu, hit);
       int pos = cnt + __popc(hm & ((1u << lane) - 1));
       // survivor number `pos` goes to lane `pos`
@@ -618,20 +536,10 @@ __global__ void __launch_bounds__(256) shortlist_kernel(ShortlistArgs a) {
       if (cnt > kWorkCandCap) overflow = true;
     }
     const int first = __shfl_sync(0xffffffffu, mine, 0);
-    const bool unique = !overflow && cnt == 1 && !a.force_rescore;
-    if (unique) {
-      if (lane == 0) {
-        a.idx_out[n] = (long long)first + a.code_base;
-        if (a.counts_out) atomicAdd(a.counts_out + first, 1ull);
-      }
+    if (!overflow && cnt == 1 && !a.out.force_rescore) {
+      if (lane == 0) settle_row(a.out, n, first);
     } else {
-      int slot = 0;
-      if (lane == 0) slot = atomicAdd(a.work_count, 1);
-      slot = __shfl_sync(0xffffffffu, slot, 0);
-      int* rec = reinterpret_cast<int*>(a.work + slot);
-      const int nc = (overflow || cnt == 0) ? kWorkCandCap + 1 : cnt;
-      if (lane == 0) { rec[0] = (int)n; rec[1] = nc; }
-      if (lane < kWorkCandCap && lane < cnt && !overflow) rec[4 + lane] = mine;
+      defer_row_warp(a.out, n, cnt, overflow, mine, lane);
     }
   }
 }

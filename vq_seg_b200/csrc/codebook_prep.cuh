@@ -87,7 +87,7 @@ __device__ inline void prep_pack(const float* __restrict__ E, int K, int D, unsi
     float v = k < K ? (ip ? 0.f : enorm[k] * s * cinv) : 60000.f;
     __half h1, h2, h3;
     if (k < K) {
-      if (!(v <= 60000.f)) { atomicOr(&hdr->flags, 1u); v = 60000.f; }
+      if (!(v <= 60000.f)) { atomicOr(&hdr->flags, kBlobFlagDeferAll); v = 60000.f; }
       h1 = __float2half_rn(v);
       const float r1 = v - __half2float(h1);
       h2 = __float2half_rn(r1);

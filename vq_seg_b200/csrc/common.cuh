@@ -56,7 +56,7 @@ struct BlobHeader {
   uint32_t max_abs_bits;            // max |e_kd| bits
   uint64_t off_enorm, off_image, off_aug;
   float    aug_c;        // power of two: s|e_k|^2 = aug_c * (h1 + h2 + h3), three fp16 limbs per code
-  uint32_t flags;        // bit 0: limbs not representable -> tensor-core filter must defer every row; bit 1: kBlobFlagIp
+  uint32_t flags;        // kBlobFlagDeferAll | kBlobFlagIp
   uint32_t max_de2_bits; // max_k |fp16(-2 s e_k) - (-2 s e_k)|^2 : the codebook operand's rounding error, exact
   uint64_t off_hash;
   uint32_t stale;        // guard scratch: set when a row fingerprint differs from the live weights
@@ -64,7 +64,8 @@ struct BlobHeader {
   uint32_t rebuilds;     // how often the guard had to rebuild the blob (diagnostic)
 };
 constexpr uint32_t kBlobMagic = 0x42535156u;
-constexpr uint32_t kBlobFlagIp = 2u;   // flags bit 1: inner-product blob (cosine codebook): no |e|^2 limbs in the score
+constexpr uint32_t kBlobFlagDeferAll = 1u;   // flags bit 0: |e|^2 limbs not representable -> the tensor-core filters defer every row
+constexpr uint32_t kBlobFlagIp = 2u;         // flags bit 1: inner-product blob (cosine codebook): no |e|^2 limbs in the score
 constexpr int kCodeBlock = 128;     // codes per packed tile
 constexpr int kDChunk = 64;         // dims per packed tile (64 fp16 = one 128-byte swizzle row)
 constexpr int kTileBytes = kCodeBlock * kDChunk * 2;

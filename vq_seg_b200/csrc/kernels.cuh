@@ -11,6 +11,16 @@ namespace vqseg {
 constexpr int kWorkCandCap = 8;
 struct alignas(16) WorkRec { int row; int cnt; int pad0; int pad1; int cand[kWorkCandCap]; };
 
+// What a tensor-core filter writes (filter_epilogue.cuh): the index and count of every row it decides, one WorkRec per
+// row it leaves to the rescoring pass.
+struct FilterOut {
+  int K;
+  long long* idx_out; unsigned long long* counts_out; long long code_base;
+  int force_rescore;              // 1 -> every row goes to the exact pass (sharded mode needs exact distances)
+  float slack_t2;                 // coefficient of the |x|^2-magnitude roundings in the filter's slack (common.cuh filter_slack)
+  WorkRec* work; int* work_count;
+};
+
 // ---- exact.cu: exact fp32 scorer (brute force over all codes, or the rescoring pass over the filter's short-lists)
 constexpr int kOvfSplitCap = 512;   // overflow rows up to which each row's codes are split over several blocks
 struct ExactArgs {
@@ -36,13 +46,7 @@ struct TcArgs {
   const unsigned char* blob;      // prepared codebook
   long long n_rows;
   int n_tiles, n_cc, n_dc;        // tiles of 128 rows, code chunks of 256, dim chunks of 64
-  int K;
-  float tau;                      // relative error bound of one fp16 x fp16 score vs the exact fp32 scorer
-  // outputs
-  long long* idx_out; unsigned long long* counts_out; long long code_base;
-  int force_rescore;              // 1 -> every row goes to the exact pass (sharded mode needs exact distances)
-  float slack_t2;                 // coefficient of the |x|^2-magnitude roundings in the filter's slack (common.cuh filter_slack)
-  WorkRec* work; int* work_count;
+  FilterOut out;
   long long* trace;               // optional (dev tool): [cta][role][256] clock64 stamps
 };
 int launch_pack(const float* E, int K, int D, unsigned char* blob, cudaStream_t st);
@@ -54,13 +58,9 @@ struct Tc2Args {
   const unsigned char* blob;
   long long n_rows;
   int n_ptiles, n_cc, n_dc;       // pair tiles of 256 rows, code chunks of 256, dim chunks of 64
-  int K, K_pad;
+  int K_pad;
   unsigned long long off_image, off_aug, off_enorm;
-  float tau;
-  long long* idx_out; unsigned long long* counts_out; long long code_base;
-  int force_rescore;
-  float slack_t2;                 // coefficient of the |x|^2-magnitude roundings in the filter's slack (common.cuh filter_slack)
-  WorkRec* work; int* work_count;
+  FilterOut out;
   long long* trace;
 };
 bool tc2_supported(int n_cc, int n_dc);
@@ -73,12 +73,9 @@ struct Tc3Args {
   const unsigned char* blob;
   int n_tiles, tiles_per_image;   // tiles of 128 pixels, never straddling an image
   int n_ptiles, n_cc, n_dc;       // pair tiles (two tiles), code chunks of 256, dim chunks of 64
-  int K, K_pad;
+  int K_pad;
   unsigned long long off_image, off_aug, off_enorm;
-  long long* idx_out; unsigned long long* counts_out; long long code_base;
-  int force_rescore;
-  float slack_t2;                 // coefficient of the |x|^2-magnitude roundings in the filter's slack (common.cuh filter_slack)
-  WorkRec* work; int* work_count;
+  FilterOut out;
   long long* trace;
 };
 bool tc3_supported(const Rows& x, int n_cc, int n_dc);
@@ -96,20 +93,16 @@ struct Tc4Args {
   float* part_norms;              //               [n_rows][2] {|x|^2, |fp16(x) - x|^2}
   const unsigned char* samp_img;  // MODE 2 (prepared samples): fp16 A tiles [row tile][dim chunk] x 16 KiB
   const float2* samp_norms;       //                            [padded rows] {|x|^2, |fp16(x) - x|^2}
-  int K, K_pad;
+  int K_pad;
   unsigned long long off_image, off_aug, off_enorm;
-  long long* idx_out; unsigned long long* counts_out; long long code_base;
-  int force_rescore;
-  float slack_t2;                 // coefficient of the |x|^2-magnitude roundings in the filter's slack (common.cuh filter_slack)
-  WorkRec* work; int* work_count;
+  FilterOut out;
   long long* trace;
 };
 // split-D mode's second step: per row the short-list over the summed scores (same rule as the filters' epilogues)
 struct ShortlistArgs {
-  const float* scores; const float* norms; long long n_rows; int K, K_pad, D;
+  const float* scores; const float* norms; long long n_rows; int K_pad, D;
   const unsigned char* blob;
-  long long* idx_out; unsigned long long* counts_out; long long code_base; int force_rescore; float slack_t2;
-  WorkRec* work; int* work_count;
+  FilterOut out;
 };
 int launch_shortlist(const ShortlistArgs& a, cudaStream_t st);
 int tc4_layout(const Rows& x, long long K_pad, int n_dc);   // 0: unsupported, 1: NCHW maps, 2: packed rows
