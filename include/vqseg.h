@@ -54,6 +54,8 @@ extern "C" {
 #define VQSEG_MODE_TRAIN       1     /* quantize = x + (E[idx] - x), two roundings (vq_img.py:236)     */
 #define VQSEG_MODE_TRAIN_AMP   2     /* as TRAIN with E[idx] rounded through fp16 (autocast matmul)    */
 #define VQSEG_MODE_EVAL_AMP    3
+#define VQSEG_MODE_TRAIN_AMP_BF16 4  /* as TRAIN with E[idx] rounded through bf16 (autocast matmul)   */
+#define VQSEG_MODE_EVAL_AMP_BF16  5  /* as EVAL with E[idx] rounded through bf16 (autocast matmul)    */
 
 int         vqseg_version(void);
 const char* vqseg_error_string(int code);

@@ -2,6 +2,7 @@
 // loss, its backward, per-code statistics for k-means, and small helpers.
 // Reference call sites are cited per kernel (paths relative to the reference root).
 #include <climits>
+#include <cuda_bf16.h>
 
 #include "common.cuh"
 
@@ -17,7 +18,18 @@ constexpr int kGTile = 32;       // dims per tile (128 x 32 tiles: 2048 blocks a
                                  // 128 x 64 tiles gave 1024 blocks on 888 slots, i.e. a second wave 15 % full)
 constexpr int kGPix = 128;       // pixels per tile
 
-__device__ __forceinline__ float round_fp16(float v) { return __half2float(__float2half_rn(v)); }
+constexpr bool gather_train(int mode) {
+  return mode == VQSEG_MODE_TRAIN || mode == VQSEG_MODE_TRAIN_AMP || mode == VQSEG_MODE_TRAIN_AMP_BF16;
+}
+// the code as the reference's autocast matmul produces it: rounded (to nearest even) through fp16 / bf16 per mode.
+// Signed zeros and infinities pass through, fp32 values beyond the type's range become inf of their sign, and a NaN
+// stays a NaN (the canonical one; its sign and payload carry no meaning).
+template <int MODE>
+__device__ __forceinline__ float round_code(float v) {
+  if (MODE == VQSEG_MODE_TRAIN_AMP || MODE == VQSEG_MODE_EVAL_AMP) return __half2float(__float2half_rn(v));
+  if (MODE == VQSEG_MODE_TRAIN_AMP_BF16 || MODE == VQSEG_MODE_EVAL_AMP_BF16) return __bfloat162float(__float2bfloat16_rn(v));
+  return v;
+}
 // pixel p of a tile lives in column (p % 4) * 32 + p / 4: a lane that owns pixels 4*lane .. 4*lane+3 then reads
 // columns lane, 32 + lane, 64 + lane, 96 + lane -- conflict-free (straight columns gave 4-way bank conflicts)
 __device__ __forceinline__ int gcol(int p) { return ((p & 3) << 5) | (p >> 2); }
@@ -74,8 +86,7 @@ __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float
   const long long n0 = (long long)blockIdx.x * kGPix;
   const int d0 = blockIdx.y * kGTile;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  constexpr bool kTrain = (MODE == VQSEG_MODE_TRAIN || MODE == VQSEG_MODE_TRAIN_AMP);
-  constexpr bool kAmp = (MODE == VQSEG_MODE_TRAIN_AMP || MODE == VQSEG_MODE_EVAL_AMP);
+  constexpr bool kTrain = gather_train(MODE);
   if (threadIdx.x < kGPix) {
     long long n = n0 + threadIdx.x;
     long long k = n < n_rows ? idx[n] : 0;
@@ -101,7 +112,7 @@ __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float
 #pragma unroll
     for (int u = 0; u < 8; ++u)
 #pragma unroll
-      for (int h = 0; h < kGTile / 32; ++h) tile[lane + 32 * h][gcol(p0 + 8 * u)] = kAmp ? round_fp16(v[u][h]) : v[u][h];
+      for (int h = 0; h < kGTile / 32; ++h) tile[lane + 32 * h][gcol(p0 + 8 * u)] = round_code<MODE>(v[u][h]);
   }
   __syncthreads();
   // phase 2: stream pixels; lane owns 4 consecutive pixels, warps take the dims round-robin
@@ -201,9 +212,8 @@ __global__ void __launch_bounds__(256) gather_ste_generic_kernel(Rows x, const f
     const float* xr = x.row(n);
     float* qr = q.row(n);
     for (int d = lane; d < D; d += 32) {
-      float e = __ldg(er + d);
-      if (MODE == VQSEG_MODE_TRAIN_AMP || MODE == VQSEG_MODE_EVAL_AMP) e = round_fp16(e);
-      if (MODE == VQSEG_MODE_EVAL || MODE == VQSEG_MODE_EVAL_AMP) {
+      const float e = round_code<MODE>(__ldg(er + d));
+      if (!gather_train(MODE)) {
         qr[(long long)d * q.sD] = e;
       } else {
         float xv = __ldg(xr + (long long)d * x.sD);
@@ -249,7 +259,7 @@ static int launch_gather(const Rows& x, const float* E, int K, const long long* 
                          float* loss_out, float* partial, size_t partial_cap, cudaStream_t st, int* ticket = nullptr,
                          const unsigned long long* counts = nullptr, float* usage_out = nullptr) {
   const long long n_rows = x.n_rows();
-  const bool train = (MODE == VQSEG_MODE_TRAIN || MODE == VQSEG_MODE_TRAIN_AMP);
+  const bool train = gather_train(MODE);
   const bool want_loss = train && loss_out != nullptr;
   const bool want_usage = ticket && counts && usage_out;
   // ticket (zeroed by the caller): the kernel's last block reduces the loss (and the code usage) itself
@@ -1167,7 +1177,7 @@ int vqseg_gather_ste_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_
                          float* q_out, int64_t qB, int64_t qP, int64_t qD,
                          float* loss_out, int mode, void* ws, size_t ws_bytes, void* stream) {
   if (!E || !idx || !q_out || B < 0 || P < 0 || D <= 0 || K <= 0) return VQSEG_EINVAL;
-  const bool train = mode == VQSEG_MODE_TRAIN || mode == VQSEG_MODE_TRAIN_AMP;
+  const bool train = gather_train(mode);
   if (train && !x) return VQSEG_EINVAL;
   if (B * P == 0) return 0;
   Rows xr{x, B, P, D, sB, sP, sD};
@@ -1182,6 +1192,8 @@ int vqseg_gather_ste_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_
     case VQSEG_MODE_EVAL_AMP:  return launch_gather<VQSEG_MODE_EVAL_AMP>(xr, E, (int)K, ix, qr, nullptr, partial, cap, st);
     case VQSEG_MODE_TRAIN:     return launch_gather<VQSEG_MODE_TRAIN>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st);
     case VQSEG_MODE_TRAIN_AMP: return launch_gather<VQSEG_MODE_TRAIN_AMP>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st);
+    case VQSEG_MODE_EVAL_AMP_BF16:  return launch_gather<VQSEG_MODE_EVAL_AMP_BF16>(xr, E, (int)K, ix, qr, nullptr, partial, cap, st);
+    case VQSEG_MODE_TRAIN_AMP_BF16: return launch_gather<VQSEG_MODE_TRAIN_AMP_BF16>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st);
   }
   return VQSEG_EINVAL;
 }
@@ -1194,7 +1206,7 @@ int vqseg_internal_gather_ticket(const float* x, int64_t B, int64_t P, int64_t D
                                  void* ws, size_t ws_bytes, void* stream, int* ticket,
                                  const int64_t* counts, float* usage_out) {
   if (!E || !idx || !q_out || B < 0 || P < 0 || D <= 0 || K <= 0) return VQSEG_EINVAL;
-  const bool train = mode == VQSEG_MODE_TRAIN || mode == VQSEG_MODE_TRAIN_AMP;
+  const bool train = gather_train(mode);
   if (train && !x) return VQSEG_EINVAL;
   if (B * P == 0) return 0;
   Rows xr{x, B, P, D, sB, sP, sD};
@@ -1210,6 +1222,8 @@ int vqseg_internal_gather_ticket(const float* x, int64_t B, int64_t P, int64_t D
     case VQSEG_MODE_EVAL_AMP:  return launch_gather<VQSEG_MODE_EVAL_AMP>(xr, E, (int)K, ix, qr, nullptr, partial, cap, st, ticket, cu, usage_out);
     case VQSEG_MODE_TRAIN:     return launch_gather<VQSEG_MODE_TRAIN>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st, ticket, cu, usage_out);
     case VQSEG_MODE_TRAIN_AMP: return launch_gather<VQSEG_MODE_TRAIN_AMP>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st, ticket, cu, usage_out);
+    case VQSEG_MODE_EVAL_AMP_BF16:  return launch_gather<VQSEG_MODE_EVAL_AMP_BF16>(xr, E, (int)K, ix, qr, nullptr, partial, cap, st, ticket, cu, usage_out);
+    case VQSEG_MODE_TRAIN_AMP_BF16: return launch_gather<VQSEG_MODE_TRAIN_AMP_BF16>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st, ticket, cu, usage_out);
   }
   return VQSEG_EINVAL;
 }

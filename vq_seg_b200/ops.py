@@ -13,6 +13,7 @@ from . import _native
 ALGO_AUTO, ALGO_EXACT, ALGO_TC, ALGO_TC_STREAM, ALGO_TC_PAIR, ALGO_TC_TMA, ALGO_TC_STREAM_PAIR = 0, 1, 2, 3, 4, 5, 6
 METRIC_IP = 0x100        # OR into an algo: first argmax of the fp32 inner product (cosine codebook) instead of cdist + argmin
 MODE_EVAL, MODE_TRAIN, MODE_TRAIN_AMP, MODE_EVAL_AMP = 0, 1, 2, 3
+MODE_TRAIN_AMP_BF16, MODE_EVAL_AMP_BF16 = 4, 5     # as MODE_*_AMP with E[idx] rounded through bf16 instead of fp16
 _last_assign_ws = None
 
 
@@ -946,25 +947,46 @@ class _FusedEvalForward(torch.autograd.Function):
         return ge, None, None, None, None
 
 
-def fused_forward(x, weight, blob, training, amp_fp16=False, algo=ALGO_AUTO):
-    """(q, idx, mse, usage) with autograd attached when needed."""
+def autocast_code_dtype(amp_compat=True):
+    """The dtype the reference's one-hot matmul (vq_img.py:169-170) rounds the gathered code through in this context:
+    torch.float16 / torch.bfloat16 under CUDA autocast to that dtype, None (exact fp32 codes) without autocast or
+    with amp_compat=False.  Indices are not affected: cdist is on autocast's fp32 list."""
+    if not (amp_compat and torch.is_autocast_enabled()):
+        return None
+    dtype = torch.get_autocast_dtype('cuda')
+    return dtype if dtype in (torch.float16, torch.bfloat16) else None
+
+
+def gather_mode(training, amp=None):
+    """The gather mode (MODE_*) that rounds the code through `amp`: None for exact fp32 codes, torch.float16 or
+    torch.bfloat16 (autocast_code_dtype()); False / True stand for None / torch.float16."""
+    if amp is None or amp is False:
+        return MODE_TRAIN if training else MODE_EVAL
+    if amp is True or amp == torch.float16:
+        return MODE_TRAIN_AMP if training else MODE_EVAL_AMP
+    if amp == torch.bfloat16:
+        return MODE_TRAIN_AMP_BF16 if training else MODE_EVAL_AMP_BF16
+    raise ValueError(f"the gathered code can be rounded through torch.float16 or torch.bfloat16, not {amp}")
+
+
+def fused_forward(x, weight, blob, training, amp=None, algo=ALGO_AUTO):
+    """(q, idx, mse, usage) with autograd attached when needed; `amp` as in gather_mode."""
+    mode = gather_mode(training, amp)
     if training:
-        mode = MODE_TRAIN_AMP if amp_fp16 else MODE_TRAIN
         if torch.is_grad_enabled() and x.requires_grad:
             return _FusedTrainForward.apply(x, weight.detach(), blob, mode, algo)
         return (_vq_forward_impl if _fast() else vq_forward)(x, weight, blob, mode, algo)
-    mode = MODE_EVAL_AMP if amp_fp16 else MODE_EVAL
     if torch.is_grad_enabled() and weight.requires_grad:
         return _FusedEvalForward.apply(weight, x, blob, mode, algo)
     return (_vq_forward_impl if _fast() else vq_forward)(x, weight, blob, mode, algo)
 
 
-def straight_through(x, codebook, idx, amp_fp16=False):
-    return _StraightThrough.apply(x, codebook, idx, MODE_TRAIN_AMP if amp_fp16 else MODE_TRAIN)
+def straight_through(x, codebook, idx, amp=None):
+    return _StraightThrough.apply(x, codebook, idx, gather_mode(True, amp))
 
 
-def eval_gather(codebook, x_like, idx, amp_fp16=False):
-    return _EvalGather.apply(codebook, x_like, idx, MODE_EVAL_AMP if amp_fp16 else MODE_EVAL)
+def eval_gather(codebook, x_like, idx, amp=None):
+    return _EvalGather.apply(codebook, x_like, idx, gather_mode(False, amp))
 
 
 def fast_assign(x, codebook, blob, algo=ALGO_AUTO, kblock=0, samples=None):

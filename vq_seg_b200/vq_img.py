@@ -279,7 +279,7 @@ class VectorQuantizer(nn.Module):
         self.codebook = codebook_class(embedding_dim=embedding_dim, num_embeddings=num_embeddings,
                                        kmeans_init=kmeans_init, kmeans_iters=kmeans_iters, decay=decay,
                                        eps=eps, num_codebook=num_codebook)
-        self.amp_compat = True    # under fp16 autocast round the gathered code through fp16 like the reference's matmul
+        self.amp_compat = True    # round the gathered code through the fp16 / bf16 autocast dtype like the reference's matmul
         self._graphs = None       # opt-in CUDA-graph cache of the no-grad forward (enable_cuda_graphs)
 
     def enable_cuda_graphs(self, max_entries: int = 16):
@@ -300,9 +300,9 @@ class VectorQuantizer(nn.Module):
         return self
 
     def _graph_forward(self, x):
-        amp16 = bool(self.amp_compat and torch.is_autocast_enabled() and torch.get_autocast_dtype('cuda') == torch.float16)
+        amp = ops.autocast_code_dtype(self.amp_compat)
         w = self.codebook.embedding.weight
-        key = (x.data_ptr(), tuple(x.shape), tuple(x.stride()), x.dtype, amp16, w.data_ptr(), torch.cuda.current_device())
+        key = (x.data_ptr(), tuple(x.shape), tuple(x.stride()), x.dtype, amp, w.data_ptr(), torch.cuda.current_device())
         ent = self._graphs.get(key)
         if ent is None:
             if len(self._graphs) >= self._graphs_max:
@@ -347,8 +347,7 @@ class VectorQuantizer(nn.Module):
         device = x.device
         xv = x.reshape(b, c, h * w).permute(0, 2, 1)          # the 'b c h w -> b (h w) c' VIEW, no copy
         cb = self.codebook
-        amp16 = bool(self.amp_compat and torch.is_autocast_enabled()
-                     and torch.get_autocast_dtype('cuda') == torch.float16)
+        amp = ops.autocast_code_dtype(self.amp_compat)
         cosine = isinstance(cb, CosinesimCodebook)
         if cb.kmeans_init and self.training and not cb.initted:
             cb._kmeans_init(ops.l2norm_rows(xv) if cosine else xv, cosine=cosine)
@@ -356,15 +355,15 @@ class VectorQuantizer(nn.Module):
             idx, counts = cb.lookup(xv)
             code_usage = ops.fast_code_usage(counts)
             if self.training:
-                quantize, mse = ops.straight_through(xv, cb.embedding.weight.detach(), idx, amp16)
+                quantize, mse = ops.straight_through(xv, cb.embedding.weight.detach(), idx, amp)
             else:
-                quantize, mse = ops.eval_gather(cb.embedding.weight, xv, idx, amp16), None
+                quantize, mse = ops.eval_gather(cb.embedding.weight, xv, idx, amp), None
         else:
             # Euclidean: lookup + gather + STE + mse + usage are enqueued by one host call
             if xv.shape[-1] != cb.embedding_dim:
                 raise RuntimeError(f"X1 and X2 must have the same number of columns. X1: {xv.shape[-1]} X2: {cb.embedding_dim}")
             blob = cb._prepared() if cb.algo != ops.ALGO_EXACT else None
-            quantize, idx, mse, code_usage = ops.fused_forward(xv, cb.embedding.weight, blob, self.training, amp16, cb.algo)
+            quantize, idx, mse, code_usage = ops.fused_forward(xv, cb.embedding.weight, blob, self.training, amp, cb.algo)
         # loss (vq_img.py:230,239-241): [0.] + mse * w.  0 + v and v * 1 are exact in fp32, so for the default weight
         # the kernel's (1,) mse IS the loss (no fill / mul / add launches); eval: the kernel's zeroed (1,) output
         if self.training and self.commitment_weight > 0 and (mse.requires_grad or not torch.is_grad_enabled()):

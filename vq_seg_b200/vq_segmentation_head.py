@@ -144,17 +144,16 @@ class VQSegmentationHead(nn.Module):
             distance, embed_idx, counts = cb.lookup(xv)
         code_usage = ops.fast_code_usage(counts)
         loss = torch.zeros(1, device=x.device, dtype=torch.float32, requires_grad=self.training)
-        # under fp16 autocast the reference's one_hot @ weight is an fp16 matmul: the gathered code is half(E[idx])
-        # (same switch as VectorQuantizer.amp_compat; bf16 autocast is not emulated: fp32 codes)
-        amp16 = bool(getattr(self, "amp_compat", True) and torch.is_autocast_enabled()
-                     and torch.get_autocast_dtype('cuda') == torch.float16)
+        # under fp16 / bf16 autocast the reference's one_hot @ weight is a matmul in that dtype: the gathered code is
+        # E[idx] rounded through it (same switch as VectorQuantizer.amp_compat)
+        amp = ops.autocast_code_dtype(getattr(self, "amp_compat", True))
         if self.training:
             # quantize = x + (quantize - x).detach(); loss = mse(quantize.detach(), x) * w   (:237-242)
-            quantize, mse = ops.straight_through(xv, cb.embedding.weight.detach(), embed_idx, amp16)
+            quantize, mse = ops.straight_through(xv, cb.embedding.weight.detach(), embed_idx, amp)
             if self.commitment_weight > 0:
                 loss = loss + mse * self.commitment_weight
         else:
-            quantize = ops.eval_gather(cb.embedding.weight, xv, embed_idx, amp16)      # one_hot @ weight (:170-171)
+            quantize = ops.eval_gather(cb.embedding.weight, xv, embed_idx, amp)      # one_hot @ weight (:170-171)
         # the maps are stored as (B, K, HW): 'b (h w) c -> b c h w' is a view of them
         if fused:
             score = score_bpk.permute(0, 2, 1).reshape(b, -1, h, w)
