@@ -56,6 +56,10 @@ extern "C" {
 #define VQSEG_MODE_EVAL_AMP    3
 #define VQSEG_MODE_TRAIN_AMP_BF16 4  /* as TRAIN with E[idx] rounded through bf16 (autocast matmul)   */
 #define VQSEG_MODE_EVAL_AMP_BF16  5  /* as EVAL with E[idx] rounded through bf16 (autocast matmul)    */
+#define VQSEG_MODE_ROTATE   0x10     /* OR into a TRAIN mode (opt-in rotation trick, see vqseg_rotate_bwd_f32): quantize = c,
+                                        the code after the mode's rounding (bit-equal to the matching EVAL mode's output),
+                                        not x + (c - x); the loss is mean((c - x)^2) with the same fixed reduction.  With an
+                                        EVAL mode, or with any other unknown bit, the gather returns VQSEG_EINVAL. */
 
 int         vqseg_version(void);
 const char* vqseg_error_string(int code);
@@ -154,6 +158,30 @@ int    vqseg_ste_bwd_f32(const float* g_q, int64_t gB, int64_t gP, int64_t gD,
                          const float* coef_dev, float coef_scale,
                          float* gx, int64_t oB, int64_t oP, int64_t oD,
                          int64_t B, int64_t P, int64_t D, void* stream);
+
+/* ---- backward w.r.t. x of the rotation trick: OPT-IN EXTENSION, no reference counterpart ------------------------
+ * Fifty et al., "Restructuring Vector Quantization with the Rotation Trick" (arXiv 2410.06424, §4.2); rotation_trick of
+ * lucidrains/vector-quantize-pytorch.  For the forward of a TRAIN | VQSEG_MODE_ROTATE gather (quantize = c), per row n
+ * with x the input, c the SAVED quantize (never E[idx]: the EMA update may have rewritten E in between), g = g_q (0 when
+ * g_q is null) and lam = coef_scale * (*coef_dev) (0 when coef_dev is null; the convention of vqseg_ste_bwd_f32):
+ *   gx = s (g - 2 (w.g) w + 2 (q^.g) u) + lam (x - c), the gradient of quantize = s (x - 2 (x.w) w + 2 (x.u) q^) with
+ *        u = x/|x|, q^ = c/|c|, w = (u + q^)/|u + q^| and s = |c|/|x| held constant (the forward value is c), plus the
+ *        commitment term.  Evaluated in fp32 with IEEE sqrt and division and no contraction as:
+ *   xx, cc, xc, xg, cg = row sums of x*x, c*c, x*c, x*g, c*g, each as eight chains a_l = fl(fl(p_d) + a_l) over
+ *        d = l, l+8, l+16, ... ascending (l = 0..7), then ((a0 + a1) + (a2 + a3)) + ((a4 + a5) + (a6 + a7));
+ *   xx == 0 or cc == 0:  alpha = 1, beta = lam, gamma = -lam  (the straight-through gradient);
+ *   else  nx = sqrt(xx), nc = sqrt(cc), s = nc / nx, rho = (xc / nx) / nc, a = xg / nx, b = cg / nc, t = 1 + rho,
+ *         h = (a + b) / t if t > 0 else 0  (antipodal rows: the reflection),
+ *         alpha = s, beta = ((s (2b - h)) / nx) + lam, gamma = (-((s h) / nc)) - lam;
+ *   gx_d = ((alpha g_d) + (beta x_d)) + (gamma c_d).
+ * The order of the sums does not depend on the strides: gx is bit-identical for every layout of the inputs and the
+ * output and from run to run (no atomics).  Arguments as in vqseg_ste_bwd_f32; x and q are required.  16 N D bytes. */
+int    vqseg_rotate_bwd_f32(const float* g_q, int64_t gB, int64_t gP, int64_t gD,
+                            const float* x, int64_t sB, int64_t sP, int64_t sD,
+                            const float* q, int64_t qB, int64_t qP, int64_t qD,
+                            const float* coef_dev, float coef_scale,
+                            float* gx, int64_t oB, int64_t oP, int64_t oD,
+                            int64_t B, int64_t P, int64_t D, void* stream);
 
 /* gradient of the eval-mode gather w.r.t. the codebook: gE[idx[n], :] += g_q[n, :]              */
 int    vqseg_gather_bwd_codebook_f32(const float* g_q, int64_t B, int64_t P, int64_t D,

@@ -33,6 +33,8 @@ SIGNATURES = {
                                   ci, ci, ci, vp, sz, vp, vp]),
     "vqseg_ste_bwd_f32": (ci, [vp, i64, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64, vp, f32,
                                vp, i64, i64, i64, i64, i64, i64, vp]),
+    "vqseg_rotate_bwd_f32": (ci, [vp, i64, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64, vp, f32,
+                                  vp, i64, i64, i64, i64, i64, i64, vp]),
     "vqseg_gather_bwd_codebook_f32": (ci, [vp, i64, i64, i64, i64, i64, i64, vp, vp, i64, vp]),
     "vqseg_code_stats_workspace_bytes": (sz, [i64, i64, i64, ci]),
     "vqseg_code_stats_f32": (ci, [vp, i64, i64, i64, i64, i64, i64, vp, i64, vp, vp, ci, vp, sz, vp]),

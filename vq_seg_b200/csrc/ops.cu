@@ -18,7 +18,11 @@ constexpr int kGTile = 32;       // dims per tile (128 x 32 tiles: 2048 blocks a
                                  // 128 x 64 tiles gave 1024 blocks on 888 slots, i.e. a second wave 15 % full)
 constexpr int kGPix = 128;       // pixels per tile
 
+// VQSEG_MODE_ROTATE is ORed into a train mode: it changes what is written (c instead of x + (c - x)), not how the code
+// is rounded or that x is read
+constexpr int base_mode(int mode) { return mode & ~VQSEG_MODE_ROTATE; }
 constexpr bool gather_train(int mode) {
+  mode = base_mode(mode);
   return mode == VQSEG_MODE_TRAIN || mode == VQSEG_MODE_TRAIN_AMP || mode == VQSEG_MODE_TRAIN_AMP_BF16;
 }
 // the code as the reference's autocast matmul produces it: rounded (to nearest even) through fp16 / bf16 per mode.
@@ -26,8 +30,9 @@ constexpr bool gather_train(int mode) {
 // stays a NaN (the canonical one; its sign and payload carry no meaning).
 template <int MODE>
 __device__ __forceinline__ float round_code(float v) {
-  if (MODE == VQSEG_MODE_TRAIN_AMP || MODE == VQSEG_MODE_EVAL_AMP) return __half2float(__float2half_rn(v));
-  if (MODE == VQSEG_MODE_TRAIN_AMP_BF16 || MODE == VQSEG_MODE_EVAL_AMP_BF16) return __bfloat162float(__float2bfloat16_rn(v));
+  constexpr int M = base_mode(MODE);
+  if (M == VQSEG_MODE_TRAIN_AMP || M == VQSEG_MODE_EVAL_AMP) return __half2float(__float2half_rn(v));
+  if (M == VQSEG_MODE_TRAIN_AMP_BF16 || M == VQSEG_MODE_EVAL_AMP_BF16) return __bfloat162float(__float2bfloat16_rn(v));
   return v;
 }
 // pixel p of a tile lives in column (p % 4) * 32 + p / 4: a lane that owns pixels 4*lane .. 4*lane+3 then reads
@@ -87,6 +92,7 @@ __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float
   const int d0 = blockIdx.y * kGTile;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   constexpr bool kTrain = gather_train(MODE);
+  constexpr bool kRot = (MODE & VQSEG_MODE_ROTATE) != 0;     // write c itself; the loss term is (c - x)^2
   if (threadIdx.x < kGPix) {
     long long n = n0 + threadIdx.x;
     long long k = n < n_rows ? idx[n] : 0;
@@ -145,8 +151,10 @@ __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float
           float4 o = e;
           if (kTrain) {
             const float4 xv = xr[u];
-            o.x = __fadd_rn(xv.x, __fsub_rn(e.x, xv.x)); o.y = __fadd_rn(xv.y, __fsub_rn(e.y, xv.y));   // x + (q - x)
-            o.z = __fadd_rn(xv.z, __fsub_rn(e.z, xv.z)); o.w = __fadd_rn(xv.w, __fsub_rn(e.w, xv.w));
+            if (!kRot) {
+              o.x = __fadd_rn(xv.x, __fsub_rn(e.x, xv.x)); o.y = __fadd_rn(xv.y, __fsub_rn(e.y, xv.y));   // x + (q - x)
+              o.z = __fadd_rn(xv.z, __fsub_rn(e.z, xv.z)); o.w = __fadd_rn(xv.w, __fsub_rn(e.w, xv.w));
+            }
             float f;
             f = __fsub_rn(o.x, xv.x); acc = __fmaf_rn(f, f, acc); f = __fsub_rn(o.y, xv.y); acc = __fmaf_rn(f, f, acc);
             f = __fsub_rn(o.z, xv.z); acc = __fmaf_rn(f, f, acc); f = __fsub_rn(o.w, xv.w); acc = __fmaf_rn(f, f, acc);
@@ -170,7 +178,7 @@ __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float
             float o = e;
             if (kTrain) {
               float xv = __ldg(xb + (long long)(d0 + d) * x.sD);
-              o = __fadd_rn(xv, __fsub_rn(e, xv));
+              if (!kRot) o = __fadd_rn(xv, __fsub_rn(e, xv));
               float f = __fsub_rn(o, xv);
               acc = __fmaf_rn(f, f, acc);
             }
@@ -217,7 +225,7 @@ __global__ void __launch_bounds__(256) gather_ste_generic_kernel(Rows x, const f
         qr[(long long)d * q.sD] = e;
       } else {
         float xv = __ldg(xr + (long long)d * x.sD);
-        float qs = __fadd_rn(xv, __fsub_rn(e, xv));
+        float qs = (MODE & VQSEG_MODE_ROTATE) ? e : __fadd_rn(xv, __fsub_rn(e, xv));
         qr[(long long)d * q.sD] = qs;
         float df = __fsub_rn(qs, xv);
         acc = __fmaf_rn(df, df, acc);
@@ -330,6 +338,183 @@ __global__ void __launch_bounds__(256) ste_bwd_flat_kernel(const float4* __restr
       r.z = __fmaf_rn(coef, __fsub_rn(xv.z, qv.z), r.z); r.w = __fmaf_rn(coef, __fsub_rn(xv.w, qv.w), r.w);
     }
     o[i] = r;
+  }
+}
+
+// =================================================================================================
+// backward w.r.t. x of the rotation trick (opt-in extension, no reference counterpart: Fifty et al., arXiv 2410.06424
+// §4.2; rotation_trick of lucidrains/vector-quantize-pytorch).  Per row gx = alpha g + beta x + gamma c, with the
+// coefficients of vqseg.h from five row sums.  Each sum is eight chains a_l over d = l, l + 8, ... (ascending), combined
+// ((a0 + a1) + (a2 + a3)) + ((a4 + a5) + (a6 + a7)); all three layout paths below keep that order, so gx is the same
+// bits whatever the strides.
+// =================================================================================================
+constexpr int kRotSums = 5;                     // x.x, c.c, x.c, x.g, c.g
+__device__ __forceinline__ void rot_accum(float (&a)[kRotSums], float x, float c, float g) {
+  a[0] = __fadd_rn(a[0], __fmul_rn(x, x));
+  a[1] = __fadd_rn(a[1], __fmul_rn(c, c));
+  a[2] = __fadd_rn(a[2], __fmul_rn(x, c));
+  a[3] = __fadd_rn(a[3], __fmul_rn(x, g));
+  a[4] = __fadd_rn(a[4], __fmul_rn(c, g));
+}
+__device__ __forceinline__ float rot_tree(const float (&a)[8]) {
+  return __fadd_rn(__fadd_rn(__fadd_rn(a[0], a[1]), __fadd_rn(a[2], a[3])),
+                   __fadd_rn(__fadd_rn(a[4], a[5]), __fadd_rn(a[6], a[7])));
+}
+// (alpha, beta, gamma) from the row sums; a zero x or c row takes the straight-through gradient
+__device__ __forceinline__ float3 rot_coefs(const float (&s)[kRotSums], float lam) {
+  if (s[0] == 0.f || s[1] == 0.f) return make_float3(1.f, lam, -lam);
+  const float nx = __fsqrt_rn(s[0]), nc = __fsqrt_rn(s[1]);
+  const float sc = __fdiv_rn(nc, nx);
+  const float rho = __fdiv_rn(__fdiv_rn(s[2], nx), nc);
+  const float a = __fdiv_rn(s[3], nx), b = __fdiv_rn(s[4], nc);
+  const float t = __fadd_rn(1.f, rho);
+  const float h = t > 0.f ? __fdiv_rn(__fadd_rn(a, b), t) : 0.f;     // antipodal rows: w = 0, the reflection
+  const float beta = __fadd_rn(__fdiv_rn(__fmul_rn(sc, __fsub_rn(__fmul_rn(2.f, b), h)), nx), lam);
+  const float gamma = __fsub_rn(-__fdiv_rn(__fmul_rn(sc, h), nc), lam);
+  return make_float3(sc, beta, gamma);
+}
+__device__ __forceinline__ float rot_out(float3 k, float g, float x, float c) {
+  return __fadd_rn(__fadd_rn(__fmul_rn(k.x, g), __fmul_rn(k.y, x)), __fmul_rn(k.z, c));
+}
+
+// Pixel-contiguous maps (sP == 1): a block owns 32 neighbouring pixels of one image (lane = pixel) and stages chunks of
+// up to kRotChunk channels of x, c and g in shared memory (coalesced 128-byte lines); warp w runs the chains of class
+// d = w (mod 8), the tree combines them through shared memory, and gx is written from the staged tile when the whole
+// row fits (D <= kRotChunk: x, c and g are read from HBM once), else from a second read.
+// (Tried: each warp holding its 32 channels of x, c and g in registers instead of the 96 KB tile, 96 loads in flight per
+// thread: 70 us against 62 on the config-2 map, and slower on every config-1 layer.)
+constexpr int kRotChunk = 256;
+__global__ void __launch_bounds__(256) rotate_bwd_px_kernel(View g, View x, View q, const float* __restrict__ coef_dev,
+                                                            float coef_scale, RowsOut o, int ch) {
+  extern __shared__ float rot_tile[];            // [3][ch][32]: x, c, g
+  __shared__ float s_part[kRotSums][8][32];
+  __shared__ float s_k[3][32];
+  float* tx = rot_tile;
+  float* tc = rot_tile + ch * 32;
+  float* tg = rot_tile + 2 * ch * 32;
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int D = (int)o.D;
+  const float lam = coef_dev ? __fmul_rn(coef_scale, __ldg(coef_dev)) : 0.f;
+  const long long groups_per_image = (o.P + 31) / 32;
+  for (long long gidx = blockIdx.x; gidx < o.B * groups_per_image; gidx += gridDim.x) {
+    const long long b = gidx / groups_per_image, p = (gidx % groups_per_image) * 32 + lane;
+    const bool on = p < o.P;
+    const long long pp = on ? p : 0;
+    const float* xp = x.ptr + b * x.sB + pp * x.sP;
+    const float* cp = q.ptr + b * q.sB + pp * q.sP;
+    const float* gp = g.ptr ? g.ptr + b * g.sB + pp * g.sP : nullptr;
+    float a[kRotSums] = {0.f, 0.f, 0.f, 0.f, 0.f};
+    for (int d0 = 0; d0 < D; d0 += ch) {         // ch % 8 == 0: class w stays with warp w across chunks
+      const int dn = min(ch, D - d0);
+      __syncthreads();
+#pragma unroll 4
+      for (int j = wib; j < dn; j += 8) {
+        const long long d = d0 + j;
+        tx[j * 32 + lane] = on ? __ldg(xp + d * x.sD) : 0.f;
+        tc[j * 32 + lane] = on ? __ldg(cp + d * q.sD) : 0.f;
+        tg[j * 32 + lane] = (on && gp) ? __ldg(gp + d * g.sD) : 0.f;
+      }
+      __syncthreads();
+      for (int j = wib; j < dn; j += 8) rot_accum(a, tx[j * 32 + lane], tc[j * 32 + lane], tg[j * 32 + lane]);
+    }
+#pragma unroll
+    for (int i = 0; i < kRotSums; ++i) s_part[i][wib][lane] = a[i];
+    __syncthreads();
+    if (wib == 0) {
+      float s[kRotSums];
+#pragma unroll
+      for (int i = 0; i < kRotSums; ++i) {
+        float v[8];
+#pragma unroll
+        for (int w = 0; w < 8; ++w) v[w] = s_part[i][w][lane];
+        s[i] = rot_tree(v);
+      }
+      const float3 k = rot_coefs(s, lam);
+      s_k[0][lane] = k.x; s_k[1][lane] = k.y; s_k[2][lane] = k.z;
+    }
+    __syncthreads();
+    const float3 k = make_float3(s_k[0][lane], s_k[1][lane], s_k[2][lane]);
+    if (on) {
+      float* op = o.ptr + b * o.sB + p * o.sP;
+      if (D <= ch) {
+        for (int d = wib; d < D; d += 8)
+          op[(long long)d * o.sD] = rot_out(k, tg[d * 32 + lane], tx[d * 32 + lane], tc[d * 32 + lane]);
+      } else {
+        for (int d = wib; d < D; d += 8) {
+          const float gv = gp ? __ldg(gp + (long long)d * g.sD) : 0.f;
+          op[(long long)d * o.sD] = rot_out(k, gv, __ldg(xp + (long long)d * x.sD), __ldg(cp + (long long)d * q.sD));
+        }
+      }
+    }
+  }
+}
+
+// Packed rows (sD == 1 of x): eight lanes per row, lane l runs chain l; the butterfly over lanes 1, 2, 4 is the tree.
+__global__ void __launch_bounds__(256) rotate_bwd_rows_kernel(View g, View x, View q, const float* __restrict__ coef_dev,
+                                                              float coef_scale, RowsOut o) {
+  const int l8 = threadIdx.x & 7;
+  const long long n = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 3;
+  const bool on = n < o.B * o.P;                 // (whole groups of 8 lanes are on or off together)
+  const int D = on ? (int)o.D : 0;
+  long long b, p;
+  split_row(on ? n : 0, o.P, b, p);
+  const float* xr = x.ptr + b * x.sB + p * x.sP;
+  const float* cr = q.ptr + b * q.sB + p * q.sP;
+  const float* gr = g.ptr ? g.ptr + b * g.sB + p * g.sP : nullptr;
+  float a[kRotSums] = {0.f, 0.f, 0.f, 0.f, 0.f};
+  for (int d = l8; d < D; d += 8)
+    rot_accum(a, __ldg(xr + (long long)d * x.sD), __ldg(cr + (long long)d * q.sD), gr ? __ldg(gr + (long long)d * g.sD) : 0.f);
+#pragma unroll
+  for (int i = 0; i < kRotSums; ++i)
+#pragma unroll
+    for (int m = 1; m < 8; m <<= 1) a[i] = __fadd_rn(a[i], __shfl_xor_sync(0xffffffffu, a[i], m));
+  const float lam = coef_dev ? __fmul_rn(coef_scale, __ldg(coef_dev)) : 0.f;
+  const float3 k = rot_coefs(a, lam);
+  float* orow = o.ptr + b * o.sB + p * o.sP;
+  for (int d = l8; d < D; d += 8) {
+    const float gv = gr ? __ldg(gr + (long long)d * g.sD) : 0.f;
+    orow[(long long)d * o.sD] = rot_out(k, gv, __ldg(xr + (long long)d * x.sD), __ldg(cr + (long long)d * q.sD));
+  }
+}
+
+// Any other strides (CNHW-like views with sP > 1 and sD > 1): one thread per row, eight chains in registers.
+__global__ void __launch_bounds__(256) rotate_bwd_strided_kernel(View g, View x, View q, const float* __restrict__ coef_dev,
+                                                                 float coef_scale, RowsOut o) {
+  const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= o.B * o.P) return;
+  const int D = (int)o.D;
+  long long b, p;
+  split_row(n, o.P, b, p);
+  const float* xr = x.ptr + b * x.sB + p * x.sP;
+  const float* cr = q.ptr + b * q.sB + p * q.sP;
+  const float* gr = g.ptr ? g.ptr + b * g.sB + p * g.sP : nullptr;
+  float a[kRotSums][8];
+#pragma unroll
+  for (int i = 0; i < kRotSums; ++i)
+#pragma unroll
+    for (int l = 0; l < 8; ++l) a[i][l] = 0.f;
+  for (int d0 = 0; d0 < D; d0 += 8) {
+#pragma unroll
+    for (int l = 0; l < 8; ++l) {
+      const long long d = d0 + l;
+      if (d < D) {
+        const float xv = __ldg(xr + d * x.sD), cv = __ldg(cr + d * q.sD), gv = gr ? __ldg(gr + d * g.sD) : 0.f;
+        float t[kRotSums] = {a[0][l], a[1][l], a[2][l], a[3][l], a[4][l]};
+        rot_accum(t, xv, cv, gv);
+#pragma unroll
+        for (int i = 0; i < kRotSums; ++i) a[i][l] = t[i];
+      }
+    }
+  }
+  float s[kRotSums];
+#pragma unroll
+  for (int i = 0; i < kRotSums; ++i) s[i] = rot_tree(a[i]);
+  const float lam = coef_dev ? __fmul_rn(coef_scale, __ldg(coef_dev)) : 0.f;
+  const float3 k = rot_coefs(s, lam);
+  float* orow = o.ptr + b * o.sB + p * o.sP;
+  for (long long d = 0; d < D; ++d) {
+    const float gv = gr ? __ldg(gr + d * g.sD) : 0.f;
+    orow[d * o.sD] = rot_out(k, gv, __ldg(xr + d * x.sD), __ldg(cr + d * q.sD));
   }
 }
 
@@ -1194,6 +1379,9 @@ int vqseg_gather_ste_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_
     case VQSEG_MODE_TRAIN_AMP: return launch_gather<VQSEG_MODE_TRAIN_AMP>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st);
     case VQSEG_MODE_EVAL_AMP_BF16:  return launch_gather<VQSEG_MODE_EVAL_AMP_BF16>(xr, E, (int)K, ix, qr, nullptr, partial, cap, st);
     case VQSEG_MODE_TRAIN_AMP_BF16: return launch_gather<VQSEG_MODE_TRAIN_AMP_BF16>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st);
+    case VQSEG_MODE_TRAIN | VQSEG_MODE_ROTATE: return launch_gather<VQSEG_MODE_TRAIN | VQSEG_MODE_ROTATE>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st);
+    case VQSEG_MODE_TRAIN_AMP | VQSEG_MODE_ROTATE: return launch_gather<VQSEG_MODE_TRAIN_AMP | VQSEG_MODE_ROTATE>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st);
+    case VQSEG_MODE_TRAIN_AMP_BF16 | VQSEG_MODE_ROTATE: return launch_gather<VQSEG_MODE_TRAIN_AMP_BF16 | VQSEG_MODE_ROTATE>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st);
   }
   return VQSEG_EINVAL;
 }
@@ -1224,6 +1412,9 @@ int vqseg_internal_gather_ticket(const float* x, int64_t B, int64_t P, int64_t D
     case VQSEG_MODE_TRAIN_AMP: return launch_gather<VQSEG_MODE_TRAIN_AMP>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st, ticket, cu, usage_out);
     case VQSEG_MODE_EVAL_AMP_BF16:  return launch_gather<VQSEG_MODE_EVAL_AMP_BF16>(xr, E, (int)K, ix, qr, nullptr, partial, cap, st, ticket, cu, usage_out);
     case VQSEG_MODE_TRAIN_AMP_BF16: return launch_gather<VQSEG_MODE_TRAIN_AMP_BF16>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st, ticket, cu, usage_out);
+    case VQSEG_MODE_TRAIN | VQSEG_MODE_ROTATE: return launch_gather<VQSEG_MODE_TRAIN | VQSEG_MODE_ROTATE>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st, ticket, cu, usage_out);
+    case VQSEG_MODE_TRAIN_AMP | VQSEG_MODE_ROTATE: return launch_gather<VQSEG_MODE_TRAIN_AMP | VQSEG_MODE_ROTATE>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st, ticket, cu, usage_out);
+    case VQSEG_MODE_TRAIN_AMP_BF16 | VQSEG_MODE_ROTATE: return launch_gather<VQSEG_MODE_TRAIN_AMP_BF16 | VQSEG_MODE_ROTATE>(xr, E, (int)K, ix, qr, loss_out, partial, cap, st, ticket, cu, usage_out);
   }
   return VQSEG_EINVAL;
 }
@@ -1256,6 +1447,40 @@ int vqseg_ste_bwd_f32(const float* g_q, int64_t gB, int64_t gP, int64_t gD,
   RowsOut o{gx, B, P, D, oB, oP, oD};
   bool px_fast = (oP == 1);
   ste_bwd_kernel<<<grid_for(B * P * D, 256, 16), 256, 0, (cudaStream_t)stream>>>(g, xv, qv, coef_dev, coef_scale, o, px_fast);
+  VQSEG_LAUNCH_CHECK();
+  return 0;
+}
+
+int vqseg_rotate_bwd_f32(const float* g_q, int64_t gB, int64_t gP, int64_t gD,
+                         const float* x, int64_t sB, int64_t sP, int64_t sD,
+                         const float* q, int64_t qB, int64_t qP, int64_t qD,
+                         const float* coef_dev, float coef_scale,
+                         float* gx, int64_t oB, int64_t oP, int64_t oD,
+                         int64_t B, int64_t P, int64_t D, void* stream) {
+  if (!gx || !x || !q || B < 0 || P < 0 || D <= 0 || D >= (1ll << 31)) return VQSEG_EINVAL;
+  const long long n_rows = B * P;
+  if (n_rows == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  View g{g_q, gB, gP, gD}, xv{x, sB, sP, sD}, qv{q, qB, qP, qD};
+  RowsOut o{gx, B, P, D, oB, oP, oD};
+  // the path follows x's layout (the order of the sums does not depend on it)
+  if (sD == 1) {
+    rotate_bwd_rows_kernel<<<(unsigned)((n_rows * 8 + 255) / 256), 256, 0, st>>>(g, xv, qv, coef_dev, coef_scale, o);
+  } else if (sP == 1) {
+    const int ch = (int)(D < kRotChunk ? round_up(D, 8) : kRotChunk);
+    const size_t smem = (size_t)3 * ch * 32 * sizeof(float);
+    static size_t configured[kMaxDevices] = {0};
+    static bool carved[kMaxDevices] = {false};
+    if (int rc = ensure_dynamic_smem(rotate_bwd_px_kernel, smem, configured)) return rc;
+    if (!carved[current_device()]) {             // 96 KB per block at D >= 256: ask for the large carve-out
+      cudaFuncSetAttribute(rotate_bwd_px_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+      carved[current_device()] = true;
+    }
+    const long long groups = B * ((P + 31) / 32), cap = (long long)num_sms() * 8;
+    rotate_bwd_px_kernel<<<(unsigned)(groups < cap ? groups : cap), 256, smem, st>>>(g, xv, qv, coef_dev, coef_scale, o, ch);
+  } else {
+    rotate_bwd_strided_kernel<<<(unsigned)((n_rows + 255) / 256), 256, 0, st>>>(g, xv, qv, coef_dev, coef_scale, o);
+  }
   VQSEG_LAUNCH_CHECK();
   return 0;
 }

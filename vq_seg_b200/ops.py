@@ -14,6 +14,7 @@ ALGO_AUTO, ALGO_EXACT, ALGO_TC, ALGO_TC_STREAM, ALGO_TC_PAIR, ALGO_TC_TMA, ALGO_
 METRIC_IP = 0x100        # OR into an algo: first argmax of the fp32 inner product (cosine codebook) instead of cdist + argmin
 MODE_EVAL, MODE_TRAIN, MODE_TRAIN_AMP, MODE_EVAL_AMP = 0, 1, 2, 3
 MODE_TRAIN_AMP_BF16, MODE_EVAL_AMP_BF16 = 4, 5     # as MODE_*_AMP with E[idx] rounded through bf16 instead of fp16
+MODE_ROTATE = 0x10       # OR into a train mode: quantize = E[idx] itself, gradient to x by the rotation trick (rotate_bwd)
 _last_assign_ws = None
 
 
@@ -275,6 +276,43 @@ ste_bwd = torch.library.custom_op("vqseg::ste_bwd", mutates_args=())(_ste_bwd_im
 @ste_bwd.register_fake
 def _(grad_q, x, q_ste, grad_mse, coef_scale):
     return torch.empty_like(x, dtype=torch.float32)
+
+
+def _rotate_bwd_impl(grad_q: Optional[torch.Tensor], x: torch.Tensor, q: torch.Tensor,
+                     grad_mse: Optional[torch.Tensor], coef_scale: float) -> torch.Tensor:
+    """The rotation trick's gradient w.r.t. x (vqseg.h, vqseg_rotate_bwd_f32): grad_q carried from q = E[idx] to x by the
+    rotation taking x onto q, scaled by |q| / |x|, plus coef_scale * grad_mse * (x - q).  q is the forward's output."""
+    _require_cuda(x, q, grad_q, grad_mse)
+    L = _native.lib()
+    b, p, d, sb, sp, sd = _bpd(x)
+    gx = torch.empty_like(x, dtype=torch.float32)      # preserve_format keeps the NCHW-view strides
+    gq = grad_q
+    if gq is not None and gq.dtype != torch.float32:
+        gq = gq.float()
+    g = (gq.data_ptr(), gq.stride(0), gq.stride(1), gq.stride(2)) if gq is not None else (None, 0, 0, 0)
+    gm = grad_mse.reshape(-1)[:1].float().contiguous() if grad_mse is not None else None
+    with torch.cuda.device(x.device):
+        _native.check(L.vqseg_rotate_bwd_f32(g[0], g[1], g[2], g[3], x.data_ptr(), sb, sp, sd,
+                                             q.data_ptr(), q.stride(0), q.stride(1), q.stride(2),
+                                             gm.data_ptr() if gm is not None else None, coef_scale,
+                                             gx.data_ptr(), gx.stride(0), gx.stride(1), gx.stride(2),
+                                             b, p, d, _stream()), "rotate_bwd")
+    return gx
+
+
+rotate_bwd = torch.library.custom_op("vqseg::rotate_bwd", mutates_args=())(_rotate_bwd_impl)
+
+
+@rotate_bwd.register_fake
+def _(grad_q, x, q, grad_mse, coef_scale):
+    return torch.empty_like(x, dtype=torch.float32)
+
+
+def _x_grad(mode, grad_q, x, q, grad_mse):
+    """gradient w.r.t. x of a training forward in `mode`: straight-through, or the rotation trick with MODE_ROTATE"""
+    if mode & MODE_ROTATE:
+        return (_rotate_bwd_impl if _fast() else rotate_bwd)(grad_q, x, q, grad_mse, 2.0 / x.numel())
+    return (_ste_bwd_impl if _fast() else ste_bwd)(grad_q, x, q, grad_mse, 2.0 / x.numel())
 
 
 def _gather_bwd_codebook_impl(grad_q: torch.Tensor, idx: torch.Tensor, num_codes: int) -> torch.Tensor:
@@ -864,13 +902,15 @@ def _fast():
 class _StraightThrough(torch.autograd.Function):
     """Training forward of vq_img.py:235-240: q_ste = x + (E[idx] - x), mse = mean((q_ste - x)^2).
     Gradients: d q_ste / dx = I (straight-through), d mse / dx = 2 (x - q_ste) / numel; the codebook
-    gets none (the reference detaches it, SURVEY.md §0)."""
+    gets none (the reference detaches it, SURVEY.md §0).  With MODE_ROTATE in `mode`: q = E[idx] and the
+    rotation trick's gradient (rotate_bwd)."""
 
     @staticmethod
     def forward(ctx, x, codebook, idx, mode):
         q, mse = (_gather_ste_impl if _fast() else gather_ste)(x, codebook, idx, mode)
         ctx.save_for_backward(x, q)
         ctx.mark_non_differentiable(idx)
+        ctx.mode = mode
         return q, mse
 
     @staticmethod
@@ -878,8 +918,7 @@ class _StraightThrough(torch.autograd.Function):
         x, q = ctx.saved_tensors
         if not ctx.needs_input_grad[0]:
             return None, None, None, None
-        gx = (_ste_bwd_impl if _fast() else ste_bwd)(grad_q, x, q, grad_mse, 2.0 / x.numel())
-        return gx, None, None, None
+        return _x_grad(ctx.mode, grad_q, x, q, grad_mse), None, None, None
 
 
 def _codebook_grad(grad_q, idx, num_codes):
@@ -911,13 +950,15 @@ class _EvalGather(torch.autograd.Function):
 
 class _FusedTrainForward(torch.autograd.Function):
     """Training forward in one host call: lookup + STE + commitment mse + usage.  Same gradients as
-    _StraightThrough (identity to x, 2 (x - q) / numel from the mse; nothing to the codebook)."""
+    _StraightThrough (identity to x, 2 (x - q) / numel from the mse; nothing to the codebook; the rotation
+    trick with MODE_ROTATE)."""
 
     @staticmethod
     def forward(ctx, x, codebook, blob, mode, algo):
         q, idx, mse, usage = (_vq_forward_impl if _fast() else vq_forward)(x, codebook, blob, mode, algo)
         ctx.save_for_backward(x, q)
         ctx.mark_non_differentiable(idx, usage)
+        ctx.mode = mode
         return q, idx, mse, usage
 
     @staticmethod
@@ -925,8 +966,7 @@ class _FusedTrainForward(torch.autograd.Function):
         x, q = ctx.saved_tensors
         if not ctx.needs_input_grad[0]:
             return None, None, None, None, None
-        gx = (_ste_bwd_impl if _fast() else ste_bwd)(grad_q, x, q, grad_mse, 2.0 / x.numel())
-        return gx, None, None, None, None
+        return _x_grad(ctx.mode, grad_q, x, q, grad_mse), None, None, None, None
 
 
 class _FusedEvalForward(torch.autograd.Function):
@@ -957,21 +997,25 @@ def autocast_code_dtype(amp_compat=True):
     return dtype if dtype in (torch.float16, torch.bfloat16) else None
 
 
-def gather_mode(training, amp=None):
+def gather_mode(training, amp=None, rotate=False):
     """The gather mode (MODE_*) that rounds the code through `amp`: None for exact fp32 codes, torch.float16 or
-    torch.bfloat16 (autocast_code_dtype()); False / True stand for None / torch.float16."""
+    torch.bfloat16 (autocast_code_dtype()); False / True stand for None / torch.float16.  rotate=True (training only)
+    adds MODE_ROTATE: the rotation trick instead of the straight-through estimator."""
+    if rotate and not training:
+        raise ValueError("the rotation trick applies to training forwards only")
+    rot = MODE_ROTATE if rotate else 0
     if amp is None or amp is False:
-        return MODE_TRAIN if training else MODE_EVAL
+        return MODE_TRAIN | rot if training else MODE_EVAL
     if amp is True or amp == torch.float16:
-        return MODE_TRAIN_AMP if training else MODE_EVAL_AMP
+        return MODE_TRAIN_AMP | rot if training else MODE_EVAL_AMP
     if amp == torch.bfloat16:
-        return MODE_TRAIN_AMP_BF16 if training else MODE_EVAL_AMP_BF16
+        return MODE_TRAIN_AMP_BF16 | rot if training else MODE_EVAL_AMP_BF16
     raise ValueError(f"the gathered code can be rounded through torch.float16 or torch.bfloat16, not {amp}")
 
 
-def fused_forward(x, weight, blob, training, amp=None, algo=ALGO_AUTO):
-    """(q, idx, mse, usage) with autograd attached when needed; `amp` as in gather_mode."""
-    mode = gather_mode(training, amp)
+def fused_forward(x, weight, blob, training, amp=None, algo=ALGO_AUTO, rotate=False):
+    """(q, idx, mse, usage) with autograd attached when needed; `amp` and `rotate` as in gather_mode."""
+    mode = gather_mode(training, amp, rotate)
     if training:
         if torch.is_grad_enabled() and x.requires_grad:
             return _FusedTrainForward.apply(x, weight.detach(), blob, mode, algo)
@@ -981,8 +1025,8 @@ def fused_forward(x, weight, blob, training, amp=None, algo=ALGO_AUTO):
     return (_vq_forward_impl if _fast() else vq_forward)(x, weight, blob, mode, algo)
 
 
-def straight_through(x, codebook, idx, amp=None):
-    return _StraightThrough.apply(x, codebook, idx, gather_mode(True, amp))
+def straight_through(x, codebook, idx, amp=None, rotate=False):
+    return _StraightThrough.apply(x, codebook, idx, gather_mode(True, amp, rotate))
 
 
 def eval_gather(codebook, x_like, idx, amp=None):

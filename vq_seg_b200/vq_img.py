@@ -280,6 +280,7 @@ class VectorQuantizer(nn.Module):
                                        kmeans_init=kmeans_init, kmeans_iters=kmeans_iters, decay=decay,
                                        eps=eps, num_codebook=num_codebook)
         self.amp_compat = True    # round the gathered code through the fp16 / bf16 autocast dtype like the reference's matmul
+        self.rotation_trick = False  # opt-in: carry the gradient to x by the rotation trick instead of straight-through
         self._graphs = None       # opt-in CUDA-graph cache of the no-grad forward (enable_cuda_graphs)
 
     def enable_cuda_graphs(self, max_entries: int = 16):
@@ -349,13 +350,14 @@ class VectorQuantizer(nn.Module):
         cb = self.codebook
         amp = ops.autocast_code_dtype(self.amp_compat)
         cosine = isinstance(cb, CosinesimCodebook)
+        rotate = self.rotation_trick and self.training
         if cb.kmeans_init and self.training and not cb.initted:
             cb._kmeans_init(ops.l2norm_rows(xv) if cosine else xv, cosine=cosine)
         if cosine:
             idx, counts = cb.lookup(xv)
             code_usage = ops.fast_code_usage(counts)
             if self.training:
-                quantize, mse = ops.straight_through(xv, cb.embedding.weight.detach(), idx, amp)
+                quantize, mse = ops.straight_through(xv, cb.embedding.weight.detach(), idx, amp, rotate)
             else:
                 quantize, mse = ops.eval_gather(cb.embedding.weight, xv, idx, amp), None
         else:
@@ -363,7 +365,8 @@ class VectorQuantizer(nn.Module):
             if xv.shape[-1] != cb.embedding_dim:
                 raise RuntimeError(f"X1 and X2 must have the same number of columns. X1: {xv.shape[-1]} X2: {cb.embedding_dim}")
             blob = cb._prepared() if cb.algo != ops.ALGO_EXACT else None
-            quantize, idx, mse, code_usage = ops.fused_forward(xv, cb.embedding.weight, blob, self.training, amp, cb.algo)
+            quantize, idx, mse, code_usage = ops.fused_forward(xv, cb.embedding.weight, blob, self.training, amp,
+                                                                cb.algo, rotate)
         # loss (vq_img.py:230,239-241): [0.] + mse * w.  0 + v and v * 1 are exact in fp32, so for the default weight
         # the kernel's (1,) mse IS the loss (no fill / mul / add launches); eval: the kernel's zeroed (1,) output
         if self.training and self.commitment_weight > 0 and (mse.requires_grad or not torch.is_grad_enabled()):
