@@ -151,6 +151,7 @@ int    vqseg_vq_forward_f32(const float* x, int64_t B, int64_t P, int64_t D,
  * Replaces autograd through vq_img.py:236-240:  gx = g_q + coef * (x - q_ste), with
  * coef = g_loss * commitment_weight * 2 / numel read from device memory (coef_dev, 1 float) so no
  * host sync is needed.  g_q may be null (treated as zeros), coef_dev may be null (no loss term).
+ * q_ste may be null (treated as zeros: gx = fma(coef, x, g_q), the residual VQ backward with x = A below).
  * All tensors share the (B,P,D) logical shape; each has its own strides.                        */
 int    vqseg_ste_bwd_f32(const float* g_q, int64_t gB, int64_t gP, int64_t gD,
                          const float* x, int64_t sB, int64_t sP, int64_t sD,
@@ -182,6 +183,51 @@ int    vqseg_rotate_bwd_f32(const float* g_q, int64_t gB, int64_t gP, int64_t gD
                             const float* coef_dev, float coef_scale,
                             float* gx, int64_t oB, int64_t oP, int64_t oD,
                             int64_t B, int64_t P, int64_t D, void* stream);
+
+/* ---- residual vector quantization: OPT-IN EXTENSION, no reference counterpart (ResidualVQ of
+ * lucidrains/vector-quantize-pytorch; parity unpinned).  Q codebooks E_0 .. E_{Q-1} quantize x, then what the first left,
+ * and so on.  x is the (B, P, D) view of the input map, w the commitment weight, rho the gather mode's rounding of the
+ * code (identity in TRAIN / EVAL, fp16 or bf16 round-to-nearest-even in the AMP modes); every operation is a separately
+ * rounded fp32 operation with no contraction, and "ascending" means l = 0, 1, ...:
+ *   r_0 = x;  for l = 0 .. Q-1:
+ *     idx_l = the lookup of r_l: Euclidean, the first argmin of vqseg_assign_f32; cosine (rn given), the first argmax of
+ *             l2norm(r_l) . E_l^T (vqseg_assign_f32 with VQSEG_METRIC_IP on rn = l2norm(r_l), E_l already renormalised)
+ *     c_l   = rho(E_l[idx_l]);   S = c_l if l == 0 else S + c_l
+ *     TRAIN:           q_l = r_l + (c_l - r_l);  m_l = mean((q_l - r_l)^2) with the gather's fixed two-stage reduction
+ *                      (exactly what vqseg_gather_ste_f32 writes as the loss for input r_l in the TRAIN mode)
+ *     TRAIN, acc given: A = (r_l - q_l) if l == 0 else A + (r_l - q_l)
+ *     r_{l+1} = r_l - c_l   (l < Q-1, in TRAIN and EVAL alike)
+ * Outputs: quantize = x + (S - x) in TRAIN, S in EVAL; loss L = w m_0, then L + w m_l ascending (TRAIN); code usage
+ * 100 * (Z / (Q K)) with Z the number of (l, k) pairs with a zero count.  With Q = 1 all of it is vqseg_vq_forward_f32.
+ * Gradient (TRAIN): gx = fma(coef, A, g) with coef = g_loss * w * 2 / (B P D): vqseg_ste_bwd_f32 with x = A and a null
+ * q_ste.  The codebooks get none; in EVAL gE_l[k] = sum over the rows with idx_l = k of g (vqseg_gather_bwd_codebook_f32).
+ *
+ * vqseg_rvq_stage_f32 runs stage `layer` of `n_layers` with ONE host call: the launches of vqseg_vq_forward_f32 (the
+ * assignment prologue and guard, filter, rescoring and overflow rows) with the stage kernel in the gather's place.  Per
+ * element the stage kernel reads r_l, the code and S (layer > 0) and writes S (into q), r_{l+1} (into r_next, unless this
+ * is the last stage), A (into acc, TRAIN only, nullable) and, in the last TRAIN stage, quantize over S from x (any strides).
+ * q, r_next and acc share q's strides; (D*P, 1, P) (NCHW memory order) lets the next stage take the same TMA-fed filter as
+ * stage 0.  r: r_l (any strides); rn: null (Euclidean) or l2norm(r_l) for the cosine lookup; idx_out: B*P int64 (this
+ * layer's slice); counts: (Q, K) int64, row `layer` zeroed and filled here; layer_mse / layer_usage: (Q,) floats, entry
+ * `layer` written (m_l, 0 in EVAL; and the layer's usage); the last stage also writes loss_out (nullable: L from
+ * layer_mse[0 .. Q-1] and w in TRAIN, 0 in EVAL) and usage_out (nullable) from all Q count rows.  mode: a TRAIN or EVAL mode without
+ * VQSEG_MODE_ROTATE; algo: as vqseg_assign_f32 without VQSEG_METRIC_IP.  ws: vqseg_rvq_stage_workspace_bytes.
+ * An empty batch (B * P == 0) writes zero counts, m_l = 0, usage 100 and loss 0.                                       */
+size_t vqseg_rvq_stage_workspace_bytes(int64_t n_rows, int64_t D, int64_t K);
+int    vqseg_rvq_stage_f32(const float* r, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
+                           const float* rn, int64_t nB, int64_t nP, int64_t nD,
+                           const float* x, int64_t xB, int64_t xP, int64_t xD,
+                           const float* E, int64_t K, void* blob,
+                           int64_t* idx_out, int64_t* counts,
+                           float* q, int64_t qB, int64_t qP, int64_t qD, float* r_next, float* acc,
+                           float* layer_mse, float* layer_usage, float* loss_out, float* usage_out,
+                           int layer, int n_layers, float weight, int mode, int algo,
+                           void* ws, size_t ws_bytes, void* stream);
+/* S of the restatement above from a (Q, B, P) int64 index array (idx[l][b][p]) and the Q codebooks packed (Q, K, D), in one
+ * launch for any Q >= 1: out = c_0, then out + c_l ascending, with the rounding of `mode` (an EVAL mode).  Bit-equal to
+ * the EVAL quantize of the same indices.  out: (B, P, D) with any strides.                                              */
+int    vqseg_rvq_decode_f32(const int64_t* idx, int64_t Q, int64_t B, int64_t P, const float* E, int64_t K, int64_t D,
+                            float* out, int64_t oB, int64_t oP, int64_t oD, int mode, void* stream);
 
 /* gradient of the eval-mode gather w.r.t. the codebook: gE[idx[n], :] += g_q[n, :]              */
 int    vqseg_gather_bwd_codebook_f32(const float* g_q, int64_t B, int64_t P, int64_t D,

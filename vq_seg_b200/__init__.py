@@ -6,6 +6,7 @@ The kernels live in libvqseg.so (C ABI: include/vqseg.h); importing this package
 the first op call does -- and raises if it is missing (no CPU fallback)."""
 from .vq_img import (VectorQuantizer, EuclideanCodebook, CosinesimCodebook, kmeans, sample_vectors,  # noqa: F401
                      batched_sample_vectors, batched_bincount, l2norm)
+from .rvq import ResidualVectorQuantizer  # noqa: F401
 from .vq_segmentation_head import VQSegmentationHead, EuclideanSegHead, CosinesimSegHead  # noqa: F401
 from .factory import make_vq_module, Identity, install  # noqa: F401
 from . import ops  # noqa: F401

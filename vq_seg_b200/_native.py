@@ -35,6 +35,10 @@ SIGNATURES = {
                                vp, i64, i64, i64, i64, i64, i64, vp]),
     "vqseg_rotate_bwd_f32": (ci, [vp, i64, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64, vp, f32,
                                   vp, i64, i64, i64, i64, i64, i64, vp]),
+    "vqseg_rvq_stage_workspace_bytes": (sz, [i64, i64, i64]),
+    "vqseg_rvq_stage_f32": (ci, [vp, i64, i64, i64, i64, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64, vp, i64, vp,
+                                 vp, vp, vp, i64, i64, i64, vp, vp, vp, vp, vp, vp, ci, ci, f32, ci, ci, vp, sz, vp]),
+    "vqseg_rvq_decode_f32": (ci, [vp, i64, i64, i64, vp, i64, i64, vp, i64, i64, i64, ci, vp]),
     "vqseg_gather_bwd_codebook_f32": (ci, [vp, i64, i64, i64, i64, i64, i64, vp, vp, i64, vp]),
     "vqseg_code_stats_workspace_bytes": (sz, [i64, i64, i64, ci]),
     "vqseg_code_stats_f32": (ci, [vp, i64, i64, i64, i64, i64, i64, vp, i64, vp, vp, ci, vp, sz, vp]),

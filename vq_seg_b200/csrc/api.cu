@@ -16,6 +16,12 @@ __global__ void blob_init_kernel(BlobHeader* h, int K, int D, int K_pad, int D_p
   h->stale = 0u; h->ticket = 0u; h->rebuilds = 0u;
 }
 
+int rvq_stage_gather(const float* r, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
+                     const float* x, int64_t xB, int64_t xP, int64_t xD, const float* E, int64_t K, const int64_t* idx,
+                     float* q, int64_t qB, int64_t qP, int64_t qD, float* r_next, float* acc,
+                     float* layer_mse, float* layer_usage, const int64_t* counts, int layer, int n_layers, float weight,
+                     float* loss_out, float* usage_out, int mode, void* ws, size_t ws_bytes, cudaStream_t st, int* ticket);
+
 extern "C" int vqseg_internal_gather_ticket(const float* x, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
                                             const float* E, int64_t K, const int64_t* idx,
                                             float* q_out, int64_t qB, int64_t qP, int64_t qD, float* loss_out, int mode,
@@ -439,6 +445,50 @@ int vqseg_vq_forward_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_
   // gather's last block reduces the loss and turns the (final) counts into the code usage
   return vqseg_internal_gather_ticket(x, B, P, D, sB, sP, sD, E, K, idx_out, q_out, qB, qP, qD, loss_out, mode,
                                       (char*)ws + wa, ws_bytes - wa, stream, (int*)ws + 2, counts_out, usage_out);
+}
+
+size_t vqseg_rvq_stage_workspace_bytes(int64_t n_rows, int64_t D, int64_t K) {
+  return vqseg_forward_workspace_bytes(n_rows, D, K);
+}
+
+int vqseg_rvq_stage_f32(const float* r, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
+                        const float* rn, int64_t nB, int64_t nP, int64_t nD,
+                        const float* x, int64_t xB, int64_t xP, int64_t xD,
+                        const float* E, int64_t K, void* blob,
+                        int64_t* idx_out, int64_t* counts,
+                        float* q, int64_t qB, int64_t qP, int64_t qD, float* r_next, float* acc,
+                        float* layer_mse, float* layer_usage, float* loss_out, float* usage_out,
+                        int layer, int n_layers, float weight, int mode, int algo,
+                        void* ws, size_t ws_bytes, void* stream) {
+  if (!counts || !layer_mse || !layer_usage || K <= 0 || B < 0 || P < 0 || D <= 0) return VQSEG_EINVAL;
+  if (n_layers < 1 || layer < 0 || layer >= n_layers) return VQSEG_EINVAL;
+  if (mode < VQSEG_MODE_EVAL || mode > VQSEG_MODE_EVAL_AMP_BF16) return VQSEG_EINVAL;     // (no VQSEG_MODE_ROTATE)
+  if (algo & VQSEG_METRIC_IP) return VQSEG_EINVAL;               // the metric follows from `rn`
+  const bool train = mode == VQSEG_MODE_TRAIN || mode == VQSEG_MODE_TRAIN_AMP || mode == VQSEG_MODE_TRAIN_AMP_BF16;
+  const bool last = layer == n_layers - 1;
+  cudaStream_t st = (cudaStream_t)stream;
+  int64_t* counts_l = counts + (int64_t)layer * K;
+  if (B * P == 0) {                                              // an empty batch: no code is used, no loss
+    cudaError_t e = cudaMemsetAsync(counts_l, 0, (size_t)K * sizeof(int64_t), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(layer_mse + layer, 0, sizeof(float), st);
+    if (e == cudaSuccess && last && loss_out) e = cudaMemsetAsync(loss_out, 0, sizeof(float), st);
+    if (e != cudaSuccess) return (int)e;
+    int rc = vqseg_code_usage(counts_l, K, layer_usage + layer, stream);
+    if (!rc && last && usage_out) rc = vqseg_code_usage(counts, (int64_t)n_layers * K, usage_out, stream);
+    return rc;
+  }
+  if (!r || !idx_out || !q || (!last && !r_next) || (train && last && !x)) return VQSEG_EINVAL;
+  const size_t wa = (size_t)round_up(vqseg_assign_workspace_bytes(B * P, D, K, algo), 256);
+  if (!ws || ws_bytes < wa + vqseg_gather_workspace_bytes(B * P, D)) return VQSEG_EWORKSPACE;
+  // the lookup: r itself (Euclidean) or its normalised rows (inner product); the prologue zeroes this layer's counts and
+  // m_l, the work counter and the tickets
+  const float* lx = rn ? rn : r;
+  int rc = assign_internal(lx, B, P, D, rn ? nB : sB, rn ? nP : sP, rn ? nD : sD, E, K, blob, idx_out, counts_l, nullptr, 0, 0,
+                           algo | (rn ? VQSEG_METRIC_IP : 0), ws, wa, stream, nullptr, layer_mse + layer, true);
+  if (rc) return rc;
+  return rvq_stage_gather(r, B, P, D, sB, sP, sD, x, xB, xP, xD, E, K, idx_out, q, qB, qP, qD, last ? nullptr : r_next, acc,
+                          layer_mse, layer_usage, counts, layer, n_layers, weight, loss_out, usage_out, mode,
+                          (char*)ws + wa, ws_bytes - wa, st, (int*)ws + 2);
 }
 
 }  // extern "C"

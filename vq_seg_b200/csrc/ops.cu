@@ -43,14 +43,15 @@ __device__ __forceinline__ int gcol(int p) { return ((p & 3) << 5) | (p >> 2); }
 // draws the last one sums all partials in the same fixed order as loss_finalize_kernel -- one launch less.
 // The same block also turns the (by then final) per-code counts into the code usage of vq_img.py:173-175.
 struct LossTail { int* ticket; float* loss_out; double inv_numel; const unsigned long long* counts; int K; float* usage_out; };
-__device__ __forceinline__ void loss_tail(const LossTail& t, const float* partial, int n_partial, int n_blocks) {
+// returns true in the block that drew the last ticket
+__device__ __forceinline__ bool loss_tail(const LossTail& t, const float* partial, int n_partial, int n_blocks) {
   __shared__ double s_dred[256];
   __shared__ int s_last;
   __threadfence();
   __syncthreads();
   if (threadIdx.x == 0) s_last = (atomicAdd(t.ticket, 1) == n_blocks - 1);
   __syncthreads();
-  if (!s_last) return;
+  if (!s_last) return false;
   __threadfence();
   if (t.loss_out) {
     double s = 0.0;
@@ -75,13 +76,77 @@ __device__ __forceinline__ void loss_tail(const LossTail& t, const float* partia
     }
     if (threadIdx.x == 0) *t.usage_out = __fmul_rn(100.f, __fdiv_rn((float)s_dred[0], (float)t.K));
   }
+  return true;
+}
+
+// Residual VQ stage (vqseg_rvq_stage_f32): the gather kernels instantiated with RVQ = true read r_l where they read x,
+// keep the loss of the gather (m_l, for quantize = r_l + (c_l - r_l)) and additionally write, per element,
+//   S = c_l (first stage) or S + c_l into q (q holds the S of the earlier stages), or in the last TRAIN stage
+//   x + (S - x) with x = x0 (the module's input, any strides);  r_next = r_l - c_l;  acc (A) = [A +] (r_l - q_l).
+// r_next and acc share q's strides.  The last block also pools the loss and usage over the layers (rvq_pool).
+struct RvqStage {
+  float* r_next;                       // r_{l+1} (null in the last stage)
+  float* acc;                          // A (null without a gradient)
+  Rows x0;                             // x0.ptr: the input, read by the last TRAIN stage only (null otherwise)
+  int first;                           // l == 0: S = c
+  const float* layer_mse;              // (Q,) m_0 .. m_l, written by the tails of the stages so far
+  const unsigned long long* counts_all;   // (Q, K) counts of every layer
+  int n_layers;                        // Q: the last stage (l == Q - 1) pools
+  float weight;                        // commitment weight w
+  float* loss_out;                     // pooled loss (nullable): L in TRAIN, 0 in EVAL
+  int train;
+  float* usage_out;                    // pooled usage (nullable)
+};
+__device__ __forceinline__ void rvq_pool(const RvqStage& r, int K) {
+  __shared__ int s_zred[256];
+  if (r.loss_out && threadIdx.x == 0) {                 // L = w m_0, then L + w m_l in ascending order
+    float L = 0.f;
+    if (r.train) {
+      L = __fmul_rn(r.weight, __ldcg(r.layer_mse));
+      for (int l = 1; l < r.n_layers; ++l) L = __fadd_rn(L, __fmul_rn(r.weight, __ldcg(r.layer_mse + l)));
+    }
+    *r.loss_out = L;
+  }
+  if (r.usage_out) {                                    // 100 * (zero (l, k) pairs / (Q K))
+    const long long QK = (long long)r.n_layers * K;
+    int z = 0;
+    for (long long i = threadIdx.x; i < QK; i += 256) z += (__ldcg(r.counts_all + i) == 0ull);
+    s_zred[threadIdx.x] = z;
+    __syncthreads();
+    for (int o = 128; o; o >>= 1) {
+      if ((int)threadIdx.x < o) s_zred[threadIdx.x] += s_zred[threadIdx.x + o];
+      __syncthreads();
+    }
+    if (threadIdx.x == 0) *r.usage_out = __fmul_rn(100.f, __fdiv_rn((float)s_zred[0], (float)QK));
+  }
+}
+// one element of a stage: c the rounded code, rv = r_l, sv = S so far (ignored in the first stage), av = A so far (ignored
+// in the first stage); returns what q receives and accumulates the loss term like the gather
+// (av: A so far in, A out; rn: r_{l+1} out; x0e: the input element in the last TRAIN stage, else null)
+template <bool kTrain>
+__device__ __forceinline__ float rvq_elem(bool first, float c, float rv, float sv, float& av, float& rn,
+                                          const float* x0e, float& acc) {
+  const float s = first ? c : __fadd_rn(sv, c);
+  if (kTrain) {
+    const float ql = __fadd_rn(rv, __fsub_rn(c, rv));
+    const float f = __fsub_rn(ql, rv);
+    acc = __fmaf_rn(f, f, acc);
+    const float a = __fsub_rn(rv, ql);
+    av = first ? a : __fadd_rn(av, a);
+  }
+  rn = __fsub_rn(rv, c);
+  if (kTrain && x0e) { const float xv = __ldg(x0e); return __fadd_rn(xv, __fsub_rn(s, xv)); }
+  return s;
+}
+__device__ __forceinline__ const float* rvq_x0(const RvqStage& rs, long long b, long long p, long long d) {
+  return rs.x0.ptr ? rs.x0.ptr + b * rs.x0.sB + p * rs.x0.sP + d * rs.x0.sD : nullptr;
 }
 
 // VEC: pixel quads are 16-byte aligned and never straddle an image (P % 4 == 0, aligned bases)
-template <int MODE, bool VEC>
+template <int MODE, bool VEC, bool RVQ = false>
 __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float* __restrict__ E, int K,
                                                              const long long* __restrict__ idx, RowsOut q,
-                                                             float* __restrict__ partial, LossTail tail) {
+                                                             float* __restrict__ partial, LossTail tail, RvqStage rs) {
   __shared__ float tile[kGTile][kGPix + 1];
   __shared__ int s_idx[kGPix];
   __shared__ float s_red[8];
@@ -125,17 +190,18 @@ __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float
   float acc = 0.f;
   const int p4 = lane * 4;
   const long long n = n0 + p4;
+  const bool load_x = kTrain || (RVQ && rs.r_next);      // a stage reads r_l to write r_{l+1} in eval too
   if (VEC) {
     if (n < n_rows) {
       long long b, pp;
       split_row(n, x.P, b, pp);
-      const float* xb = kTrain ? x.ptr + b * x.sB + pp : nullptr;
+      const float* xb = load_x ? x.ptr + b * x.sB + pp : nullptr;
       float* qb = q.ptr + b * q.sB + pp;
       float4 xr[kGTile / 8];
-      const float* xd = kTrain ? xb + (long long)(d0 + warp) * x.sD : nullptr;   // rows d0 + warp + 8u: pointer stepping
+      const float* xd = load_x ? xb + (long long)(d0 + warp) * x.sD : nullptr;   // rows d0 + warp + 8u: pointer stepping
       float* qd = qb + (long long)(d0 + warp) * q.sD;
       const long long xstep = 8 * x.sD, qstep = 8 * q.sD;
-      if (kTrain) {                                        // all row loads in flight before the first use
+      if (load_x) {                                        // all row loads in flight before the first use
 #pragma unroll
         for (int u = 0; u < kGTile / 8; ++u) {
           const int d = warp + 8 * u;
@@ -149,7 +215,21 @@ __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float
         if (d0 + d < D) {
           float4 e = make_float4(tile[d][lane], tile[d][32 + lane], tile[d][64 + lane], tile[d][96 + lane]);   // = pixels p4 .. p4+3
           float4 o = e;
-          if (kTrain) {
+          if (RVQ) {
+            float* qp = qd + u * qstep;
+            const long long off = qp - q.ptr;
+            const float4 rv = load_x ? xr[u] : make_float4(0.f, 0.f, 0.f, 0.f);
+            const float4 sv = rs.first ? e : *reinterpret_cast<const float4*>(qp);
+            float4 av = (kTrain && rs.acc && !rs.first) ? *reinterpret_cast<const float4*>(rs.acc + off) : make_float4(0.f, 0.f, 0.f, 0.f);
+            float4 rn;
+            const long long dd = d0 + d;
+            o.x = rvq_elem<kTrain>(rs.first, e.x, rv.x, sv.x, av.x, rn.x, rvq_x0(rs, b, pp, dd), acc);
+            o.y = rvq_elem<kTrain>(rs.first, e.y, rv.y, sv.y, av.y, rn.y, rvq_x0(rs, b, pp + 1, dd), acc);
+            o.z = rvq_elem<kTrain>(rs.first, e.z, rv.z, sv.z, av.z, rn.z, rvq_x0(rs, b, pp + 2, dd), acc);
+            o.w = rvq_elem<kTrain>(rs.first, e.w, rv.w, sv.w, av.w, rn.w, rvq_x0(rs, b, pp + 3, dd), acc);
+            if (kTrain && rs.acc) *reinterpret_cast<float4*>(rs.acc + off) = av;
+            if (rs.r_next) *reinterpret_cast<float4*>(rs.r_next + off) = rn;
+          } else if (kTrain) {
             const float4 xv = xr[u];
             if (!kRot) {
               o.x = __fadd_rn(xv.x, __fsub_rn(e.x, xv.x)); o.y = __fadd_rn(xv.y, __fsub_rn(e.y, xv.y));   // x + (q - x)
@@ -170,13 +250,21 @@ __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float
       if (ni < n_rows) {
         long long b, pp;
         split_row(ni, x.P, b, pp);
-        const float* xb = kTrain ? x.ptr + b * x.sB + pp * x.sP : nullptr;
+        const float* xb = load_x ? x.ptr + b * x.sB + pp * x.sP : nullptr;
         float* qb = q.ptr + b * q.sB + pp * q.sP;
         for (int d = warp; d < kGTile; d += 8) {
           if (d0 + d < D) {
             float e = tile[d][32 * i + lane];
             float o = e;
-            if (kTrain) {
+            if (RVQ) {
+              float* qp = qb + (long long)(d0 + d) * q.sD;
+              const long long off = qp - q.ptr;
+              const float rv = load_x ? __ldg(xb + (long long)(d0 + d) * x.sD) : 0.f;
+              float av = (kTrain && rs.acc && !rs.first) ? rs.acc[off] : 0.f, rn;
+              o = rvq_elem<kTrain>(rs.first, e, rv, rs.first ? e : *qp, av, rn, rvq_x0(rs, b, pp, d0 + d), acc);
+              if (kTrain && rs.acc) rs.acc[off] = av;
+              if (rs.r_next) rs.r_next[off] = rn;
+            } else if (kTrain) {
               float xv = __ldg(xb + (long long)(d0 + d) * x.sD);
               if (!kRot) o = __fadd_rn(xv, __fsub_rn(e, xv));
               float f = __fsub_rn(o, xv);
@@ -200,14 +288,17 @@ __global__ void __launch_bounds__(256) gather_ste_pxc_kernel(Rows x, const float
       partial[(long long)blockIdx.y * gridDim.x + blockIdx.x] = s;
     }
   }
-  if (tail.ticket) loss_tail(tail, partial, (int)(gridDim.x * gridDim.y), (int)(gridDim.x * gridDim.y));
+  if (tail.ticket) {
+    const bool last = loss_tail(tail, partial, (int)(gridDim.x * gridDim.y), (int)(gridDim.x * gridDim.y));
+    if (RVQ && last) rvq_pool(rs, K);
+  }
 }
 
 // Generic strides (row-major samples etc.): one warp per row, lanes along d.
-template <int MODE>
+template <int MODE, bool RVQ = false>
 __global__ void __launch_bounds__(256) gather_ste_generic_kernel(Rows x, const float* __restrict__ E, int K,
                                                                  const long long* __restrict__ idx, RowsOut q,
-                                                                 float* __restrict__ partial, LossTail tail) {
+                                                                 float* __restrict__ partial, LossTail tail, RvqStage rs) {
   __shared__ float s_red[8];
   const int D = (int)x.D;
   const long long n_rows = x.n_rows();
@@ -221,7 +312,17 @@ __global__ void __launch_bounds__(256) gather_ste_generic_kernel(Rows x, const f
     float* qr = q.row(n);
     for (int d = lane; d < D; d += 32) {
       const float e = round_code<MODE>(__ldg(er + d));
-      if (!gather_train(MODE)) {
+      if (RVQ) {
+        float* qp = qr + (long long)d * q.sD;
+        const long long off = qp - q.ptr;
+        const float rv = (gather_train(MODE) || rs.r_next) ? __ldg(xr + (long long)d * x.sD) : 0.f;
+        float av = (gather_train(MODE) && rs.acc && !rs.first) ? rs.acc[off] : 0.f, rn;
+        long long b, p;
+        split_row(n, x.P, b, p);
+        *qp = rvq_elem<gather_train(MODE)>(rs.first, e, rv, rs.first ? e : *qp, av, rn, rvq_x0(rs, b, p, d), acc);
+        if (gather_train(MODE) && rs.acc) rs.acc[off] = av;
+        if (rs.r_next) rs.r_next[off] = rn;
+      } else if (!gather_train(MODE)) {
         qr[(long long)d * q.sD] = e;
       } else {
         float xv = __ldg(xr + (long long)d * x.sD);
@@ -244,7 +345,10 @@ __global__ void __launch_bounds__(256) gather_ste_generic_kernel(Rows x, const f
       partial[blockIdx.x] = s;
     }
   }
-  if (tail.ticket) loss_tail(tail, partial, (int)gridDim.x, (int)gridDim.x);
+  if (tail.ticket) {
+    const bool last = loss_tail(tail, partial, (int)gridDim.x, (int)gridDim.x);
+    if (RVQ && last) rvq_pool(rs, K);
+  }
 }
 
 // fixed-order final reduction of the per-block partials -> mean
@@ -262,12 +366,14 @@ __global__ void __launch_bounds__(256) loss_finalize_kernel(const float* __restr
   if (threadIdx.x == 0) *loss_out = (float)(s_red[0] * inv_numel);
 }
 
-template <int MODE>
+template <int MODE, bool RVQ = false>
 static int launch_gather(const Rows& x, const float* E, int K, const long long* idx, const RowsOut& q,
                          float* loss_out, float* partial, size_t partial_cap, cudaStream_t st, int* ticket = nullptr,
-                         const unsigned long long* counts = nullptr, float* usage_out = nullptr) {
+                         const unsigned long long* counts = nullptr, float* usage_out = nullptr,
+                         const RvqStage& rs = RvqStage{}) {
   const long long n_rows = x.n_rows();
   const bool train = gather_train(MODE);
+  const bool reads_x = train || (RVQ && rs.r_next);
   const bool want_loss = train && loss_out != nullptr;
   const bool want_usage = ticket && counts && usage_out;
   // ticket (zeroed by the caller): the kernel's last block reduces the loss (and the code usage) itself
@@ -280,10 +386,11 @@ static int launch_gather(const Rows& x, const float* E, int K, const long long* 
     if (want_loss && (size_t)n_partial > partial_cap) return VQSEG_EWORKSPACE;
     auto al = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
     const bool vec = (x.P % 4 == 0) && al(q.ptr) && (q.sD % 4 == 0) && (q.sB % 4 == 0) &&
-                     (!train || (al(x.ptr) && (x.sD % 4 == 0) && (x.sB % 4 == 0)));
+                     (!reads_x || (al(x.ptr) && (x.sD % 4 == 0) && (x.sB % 4 == 0))) &&
+                     (!RVQ || (al(rs.r_next) && al(rs.acc)));
     cudaError_t le;
-    if (vec) le = launch_dependent(gather_ste_pxc_kernel<MODE, true>, grid, dim3(256), 0, st, pdl_enabled(), x, E, K, idx, q, want_loss ? partial : nullptr, tail);
-    else     le = launch_dependent(gather_ste_pxc_kernel<MODE, false>, grid, dim3(256), 0, st, pdl_enabled(), x, E, K, idx, q, want_loss ? partial : nullptr, tail);
+    if (vec) le = launch_dependent(gather_ste_pxc_kernel<MODE, true, RVQ>, grid, dim3(256), 0, st, pdl_enabled(), x, E, K, idx, q, want_loss ? partial : nullptr, tail, rs);
+    else     le = launch_dependent(gather_ste_pxc_kernel<MODE, false, RVQ>, grid, dim3(256), 0, st, pdl_enabled(), x, E, K, idx, q, want_loss ? partial : nullptr, tail, rs);
     if (le != cudaSuccess) return (int)le;
   } else {
     long long blocks = (n_rows + 7) / 8;
@@ -291,7 +398,7 @@ static int launch_gather(const Rows& x, const float* E, int K, const long long* 
     if (blocks > cap) blocks = cap;
     n_partial = (int)blocks;
     if (want_loss && (size_t)n_partial > partial_cap) return VQSEG_EWORKSPACE;
-    gather_ste_generic_kernel<MODE><<<(unsigned)blocks, 256, 0, st>>>(x, E, K, idx, q, want_loss ? partial : nullptr, tail);
+    gather_ste_generic_kernel<MODE, RVQ><<<(unsigned)blocks, 256, 0, st>>>(x, E, K, idx, q, want_loss ? partial : nullptr, tail, rs);
   }
   VQSEG_LAUNCH_CHECK();
   if (want_loss && !ticket) {
@@ -303,9 +410,11 @@ static int launch_gather(const Rows& x, const float* E, int K, const long long* 
 
 // =================================================================================================
 // backward w.r.t. x of the training forward (autograd through vq_img.py:236-240)
-// gx = g_q + coef * (x - q_ste),  coef = coef_scale * (*coef_dev)
+// gx = g_q + coef * (x - q_ste),  coef = coef_scale * (*coef_dev);  HAS_Q = false (null q_ste): gx = fma(coef, x, g_q),
+// the residual VQ backward with x = A
 // =================================================================================================
 struct View { const float* ptr; long long sB, sP, sD; };
+template <bool HAS_Q = true>
 __global__ void __launch_bounds__(256) ste_bwd_kernel(View g, View x, View q, const float* __restrict__ coef_dev,
                                                       float coef_scale, RowsOut o, bool px_fast) {
   const long long total = o.B * o.P * o.D;
@@ -318,14 +427,19 @@ __global__ void __launch_bounds__(256) ste_bwd_kernel(View g, View x, View q, co
     float r = gv;
     if (coef_dev) {
       float xv = __ldg(x.ptr + b * x.sB + p * x.sP + d * x.sD);
-      float qv = __ldg(q.ptr + b * q.sB + p * q.sP + d * q.sD);
-      r = __fmaf_rn(coef, __fsub_rn(xv, qv), gv);
+      if (HAS_Q) {
+        float qv = __ldg(q.ptr + b * q.sB + p * q.sP + d * q.sD);
+        r = __fmaf_rn(coef, __fsub_rn(xv, qv), gv);
+      } else {
+        r = __fmaf_rn(coef, xv, gv);
+      }
     }
     o.ptr[b * o.sB + p * o.sP + d * o.sD] = r;
   }
 }
 
 // same dense layout for all four tensors: flat, vectorised, memory order
+template <bool HAS_Q = true>
 __global__ void __launch_bounds__(256) ste_bwd_flat_kernel(const float4* __restrict__ g, const float4* __restrict__ x,
                                                            const float4* __restrict__ q, const float* __restrict__ coef_dev,
                                                            float coef_scale, float4* __restrict__ o, long long n4) {
@@ -333,9 +447,14 @@ __global__ void __launch_bounds__(256) ste_bwd_flat_kernel(const float4* __restr
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
     float4 r = g ? __ldg(g + i) : make_float4(0.f, 0.f, 0.f, 0.f);
     if (coef_dev) {
-      const float4 xv = __ldg(x + i), qv = __ldg(q + i);
-      r.x = __fmaf_rn(coef, __fsub_rn(xv.x, qv.x), r.x); r.y = __fmaf_rn(coef, __fsub_rn(xv.y, qv.y), r.y);
-      r.z = __fmaf_rn(coef, __fsub_rn(xv.z, qv.z), r.z); r.w = __fmaf_rn(coef, __fsub_rn(xv.w, qv.w), r.w);
+      const float4 xv = __ldg(x + i), qv = HAS_Q ? __ldg(q + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+      if (HAS_Q) {
+        r.x = __fmaf_rn(coef, __fsub_rn(xv.x, qv.x), r.x); r.y = __fmaf_rn(coef, __fsub_rn(xv.y, qv.y), r.y);
+        r.z = __fmaf_rn(coef, __fsub_rn(xv.z, qv.z), r.z); r.w = __fmaf_rn(coef, __fsub_rn(xv.w, qv.w), r.w);
+      } else {
+        r.x = __fmaf_rn(coef, xv.x, r.x); r.y = __fmaf_rn(coef, xv.y, r.y);
+        r.z = __fmaf_rn(coef, xv.z, r.z); r.w = __fmaf_rn(coef, xv.w, r.w);
+      }
     }
     o[i] = r;
   }
@@ -1348,6 +1467,61 @@ static int stats_det_range(const float* x, long long B, long long P, long long D
   return 0;
 }
 
+// ---- residual VQ --------------------------------------------------------------------------------------------------------
+// S of a (Q, B, P) index array: c_0, then S + c_l in ascending l (vqseg_rvq_decode_f32); o.sP == 1 takes pixels fastest
+template <int MODE>
+__global__ void __launch_bounds__(256) rvq_decode_kernel(const long long* __restrict__ idx, int Q, const float* __restrict__ E,
+                                                         int K, RowsOut o, bool px_fast) {
+  const long long N = o.B * o.P, total = N * o.D;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    long long b, p, d;
+    if (px_fast) { p = i % o.P; long long t = i / o.P; d = t % o.D; b = t / o.D; }
+    else         { d = i % o.D; long long t = i / o.D; p = t % o.P; b = t / o.P; }
+    const long long n = b * o.P + p;
+    float s = 0.f;
+    for (int l = 0; l < Q; ++l) {
+      long long k = __ldg(idx + l * N + n);
+      k = k < 0 ? 0 : (k >= K ? K - 1 : k);
+      const float c = round_code<MODE>(__ldg(E + ((long long)l * K + k) * o.D + d));
+      s = l ? __fadd_rn(s, c) : c;
+    }
+    o.ptr[b * o.sB + p * o.sP + d * o.sD] = s;
+  }
+}
+
+namespace vqseg {
+// the stage kernel of vqseg_rvq_stage_f32 (api.cu enqueues the assignment before it): the gather instantiated with RVQ
+int rvq_stage_gather(const float* r, int64_t B, int64_t P, int64_t D, int64_t sB, int64_t sP, int64_t sD,
+                     const float* x, int64_t xB, int64_t xP, int64_t xD, const float* E, int64_t K, const int64_t* idx,
+                     float* q, int64_t qB, int64_t qP, int64_t qD, float* r_next, float* acc,
+                     float* layer_mse, float* layer_usage, const int64_t* counts, int layer, int n_layers, float weight,
+                     float* loss_out, float* usage_out, int mode, void* ws, size_t ws_bytes, cudaStream_t st, int* ticket) {
+  const bool train = gather_train(mode);
+  const bool last = layer == n_layers - 1;
+  Rows xr{r, B, P, D, sB, sP, sD};
+  if (!train && !r_next) { xr.ptr = nullptr; xr.sB = qB; xr.sP = qP; xr.sD = qD; }   // the last eval stage reads no r
+  RowsOut qr{q, B, P, D, qB, qP, qD};
+  const unsigned long long* cu = (const unsigned long long*)counts;
+  RvqStage rs{r_next, train ? acc : nullptr, Rows{(train && last) ? x : nullptr, B, P, D, xB, xP, xD}, layer == 0,
+              layer_mse, cu, n_layers, weight, last ? loss_out : nullptr, train ? 1 : 0, last ? usage_out : nullptr};
+  float* partial = (float*)ws;
+  const size_t cap = ws ? ws_bytes / sizeof(float) : 0;
+  const long long* ix = (const long long*)idx;
+  const unsigned long long* cl = cu + (long long)layer * K;
+  float* lm = train ? layer_mse + layer : nullptr;
+  float* lu = layer_usage + layer;
+  switch (mode) {
+    case VQSEG_MODE_EVAL:      return launch_gather<VQSEG_MODE_EVAL, true>(xr, E, (int)K, ix, qr, nullptr, partial, cap, st, ticket, cl, lu, rs);
+    case VQSEG_MODE_EVAL_AMP:  return launch_gather<VQSEG_MODE_EVAL_AMP, true>(xr, E, (int)K, ix, qr, nullptr, partial, cap, st, ticket, cl, lu, rs);
+    case VQSEG_MODE_EVAL_AMP_BF16: return launch_gather<VQSEG_MODE_EVAL_AMP_BF16, true>(xr, E, (int)K, ix, qr, nullptr, partial, cap, st, ticket, cl, lu, rs);
+    case VQSEG_MODE_TRAIN:     return launch_gather<VQSEG_MODE_TRAIN, true>(xr, E, (int)K, ix, qr, lm, partial, cap, st, ticket, cl, lu, rs);
+    case VQSEG_MODE_TRAIN_AMP: return launch_gather<VQSEG_MODE_TRAIN_AMP, true>(xr, E, (int)K, ix, qr, lm, partial, cap, st, ticket, cl, lu, rs);
+    case VQSEG_MODE_TRAIN_AMP_BF16: return launch_gather<VQSEG_MODE_TRAIN_AMP_BF16, true>(xr, E, (int)K, ix, qr, lm, partial, cap, st, ticket, cl, lu, rs);
+  }
+  return VQSEG_EINVAL;
+}
+}  // namespace vqseg
+
 extern "C" {
 
 size_t vqseg_gather_workspace_bytes(int64_t n_rows, int64_t D) {
@@ -1426,7 +1600,7 @@ int vqseg_ste_bwd_f32(const float* g_q, int64_t gB, int64_t gP, int64_t gD,
                       float* gx, int64_t oB, int64_t oP, int64_t oD,
                       int64_t B, int64_t P, int64_t D, void* stream) {
   if (!gx || B < 0 || P < 0 || D <= 0) return VQSEG_EINVAL;
-  if (coef_dev && (!x || !q_ste)) return VQSEG_EINVAL;
+  if (coef_dev && !x) return VQSEG_EINVAL;
   if (B * P == 0) return 0;
   {
     auto dense = [&](int64_t b, int64_t p, int64_t d) {
@@ -1435,10 +1609,14 @@ int vqseg_ste_bwd_f32(const float* g_q, int64_t gB, int64_t gP, int64_t gD,
     auto same = [&](int64_t b, int64_t p, int64_t d) { return b == oB && p == oP && d == oD; };
     auto al = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
     const long long total = B * P * D;
-    if (dense(oB, oP, oD) && (!g_q || same(gB, gP, gD)) && (!coef_dev || (same(sB, sP, sD) && same(qB, qP, qD))) &&
+    if (dense(oB, oP, oD) && (!g_q || same(gB, gP, gD)) && (!coef_dev || (same(sB, sP, sD) && (!q_ste || same(qB, qP, qD)))) &&
         total % 4 == 0 && al(gx) && al(g_q) && al(x) && al(q_ste)) {
-      ste_bwd_flat_kernel<<<grid_for(total / 4, 256, 8), 256, 0, (cudaStream_t)stream>>>(
-          (const float4*)g_q, (const float4*)x, (const float4*)q_ste, coef_dev, coef_scale, (float4*)gx, total / 4);
+      if (coef_dev && !q_ste)
+        ste_bwd_flat_kernel<false><<<grid_for(total / 4, 256, 8), 256, 0, (cudaStream_t)stream>>>(
+            (const float4*)g_q, (const float4*)x, nullptr, coef_dev, coef_scale, (float4*)gx, total / 4);
+      else
+        ste_bwd_flat_kernel<<<grid_for(total / 4, 256, 8), 256, 0, (cudaStream_t)stream>>>(
+            (const float4*)g_q, (const float4*)x, (const float4*)q_ste, coef_dev, coef_scale, (float4*)gx, total / 4);
       VQSEG_LAUNCH_CHECK();
       return 0;
     }
@@ -1446,7 +1624,10 @@ int vqseg_ste_bwd_f32(const float* g_q, int64_t gB, int64_t gP, int64_t gD,
   View g{g_q, gB, gP, gD}, xv{x, sB, sP, sD}, qv{q_ste, qB, qP, qD};
   RowsOut o{gx, B, P, D, oB, oP, oD};
   bool px_fast = (oP == 1);
-  ste_bwd_kernel<<<grid_for(B * P * D, 256, 16), 256, 0, (cudaStream_t)stream>>>(g, xv, qv, coef_dev, coef_scale, o, px_fast);
+  if (coef_dev && !q_ste)
+    ste_bwd_kernel<false><<<grid_for(B * P * D, 256, 16), 256, 0, (cudaStream_t)stream>>>(g, xv, qv, coef_dev, coef_scale, o, px_fast);
+  else
+    ste_bwd_kernel<<<grid_for(B * P * D, 256, 16), 256, 0, (cudaStream_t)stream>>>(g, xv, qv, coef_dev, coef_scale, o, px_fast);
   VQSEG_LAUNCH_CHECK();
   return 0;
 }
@@ -1757,6 +1938,25 @@ int vqseg_l2norm_f32(const float* x, int64_t B, int64_t P, int64_t D, int64_t sB
     } else {
       l2norm_strided_kernel<<<(unsigned)((B * P + 255) / 256), 256, 0, st>>>(xr, orow);
     }
+  }
+  VQSEG_LAUNCH_CHECK();
+  return 0;
+}
+
+int vqseg_rvq_decode_f32(const int64_t* idx, int64_t Q, int64_t B, int64_t P, const float* E, int64_t K, int64_t D,
+                         float* out, int64_t oB, int64_t oP, int64_t oD, int mode, void* stream) {
+  if (Q < 1 || Q >= (1ll << 31) || B < 0 || P < 0 || D <= 0 || K <= 0 || K * D >= (1ll << 40)) return VQSEG_EINVAL;
+  if (B * P == 0) return 0;
+  if (!idx || !E || !out) return VQSEG_EINVAL;
+  RowsOut o{out, B, P, D, oB, oP, oD};
+  const unsigned grid = grid_for(B * P * D, 256, 16);
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long* ix = (const long long*)idx;
+  switch (mode) {
+    case VQSEG_MODE_EVAL: rvq_decode_kernel<VQSEG_MODE_EVAL><<<grid, 256, 0, st>>>(ix, (int)Q, E, (int)K, o, oP == 1); break;
+    case VQSEG_MODE_EVAL_AMP: rvq_decode_kernel<VQSEG_MODE_EVAL_AMP><<<grid, 256, 0, st>>>(ix, (int)Q, E, (int)K, o, oP == 1); break;
+    case VQSEG_MODE_EVAL_AMP_BF16: rvq_decode_kernel<VQSEG_MODE_EVAL_AMP_BF16><<<grid, 256, 0, st>>>(ix, (int)Q, E, (int)K, o, oP == 1); break;
+    default: return VQSEG_EINVAL;
   }
   VQSEG_LAUNCH_CHECK();
   return 0;

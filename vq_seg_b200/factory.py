@@ -5,6 +5,7 @@ import sys
 
 from torch import nn
 
+from .rvq import ResidualVectorQuantizer
 from .vq_img import VectorQuantizer
 
 
@@ -14,10 +15,16 @@ def _get(cfg, key):
 
 def make_vq_module(vq_cfg, encoder_channels, depth):
     """vq_cfg: dict / EasyDict with the reference's keys (num_embeddings int or list, distance,
-    kmeans_init, ... every VectorQuantizer kwarg).  Unknown keys raise TypeError like the reference."""
+    kmeans_init, ... every VectorQuantizer kwarg).  Unknown keys raise TypeError like the reference.
+    Extension: a `num_quantizers` key builds a ResidualVectorQuantizer with that many layers at every
+    non-Identity level instead of a VectorQuantizer."""
+    cls, extra = VectorQuantizer, {}
+    if "num_quantizers" in vq_cfg:
+        vq_cfg = copy.deepcopy(vq_cfg)
+        cls, extra = ResidualVectorQuantizer, {"num_quantizers": vq_cfg.pop("num_quantizers")}
     num_embeddings = _get(vq_cfg, "num_embeddings")
     if isinstance(num_embeddings, int):
-        codebook = nn.ModuleList([VectorQuantizer(**vq_cfg, dim=encoder_channels[i + 1]) for i in range(depth)])
+        codebook = nn.ModuleList([cls(**vq_cfg, **extra, dim=encoder_channels[i + 1]) for i in range(depth)])
     elif isinstance(num_embeddings, list):
         assert depth == len(num_embeddings), "depth and length of vq_cfg.num_embeddings must to be same number"
         lst = []
@@ -27,7 +34,7 @@ def make_vq_module(vq_cfg, encoder_channels, depth):
             if num_embed == 0:
                 lst.append(Identity())
             elif num_embed > 0:
-                lst.append(VectorQuantizer(**vq_cfg, dim=encoder_channels[i + 1]))
+                lst.append(cls(**vq_cfg, **extra, dim=encoder_channels[i + 1]))
             else:
                 raise ValueError(f"{num_embed} is not available number of embeddings")
         codebook = nn.ModuleList(lst)

@@ -249,9 +249,10 @@ def _(x, codebook, idx, mode):
             x.new_empty((1,), dtype=torch.float32))
 
 
-def _ste_bwd_impl(grad_q: Optional[torch.Tensor], x: torch.Tensor, q_ste: torch.Tensor,
+def _ste_bwd_impl(grad_q: Optional[torch.Tensor], x: torch.Tensor, q_ste: Optional[torch.Tensor],
             grad_mse: Optional[torch.Tensor], coef_scale: float) -> torch.Tensor:
-    """gx = grad_q + coef_scale * grad_mse * (x - q_ste)   (coef_scale = 2 / numel)."""
+    """gx = grad_q + coef_scale * grad_mse * (x - q_ste)   (coef_scale = 2 / numel).  q_ste=None stands for zeros:
+    gx = fma(coef, x, grad_q), the residual quantizer's backward with x = the accumulated commitment term A."""
     _require_cuda(x, q_ste, grad_q, grad_mse)
     L = _native.lib()
     b, p, d, sb, sp, sd = _bpd(x)
@@ -263,7 +264,7 @@ def _ste_bwd_impl(grad_q: Optional[torch.Tensor], x: torch.Tensor, q_ste: torch.
     gm = grad_mse.reshape(-1)[:1].float().contiguous() if grad_mse is not None else None
     with torch.cuda.device(x.device):
         _native.check(L.vqseg_ste_bwd_f32(g[0], g[1], g[2], g[3], x.data_ptr(), sb, sp, sd,
-                                          q_ste.data_ptr(), q_ste.stride(0), q_ste.stride(1), q_ste.stride(2),
+                                          *((q_ste.data_ptr(), *q_ste.stride()) if q_ste is not None else (None, 0, 0, 0)),
                                           gm.data_ptr() if gm is not None else None, coef_scale,
                                           gx.data_ptr(), gx.stride(0), gx.stride(1), gx.stride(2),
                                           b, p, d, _stream()), "ste_bwd")
@@ -313,6 +314,84 @@ def _x_grad(mode, grad_q, x, q, grad_mse):
     if mode & MODE_ROTATE:
         return (_rotate_bwd_impl if _fast() else rotate_bwd)(grad_q, x, q, grad_mse, 2.0 / x.numel())
     return (_ste_bwd_impl if _fast() else ste_bwd)(grad_q, x, q, grad_mse, 2.0 / x.numel())
+
+
+# -------------------------------------------------------------------------------------------------
+# residual vector quantization (opt-in extension, vqseg.h: vqseg_rvq_stage_f32 / vqseg_rvq_decode_f32)
+def _rvq_stage_impl(r: torch.Tensor, rn: Optional[torch.Tensor], codebook: torch.Tensor, blob: Optional[torch.Tensor],
+                    x: torch.Tensor, q: torch.Tensor, r_next: Optional[torch.Tensor], acc: Optional[torch.Tensor],
+                    idx: torch.Tensor, counts: torch.Tensor, layer_mse: torch.Tensor, layer_usage: torch.Tensor,
+                    loss: torch.Tensor, usage: torch.Tensor, layer: int, mode: int, algo: int, weight: float) -> None:
+    """Stage `layer` of Q = idx.shape[0] in one host call: the lookup of r (Euclidean, or the inner product of its
+    normalised rows rn for the cosine codebook), then per element S (into q), r_next = r - c, A (into acc, training)
+    and, in the last training stage, quantize = x + (S - x) into q.  idx (Q, B, P) and counts (Q, K) get row `layer`;
+    layer_mse / layer_usage (Q,) entry `layer`; the last stage writes the pooled loss (training) and usage."""
+    _require_cuda(r, rn, codebook, blob, x, q, r_next, acc, idx, counts)
+    L = _native.lib()
+    cb = codebook.detach()
+    if cb.dtype != torch.float32 or not cb.is_contiguous():
+        cb = cb.contiguous().float()
+    b, p, d, sb, sp, sd = _bpd(r)
+    k = cb.shape[0]
+    if cb.shape[1] != d:
+        raise RuntimeError(f"X1 and X2 must have the same number of columns. X1: {d} X2: {cb.shape[1]}")
+    nq = idx.shape[0]
+    for t in (q, r_next, acc):
+        if t is not None and t.stride() != q.stride():
+            raise RuntimeError("rvq_stage: q, r_next and acc must share strides")
+    nws = L.vqseg_rvq_stage_workspace_bytes(b * p, d, k)
+    ws = torch.empty(nws, dtype=torch.uint8, device=r.device)
+    ptr = lambda t: t.data_ptr() if t is not None and t.numel() else None  # noqa: E731
+    rnv = (ptr(rn), *rn.stride()) if rn is not None else (None, 0, 0, 0)
+    with torch.cuda.device(r.device):
+        _native.check(L.vqseg_rvq_stage_f32(ptr(r), b, p, d, sb, sp, sd, *rnv, ptr(x), *x.stride(),
+                                            cb.data_ptr(), k, ptr(blob), ptr(idx[layer]), counts.data_ptr(),
+                                            ptr(q), *q.stride(), ptr(r_next), ptr(acc),
+                                            layer_mse.data_ptr(), layer_usage.data_ptr(), ptr(loss), ptr(usage),
+                                            layer, nq, float(weight), mode, algo, ws.data_ptr(), nws, _stream()),
+                      "rvq_stage")
+
+
+rvq_stage = torch.library.custom_op(
+    "vqseg::rvq_stage",
+    mutates_args=("q", "r_next", "acc", "idx", "counts", "layer_mse", "layer_usage", "loss", "usage"))(_rvq_stage_impl)
+
+
+@rvq_stage.register_fake
+def _(r, rn, codebook, blob, x, q, r_next, acc, idx, counts, layer_mse, layer_usage, loss, usage, layer, mode, algo,
+      weight):
+    return None
+
+
+def _rvq_decode_impl(idx: torch.Tensor, codebooks: torch.Tensor, mode: int = 0) -> torch.Tensor:
+    """S = sum over l of the rounded codes codebooks[l][idx[l]] in ascending l, from (Q, B, P) indices and (Q, K, D)
+    codebooks: (B, P, D) in NCHW memory order, bit-equal to the eval forward's quantize.  mode: MODE_EVAL*."""
+    _require_cuda(idx, codebooks)
+    L = _native.lib()
+    nq, b, p = idx.shape
+    cb = codebooks.detach()
+    if cb.dtype != torch.float32 or not cb.is_contiguous():
+        cb = cb.contiguous().float()
+    k, d = cb.shape[1], cb.shape[2]
+    if cb.shape[0] != nq:
+        raise RuntimeError(f"rvq_decode: {nq} index layers for {cb.shape[0]} codebooks")
+    idx = idx.to(torch.int64).contiguous()
+    out = torch.empty_strided((b, p, d), (d * p, 1, p), dtype=torch.float32, device=idx.device)
+    with torch.cuda.device(idx.device):
+        _native.check(L.vqseg_rvq_decode_f32(idx.data_ptr() if idx.numel() else None, nq, b, p, cb.data_ptr(), k, d,
+                                             out.data_ptr() if out.numel() else None, *out.stride(), mode, _stream()),
+                      "rvq_decode")
+    return out
+
+
+rvq_decode = torch.library.custom_op("vqseg::rvq_decode", mutates_args=())(_rvq_decode_impl)
+
+
+@rvq_decode.register_fake
+def _(idx, codebooks, mode=0):
+    nq, b, p = idx.shape
+    d = codebooks.shape[2]
+    return torch.empty_strided((b, p, d), (d * p, 1, p), dtype=torch.float32, device=idx.device)
 
 
 def _gather_bwd_codebook_impl(grad_q: torch.Tensor, idx: torch.Tensor, num_codes: int) -> torch.Tensor:

@@ -241,6 +241,12 @@ class CosinesimCodebook(_CodebookBase):
         if x.shape[-1] != self.embedding_dim:
             raise RuntimeError(f"einsum(): operands do not broadcast with remapped shapes: {x.shape[-1]} vs {self.embedding_dim}")
         xn = ops.l2norm_rows(x)
+        blob = self._renormalise_and_prepare()
+        return ops.fast_assign(xn, self.embedding.weight.detach(), blob, self.algo | ops.METRIC_IP)
+
+    def _renormalise_and_prepare(self):
+        """The in-place renormalisation of the weights (vq_img.py:100), then the inner-product blob (None for
+        ALGO_EXACT) rebuilt for the renormalised rows."""
         w = self.embedding.weight
         ops.l2norm_rows_(w.data)
         blob = None
@@ -252,7 +258,7 @@ class CosinesimCodebook(_CodebookBase):
                 # rebuild the prepared image here with the multi-block kernels instead of leaving it to the assignment's
                 # guard, which rebuilds inside a single block (measured: 360-600 us per forward against ~170)
                 ops.fast_refresh_codebook(blob, w.detach(), True)
-        return ops.fast_assign(xn, w.detach(), blob, self.algo | ops.METRIC_IP)
+        return blob
 
     def forward(self, x):
         """x: (B, HxW, C) -> (quantized, embed_idx, code_usage)   [vq_img.py:93-113]"""
@@ -264,6 +270,37 @@ class CosinesimCodebook(_CodebookBase):
         idx, counts = self.lookup(x)
         quantized = ops.eval_gather(self.embedding.weight, x, idx)
         return quantized, idx, ops.code_usage(counts)
+
+
+class CudaGraphCache(dict):
+    """The opt-in CUDA-graph mode of the quantizer modules (enable_cuda_graphs): ONE captured graph of a no-grad forward
+    per (input address, shape, strides, dtype, `extra`), at most `max_entries` of them (the oldest goes first)."""
+
+    def __init__(self, max_entries: int = 16):
+        super().__init__()
+        self.max_entries = max_entries
+
+    def run(self, forward, x, extra, keep):
+        """forward(x)'s outputs, replayed from the entry's graph (captured on the first call).  `keep()` names what the
+        graph reads beyond x and the module's parameters (the prepared codebooks): the entry holds it alive."""
+        key = (x.data_ptr(), tuple(x.shape), tuple(x.stride()), x.dtype) + tuple(extra) + (torch.cuda.current_device(),)
+        ent = self.get(key)
+        if ent is None:
+            if len(self) >= self.max_entries:
+                self.pop(next(iter(self)))                        # oldest entry
+            cur = torch.cuda.current_stream()
+            side = torch.cuda.Stream()
+            side.wait_stream(cur)
+            with torch.cuda.stream(side):                         # warm-up outside the capture (lazy init, allocations)
+                forward(x)
+            cur.wait_stream(side)
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                outs = forward(x)
+            ent = (g, outs, keep())                               # what the graph reads must outlive the cache's view of it
+            self[key] = ent
+        ent[0].replay()
+        return ent[1]
 
 
 class VectorQuantizer(nn.Module):
@@ -292,8 +329,7 @@ class VectorQuantizer(nn.Module):
         address (a reused activation buffer / a static input).  Weight updates are picked up: the kernels re-check the
         prepared codebook against the live weights on the device.  Training-mode and grad-enabled calls, the k-means
         init and the EMA update take the ordinary path."""
-        self._graphs = {}
-        self._graphs_max = max_entries
+        self._graphs = CudaGraphCache(max_entries)
         return self
 
     def disable_cuda_graphs(self):
@@ -303,24 +339,7 @@ class VectorQuantizer(nn.Module):
     def _graph_forward(self, x):
         amp = ops.autocast_code_dtype(self.amp_compat)
         w = self.codebook.embedding.weight
-        key = (x.data_ptr(), tuple(x.shape), tuple(x.stride()), x.dtype, amp, w.data_ptr(), torch.cuda.current_device())
-        ent = self._graphs.get(key)
-        if ent is None:
-            if len(self._graphs) >= self._graphs_max:
-                self._graphs.pop(next(iter(self._graphs)))        # oldest entry
-            cur = torch.cuda.current_stream()
-            side = torch.cuda.Stream()
-            side.wait_stream(cur)
-            with torch.cuda.stream(side):                         # warm-up outside the capture (lazy init, allocations)
-                self._forward_impl(x)
-            cur.wait_stream(side)
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                outs = self._forward_impl(x)
-            ent = (g, outs, self.codebook._blob)                  # the blob the graph reads must outlive the cache's view of it
-            self._graphs[key] = ent
-        ent[0].replay()
-        return ent[1]
+        return self._graphs.run(self._forward_impl, x, (amp, w.data_ptr()), lambda: self.codebook._blob)
 
     def enable_ema(self, **kw):
         """Opt-in EMA codebook update with the stored `decay` and `eps`, optionally with dead-code expiry
